@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the Lanczos hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): 1920x1080 -> 3840x2160 RGB8, 2x, Lanczos-3.  One "step" is one pass of
 the hot path over a batch of `--frames` distinct synthetic frames per GPU, ONE kernel launch (the batch is ~2 GB
@@ -263,6 +263,26 @@ def bench_batch(ctx, lz, name, frames, steps, flags=0, contents=("mix",)):
     return res, st["kernel_id"], st["kernel_launches"]
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, d_out):
+    """--dump-outputs: the uint8 output batch [F][H][W][C] as float32 in path/output.npy, whole when it fits in
+    DUMP_BYTES, else the same seeded sample of pixel positions (ascending raster order) in every frame, shape
+    [F][P][C].  The inputs are seeded too, so two builds run with the same arguments can be compared value for value."""
+    import numpy as np
+    import torch
+    F, H, W, C = d_out.shape
+    per_frame = max(1, DUMP_BYTES // (4 * F * C))
+    if H * W <= per_frame:
+        out = d_out
+    else:
+        pos = torch.randperm(H * W, generator=torch.Generator().manual_seed(0))[:per_frame].sort().values
+        out = d_out.reshape(F, H * W, C).index_select(1, pos.to(d_out.device))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "output.npy"), out.cpu().numpy().astype(np.float32))
+
+
 def summarise_batch(name, frames, n_gpus, ms, peak):
     iw, ih, ow, oh, ch = WORKLOADS[name][:5]
     algo = frames * (iw * ih * ch + ow * oh * ch)
@@ -319,6 +339,8 @@ def bands_line(args, ctx, lz):
         sampler.start()
         time.sleep(0.3)
     res, st, geo, (d_in, d_out, step) = bench_bands(ctx, lz, args.band_size, steps, contents=("image_like", "noise"))
+    if args.dump_outputs and ctx.rank == 0:
+        dump_outputs(args.dump_outputs, d_out.unsqueeze(0))      # the noise band, the last content timed
     # a band step takes a few ms: keep the same kernel running (untimed) until the 50 ms clock sampler has seen it
     t_load = time.perf_counter()
     while time.perf_counter() - t_load < 0.5:
@@ -412,7 +434,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the c3 / c4 / c5_bands / single-frame sub-benchmarks")
     ap.add_argument("--flags", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the output of the last one to DIR/output.npy (float32, see "
+                         "dump_outputs); with several GPUs only rank 0's frames, each rank's being seeded differently")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's output: not with --impl reference")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -427,8 +456,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        # bounded: 1/8-frame samples, at most ~2 minutes regardless of --steps
-        steps = max(1, min(args.steps, 40))
+        steps = args.steps
         res = run_reference_cpu(steps, min(args.warmup, 2))
         line = {
             "impl": "reference", "metric": "output Mpix/s", "value": res["value"], "unit": "Mpix/s",
@@ -504,6 +532,8 @@ def main():
     ctx.barrier()
     ms_per_step = ctx.max_over_ranks(e0.elapsed_time(e1)) / args.steps
     ms_local = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out)       # before the tolerance-mode steps below overwrite d_out
     value = n_gpus * F * px_per_frame / (ms_per_step * 1e-3) / 1e6
     by_content[args.content] = {"value": value, "unit": "Mpix/s", "ms_per_step": ms_per_step,
                                 "roofline_frac": F * algo_per_frame / (ms_local * 1e-3) / 1e9 / peak}

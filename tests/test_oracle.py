@@ -41,11 +41,16 @@ def test_golden_fixtures(oracle, path):
 
 
 def test_against_compiled_reference(oracle):
-    """Bit-equality with oracle/_ref on fresh seeds (skipped when the objects are not present)."""
-    cfgs = [c for c in oracle.ref_configs() if c[0] * c[1] <= 100 * 60]
-    if not cfgs:
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    for cfg in cfgs:
+    """Bit-equality with the compiled reference: with the hashes of its outputs that tests/golden/make_golden.py stored
+    in tests/golden/ref_hashes.txt (input: xorshift seed SEED, planar), and with oracle/_ref itself on fresh seeds
+    where those objects have been built from a reference tree (oracle/Makefile targets ref, refhls)."""
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_hashes.txt")) as fh:
+        stored = [[int(v) for v in ln.split()[:8]] + [int(ln.split()[8], 16)] for ln in fh if not ln.startswith("#")]
+    assert len(stored) == 3
+    for iw, ih, ow, oh, n, d, a, c, want in stored:
+        img = oracle.xorshift_bytes(c * ih * iw).reshape(c, ih, iw)
+        assert oracle.fnv1a64(oracle.expected_planar(img, ow, oh, a, n, d)) == want, (iw, ih, ow, oh, n, d, a, c)
+    for cfg in [c for c in oracle.ref_configs() if c[0] * c[1] <= 100 * 60]:
         iw, ih, ow, oh, n, d, a, c = cfg
         for seed in (11, 12):
             img = oracle.xorshift_bytes(c * ih * iw, oracle.SEED + seed).reshape(c, ih, iw)
