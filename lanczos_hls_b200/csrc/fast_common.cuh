@@ -1,6 +1,9 @@
 // fast_common.cuh -- device/host helpers shared by the TMA + register-window kernels
 // (lanczos_v6.cu: static-phase H pass for a few ratios; lanczos_dyn.cu: any ratio with N <= 32).
 #pragma once
+#include <algorithm>
+#include <atomic>
+#include <cmath>
 #include <cstdint>
 #include <cuda.h>
 #include <cuda_runtime.h>
@@ -9,6 +12,46 @@
 
 namespace lzb {
 namespace {
+
+// ---------------------------------------------------------------------------------------------
+// kernel parameters and the static vertical phase pattern
+// ---------------------------------------------------------------------------------------------
+// What both kernel families know about a launch: the output band and how it is cut into vertical segments.  The
+// kernels read out_row0 + out_rows and vperiod0 + seg_periods together: each pair shares one 8-byte word.
+struct StripParams {
+    uint8_t *out;         // output row `out_row0` of frame 0
+    long long out_pitch, out_frame_stride;
+    int out_row0, out_rows;
+    int seg_periods;      // vertical ratio-periods per segment
+    int vperiod0;         // first vertical period covered by the launch (floor(out_row0 / N))
+    int out_w, in_row0;
+};
+
+__host__ __device__ constexpr int cdiv(int a, int b) { return (a + b - 1) / b; }
+__host__ __device__ constexpr int lcm2(int d) { return d % 2 == 0 ? d : 2 * d; }
+
+// residue s of a completing centre (c = D*t + s): its output rows are N*t + [ylo, yhi)
+template <int N, int D> __host__ __device__ constexpr int ylo(int s) { return cdiv(s * N, D); }
+template <int N, int D> __host__ __device__ constexpr int yhi(int s) { return cdiv((s + 1) * N, D); }
+template <int N, int D> __host__ __device__ constexpr int cnt(int s) {   // interpolated (phase != 0) rows among them
+    int n = 0;
+    for (int yr = ylo<N, D>(s); yr < yhi<N, D>(s); yr++) n += ((yr * D) % N != 0) ? 1 : 0;
+    return n;
+}
+template <int N, int D, int TAPS> __host__ __device__ constexpr int nslot() {   // partial sums alive while a row is processed
+    int best = 0;
+    for (int s0 = 0; s0 < D; s0++) {
+        int n = 0;
+        for (int dc = 0; dc < TAPS; dc++) n += cnt<N, D>((s0 + dc) % D);
+        best = n > best ? n : best;
+    }
+    return best;
+}
+template <int N, int D> __host__ __device__ constexpr int cntmax() {   // rows completed by one input row (at least 1)
+    int best = 1;
+    for (int s = 0; s < D; s++) best = cnt<N, D>(s) > best ? cnt<N, D>(s) : best;
+    return best;
+}
 
 // ---------------------------------------------------------------------------------------------
 // PTX helpers
@@ -61,6 +104,12 @@ __device__ __forceinline__ void word_to_f32x4(uint32_t w, float &f0, float &f1, 
     f0 = h2_lo_to_f32(a); f1 = h2_hi_to_f32(a); f2 = h2_lo_to_f32(b); f3 = h2_hi_to_f32(b);
 }
 
+__device__ __forceinline__ uint32_t hfma2(uint32_t a, uint32_t b, uint32_t c) {
+    uint32_t d;
+    asm("fma.rn.f16x2 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
+    return d;
+}
+
 // double_to_uint8 (full_TB.h:29-37) on four fp32 values, packed little-endian: clamp to [0,255],
 // truncate toward zero. ptxas fuses each cvt.rzi pair + cvt.pack into ONE F2IP.U8.F32.TRUNC.
 __device__ __forceinline__ uint32_t quantise4(float a, float b, float c, float d) {
@@ -102,6 +151,114 @@ EncodeFn get_encode() {
     return fn;
 }
 
+// ---------------------------------------------------------------------------------------------
+// host side of a launch
+// ---------------------------------------------------------------------------------------------
+// Layout requirements of the TMA map and of the 32-bit accesses: input and output row bytes %4, input pitch %16,
+// output pitch %4, 16-byte aligned input base, 4-byte aligned output base, and the same for the frame strides.
+inline bool strip_layout_ok(const KParams &k) {
+    if ((k.in_w * k.channels) % 4 != 0 || (k.out_w * k.channels) % 4 != 0) return false;
+    if (k.in_pitch % 16 != 0 || k.out_pitch % 4 != 0) return false;
+    if ((reinterpret_cast<uintptr_t>(k.in) & 15) != 0 || (reinterpret_cast<uintptr_t>(k.out) & 3) != 0) return false;
+    if (k.n_frames > 1 && (k.in_frame_stride % 16 != 0 || k.out_frame_stride % 4 != 0)) return false;
+    return true;
+}
+
+// The input frames as a 3-D tensor of 32-bit words (x, row, frame), read in boxes of box_bytes x box_rows; TMA fills
+// what lies outside the image with zeros, which are the reference's dropped taps.
+inline bool encode_input_map(CUtensorMap *map, const KParams &k, int box_bytes, int box_rows) {
+    EncodeFn encode = get_encode();
+    if (!encode) return false;
+    const cuuint64_t dims[3] = {(cuuint64_t)(k.in_w * k.channels / 4), (cuuint64_t)k.in_rows, (cuuint64_t)k.n_frames};
+    const cuuint64_t strides[2] = {(cuuint64_t)k.in_pitch, (cuuint64_t)(k.n_frames > 1 ? k.in_frame_stride : k.in_pitch * k.in_rows)};
+    const cuuint32_t box[3] = {(cuuint32_t)(box_bytes / 4), (cuuint32_t)box_rows, 1};
+    const cuuint32_t estr[3] = {1, 1, 1};
+    return encode(map, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, const_cast<uint8_t *>(k.in), dims, strides, box, estr,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+// Resident one-warp CTAs on the current device of one kernel instance that takes `smem` bytes of dynamic shared memory;
+// ctas = 0 when the kernel cannot have them (the caller then falls back to another kernel).  `ctas_per_sm` is the
+// instance's own cache, one entry per device: every instance of a family has the same function-pointer type, so each
+// launcher instantiation keeps its own.  The calls are idempotent, so two threads racing here only repeat them.
+struct Residency {
+    int sms;
+    long long ctas;
+};
+template <class Kernel>
+Residency resident_ctas(std::atomic<int> (&ctas_per_sm)[64], Kernel kern, size_t smem) {
+    // what both families are built for (__launch_bounds__(32, 16)); only used when the occupancy query fails
+    constexpr int kFallbackCtasPerSm = 16;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    std::atomic<int> &cached = ctas_per_sm[dev & 63];
+    int nb = cached.load(std::memory_order_acquire);
+    if (nb == 0) {
+        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+            cudaGetLastError();   // clear the error state: the caller falls back to another kernel
+            return {sms, 0};
+        }
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, 32, smem) != cudaSuccess || nb < 1) nb = kFallbackCtasPerSm;
+        cached.store(nb, std::memory_order_release);
+    }
+    return {sms, (long long)nb * sms};
+}
+
+// Vertical segments: the vperiods ratio periods of a launch split into segs segments of seg_periods periods each
+// (the last one may be shorter).
+struct SegPlan {
+    int segs, seg_periods;
+};
+inline SegPlan split_periods(int vperiods, int segs) {
+    const int seg_periods = cdiv(vperiods, segs);
+    return {cdiv(vperiods, seg_periods), seg_periods};
+}
+// every segment re-runs 2a-1 warm-up rows and works in whole chunks of RB rows: at least 2*RB input rows each
+inline int max_segments(int vperiods, int D, int RB) { return std::max(1, vperiods / std::max(1, (2 * RB) / D)); }
+
+// The segment count in 1 .. min(max_segs, cap) of least cost(periods per segment, segments)
+template <class Cost>
+int cheapest_segments(int vperiods, int max_segs, int cap, Cost cost) {
+    int segs = 1;
+    double best_cost = 1e300;
+    for (int sg = 1; sg <= std::min(max_segs, cap); sg++) {
+        const int per = cdiv(vperiods, sg);
+        const int sg_eff = cdiv(vperiods, per);
+        const double c = cost(per, sg_eff);
+        if (c < best_cost - 1e-9) { best_cost = c; segs = sg_eff; }
+    }
+    return segs;
+}
+
+// Segments of a batch (many waves of CTAs): cols = strips x frames CTA columns, slots = resident CTAs of the device.
+// It minimises (waves) x (rows per segment + warm-up + pipeline fill); a wave that is not full still costs a full wave
+// unless it is the only one.
+inline SegPlan plan_segments(int vperiods, int D, int A, int RB, long long cols, long long slots, int cap) {
+    const int segs = cheapest_segments(vperiods, max_segments(vperiods, D, RB), cap, [&](int per, int sg) {
+        const double rows = (double)per * D + 2 * A - 1 + 0.5 * RB;
+        const double waves = std::ceil((double)(cols * sg) / (double)slots);
+        return (cols * sg <= slots) ? rows : rows * waves;
+    });
+    return split_periods(vperiods, segs);
+}
+
+// The StripParams of a launch over the band [out_row0, out_row0 + out_rows) of k
+inline void set_strip_params(StripParams &p, const KParams &k, int vperiod0, int seg_periods) {
+    p.out = k.out;
+    p.out_pitch = k.out_pitch;
+    p.out_frame_stride = k.out_frame_stride;
+    p.out_w = k.out_w;
+    p.out_row0 = k.out_row0; p.out_rows = k.out_rows; p.in_row0 = k.in_row0;
+    p.seg_periods = seg_periods; p.vperiod0 = vperiod0;
+}
+
+// polyphase table [N][8] (padded to 8 taps) times 2^24, see kPixUnscale
+inline void fill_wtab(float *wtab, const FastHostTables &t, int A, int N) {
+    for (int ph = 0; ph < N; ph++)
+        for (int q = 0; q < 8; q++) wtab[ph * 8 + q] = q < 2 * A ? t.phase_w[ph * 2 * A + q] * 16777216.f : 0.f;
+}
 
 }  // namespace
 }  // namespace lzb

@@ -32,13 +32,7 @@ namespace lzb {
 
 namespace {
 
-struct DynParams {
-    uint8_t *out;         // output row `out_row0` of frame 0
-    long long out_pitch, out_frame_stride;
-    int in_w, in_h, out_w, out_h;
-    int out_row0, out_rows, in_row0, in_rows;
-    int seg_periods;      // vertical ratio-periods per segment
-    int vperiod0;         // first vertical period covered by the launch (floor(out_row0 / N))
+struct DynParams : StripParams {
     const int32_t *i0x;       // [out_w] first tap pixel per output pixel (plan AxisTables)
     const double *wdx, *wdy;  // per-coordinate double weights (exact evaluation)
     float guard;              // rigorous fp32 error bound (x1.06) of ascending-order chains with the phase table
@@ -48,58 +42,27 @@ struct DynParams {
     unsigned long long *strict_counter;
 };
 
-__host__ __device__ constexpr int cdivd(int a, int b) { return (a + b - 1) / b; }
-__host__ __device__ constexpr int lcm2d(int d) { return d % 2 == 0 ? d : 2 * d; }
-
 template <int C, int A, int N, int D>
 struct GeoD {
     static constexpr int VB = 4;                         // byte-columns per lane
     static constexpr int SWB = 32 * VB;                  // strip width in output bytes = ring pitch
     static constexpr int TAPS = 2 * A;
-    static constexpr int U = lcm2d(D);                   // input rows per V loop iteration (one ratio period, even)
-    static constexpr int RB = U * cdivd(TAPS > 6 ? TAPS : 6, U);   // input rows per chunk (>= 2a - 1: see the ring)
+    static constexpr int U = lcm2(D);                    // input rows per V loop iteration (one ratio period, even)
+    static constexpr int RB = U * cdiv(TAPS > 6 ? TAPS : 6, U);    // input rows per chunk (>= 2a - 1: see the ring)
     static constexpr int REGIONS = 2;
     static constexpr int RING = REGIONS * RB;
     static constexpr int STAGES = 4;
     // input pixels a strip can touch: its (SWB/C + 2) output pixels span that many * D/N input pixels, plus taps
     static constexpr int IN_PX = ((SWB / C + 2) * D) / N + 2 + TAPS;
-    static constexpr int BOX_B = 16 * cdivd(IN_PX * C + 15, 16);  // + 15: the box starts on a 16-byte boundary
-    static constexpr int STAGE_B = 128 * cdivd(RB * BOX_B, 128);
+    static constexpr int BOX_B = 16 * cdiv(IN_PX * C + 15, 16);   // + 15: the box starts on a 16-byte boundary
+    static constexpr int STAGE_B = 128 * cdiv(RB * BOX_B, 128);
     static constexpr int S0 = (((1 - 2 * A) % D) + D) % D;
     static constexpr int YROWS = N * RB / D;             // output rows completed per chunk
     static_assert(TAPS - 1 <= RB, "tap rows must not reach further back than one ring region");
     static_assert(BOX_B / 4 <= 256, "TMA box too wide");
     static_assert(N <= 32, "phase table too large for kernel params");
-    static_assert(cdivd(S0 * N, D) + YROWS <= 32, "fix mask (bit per output row) too small");
+    static_assert(cdiv(S0 * N, D) + YROWS <= 32, "fix mask (bit per output row) too small");
 };
-
-template <int N, int D> __host__ __device__ constexpr int ylod(int s) { return cdivd(s * N, D); }
-template <int N, int D> __host__ __device__ constexpr int yhid(int s) { return cdivd((s + 1) * N, D); }
-template <int N, int D> __host__ __device__ constexpr int cntd(int s) {
-    int n = 0;
-    for (int yr = ylod<N, D>(s); yr < yhid<N, D>(s); yr++) n += ((yr * D) % N != 0) ? 1 : 0;
-    return n;
-}
-template <int N, int D, int TAPS> __host__ __device__ constexpr int nslotd() {
-    int best = 0;
-    for (int s0 = 0; s0 < D; s0++) {
-        int n = 0;
-        for (int dc = 0; dc < TAPS; dc++) n += cntd<N, D>((s0 + dc) % D);
-        best = n > best ? n : best;
-    }
-    return best;
-}
-template <int N, int D> __host__ __device__ constexpr int cntmaxd() {
-    int best = 1;
-    for (int s = 0; s < D; s++) best = cntd<N, D>(s) > best ? cntd<N, D>(s) : best;
-    return best;
-}
-
-__device__ __forceinline__ uint32_t hfma2_d(uint32_t a, uint32_t b, uint32_t c) {
-    uint32_t d;
-    asm("fma.rn.f16x2 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
 
 // fma.rn.f32 WITHOUT .ftz whatever the compilation flags say (-use_fast_math would flush the denormal operand)
 __device__ __forceinline__ float fma_keep_denormals(float a, float b, float c) {
@@ -194,8 +157,8 @@ __global__ void __launch_bounds__(32, 16)
 lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ DynParams p) {
     using G = GeoD<C, A, N, D>;
     constexpr int TAPS = G::TAPS, SWB = G::SWB, VB = G::VB, RB = G::RB;
-    constexpr int NSLOT = nslotd<N, D, TAPS>();
-    constexpr int CNTMAX = cntmaxd<N, D>();
+    constexpr int NSLOT = nslot<N, D, TAPS>();
+    constexpr int CNTMAX = cntmax<N, D>();
     extern __shared__ __align__(128) uint8_t smem_raw[];
     SmemD<G> &sm = *reinterpret_cast<SmemD<G> *>(smem_raw);
 
@@ -405,7 +368,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
         auto body = [&](auto check_tag) {
             constexpr bool CHECK = decltype(check_tag)::value;
             const uint8_t *vit = vrow;
-            uint8_t *op = ocol + (long long)ylod<N, D>(G::S0) * opitch;   // next output row (rows come out in order)
+            uint8_t *op = ocol + (long long)ylo<N, D>(G::S0) * opitch;   // next output row (rows come out in order)
             int yit = ybase;
 #pragma unroll 1
             for (int it = 0; it < RB / G::U; it++) {
@@ -413,7 +376,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
 #pragma unroll
                 for (int u = 0; u < G::U; u++) {
                     const int s0 = (G::S0 + u) % D, tq = (G::S0 + u) / D;   // completing centre = D*(t + tq) + s0
-                    const int cnt0 = cntd<N, D>(s0);
+                    const int cnt0 = cnt<N, D>(s0);
                     const uint32_t w = *reinterpret_cast<const uint32_t *>(vit + u * SWB);
                     float x[VB];
                     word_to_f32x4(w, x[0], x[1], x[2], x[3]);
@@ -426,7 +389,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
                             const int sdc = (s0 + dc) % D;
                             const int k = TAPS - 1 - dc;
 #pragma unroll
-                            for (int yr = ylod<N, D>(sdc); yr < yhid<N, D>(sdc); yr++) {
+                            for (int yr = ylo<N, D>(sdc); yr < yhi<N, D>(sdc); yr++) {
                                 const int ph = (yr * D) % N;
                                 if (ph == 0) continue;
                                 const float2 wk2 = make_float2(p.wtab[ph * 8 + k], p.wtab[ph * 8 + k]);
@@ -446,7 +409,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
                     {
                         int q = 0;
 #pragma unroll
-                        for (int yr = ylod<N, D>(s0); yr < yhid<N, D>(s0); yr++) {
+                        for (int yr = ylo<N, D>(s0); yr < yhi<N, D>(s0); yr++) {
                             const int ph = (yr * D) % N;
                             const int yoff = N * tq + yr;                 // output row relative to yit
                             uint32_t qv;
@@ -470,7 +433,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
                                     for (int hsel = 0; hsel < 2; hsel++) {
                                         const uint32_t sel = hsel ? 0x4342u : 0x4140u;
                                         const uint32_t hv = __byte_perm(qv, 0u, sel);
-                                        z |= hfma2_d(__byte_perm(wa, 0u, sel), kR, hv) | hfma2_d(__byte_perm(wb, 0u, sel), kR, hv);
+                                        z |= hfma2(__byte_perm(wa, 0u, sel), kR, hv) | hfma2(__byte_perm(wb, 0u, sel), kR, hv);
                                     }
                                     doubt = (z & 0x80008000u) != 0u;
                                 }
@@ -521,8 +484,6 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
 template <int C, int A, int N, int D, int MODE>
 int launch_dyn_one(const KParams &k, const FastHostTables &t, cudaStream_t s) {
     using G = GeoD<C, A, N, D>;
-    EncodeFn encode = get_encode();
-    if (!encode) return -1;
     const int row_bytes = k.out_w * C;
     const int strips = (row_bytes + G::SWB - 1) / G::SWB;
     // every strip's input must fit the staged row: check with the host copy of the tap table
@@ -532,55 +493,19 @@ int launch_dyn_one(const KParams &k, const FastHostTables &t, cudaStream_t s) {
         const int last = (t.i0x_host[ob1 / C] + 2 * A) * C;      // one past the last byte read
         if (last - xb0 > G::BOX_B) return -1;
     }
-    const int vperiod0 = k.out_row0 / N;
-    const int vperiods = (k.out_row0 + k.out_rows + N - 1) / N - vperiod0;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    CUtensorMap map;
+    if (!encode_input_map(&map, k, G::BOX_B, G::RB)) return -1;
     auto kern = lanczos_dyn_kernel<C, A, N, D, MODE>;
     const size_t smem = sizeof(SmemD<G>) + 128;
-    // per device, set once; the calls are idempotent, so two threads racing here only repeat them
     static std::atomic<int> ctas_per_sm[64] = {};
-    if (ctas_per_sm[dev & 63].load(std::memory_order_acquire) == 0) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) { cudaGetLastError(); return -1; }   // clear the error state: the caller falls back to another kernel
-        int nb = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, 32, smem) != cudaSuccess || nb < 1) nb = 8;
-        ctas_per_sm[dev & 63].store(nb, std::memory_order_release);
-    }
-    // vertical segments: (waves) x (rows per segment + warm-up), as in lanczos_v6.cu
-    const long long slots = (long long)ctas_per_sm[dev & 63].load(std::memory_order_relaxed) * sms;
-    const long long cols = (long long)strips * k.n_frames;
-    const int max_segs = std::max(1, vperiods / std::max(1, (2 * G::RB) / D));
-    int segs = 1;
-    double best_cost = 1e300;
-    for (int sg = 1; sg <= std::min(max_segs, 512); sg++) {
-        const int per = (vperiods + sg - 1) / sg;
-        const int sg_eff = (vperiods + per - 1) / per;
-        const double rows = (double)per * D + 2 * A - 1 + 0.5 * G::RB;
-        const double waves = std::ceil((double)(cols * sg_eff) / (double)slots);
-        const double cost = (cols * sg_eff <= slots) ? rows : rows * waves;
-        if (cost < best_cost - 1e-9) { best_cost = cost; segs = sg_eff; }
-    }
-    int seg_periods = (vperiods + segs - 1) / segs;
-    segs = (vperiods + seg_periods - 1) / seg_periods;
-
-    CUtensorMap map;
-    const cuuint64_t dims[3] = {(cuuint64_t)(k.in_w * C / 4), (cuuint64_t)k.in_rows, (cuuint64_t)k.n_frames};
-    const cuuint64_t strides[2] = {(cuuint64_t)k.in_pitch, (cuuint64_t)(k.n_frames > 1 ? k.in_frame_stride : k.in_pitch * k.in_rows)};
-    const cuuint32_t box[3] = {(cuuint32_t)(G::BOX_B / 4), (cuuint32_t)G::RB, 1};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    if (encode(&map, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, const_cast<uint8_t *>(k.in), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return -1;
+    const Residency res = resident_ctas(ctas_per_sm, kern, smem);
+    if (res.ctas == 0) return -1;
+    const int vperiod0 = k.out_row0 / N;
+    const int vperiods = (k.out_row0 + k.out_rows + N - 1) / N - vperiod0;
+    const SegPlan sp = plan_segments(vperiods, D, A, G::RB, (long long)strips * k.n_frames, res.ctas, 512);
 
     DynParams p{};
-    p.out = k.out;
-    p.out_pitch = k.out_pitch;
-    p.out_frame_stride = k.out_frame_stride;
-    p.in_w = k.in_w; p.in_h = k.in_h; p.out_w = k.out_w; p.out_h = k.out_h;
-    p.out_row0 = k.out_row0; p.out_rows = k.out_rows; p.in_row0 = k.in_row0; p.in_rows = k.in_rows;
-    p.seg_periods = seg_periods; p.vperiod0 = vperiod0;
+    set_strip_params(p, k, vperiod0, sp.seg_periods);
     p.i0x = k.i0x; p.wdx = k.wdx; p.wdy = k.wdy;
     p.guard = k.guard_asc;
     // the cheap phase-0 test needs: coordinates exactly integral in double on both axes (then the weights there are
@@ -594,11 +519,10 @@ int launch_dyn_one(const KParams &k, const FastHostTables &t, cudaStream_t s) {
         }
         p.p0_filter = (A == 3 && km == 0x11 && small && t.exact_x && t.exact_y) ? 1 : 0;
     }
-    for (int ph = 0; ph < N; ph++)
-        for (int q = 0; q < 8; q++) p.wtab[ph * 8 + q] = q < 2 * A ? t.phase_w[ph * 2 * A + q] * 16777216.f : 0.f;
+    fill_wtab(p.wtab, t, A, N);
     p.strict_counter = k.strict_counter;
 
-    dim3 grid(strips, segs, k.n_frames);
+    dim3 grid(strips, sp.segs, k.n_frames);
     kern<<<grid, 32, smem, s>>>(map, p);
     return (int)cudaGetLastError();
 }
@@ -617,11 +541,7 @@ int launch_dyn(const KParams &k, const FastHostTables &t, int *kernel_id, cudaSt
 #else
 int launch_dyn_part1(const KParams &k, const FastHostTables &t, int *kernel_id, cudaStream_t s) {
 #endif
-    if ((k.in_w * k.channels) % 4 != 0 || (k.out_w * k.channels) % 4 != 0) return -1;
-    if (k.in_pitch % 16 != 0 || k.out_pitch % 4 != 0) return -1;
-    if ((reinterpret_cast<uintptr_t>(k.in) & 15) != 0 || (reinterpret_cast<uintptr_t>(k.out) & 3) != 0) return -1;
-    if (k.n_frames > 1 && (k.in_frame_stride % 16 != 0 || k.out_frame_stride % 4 != 0)) return -1;
-    if (!t.i0x_host) return -1;
+    if (!strip_layout_ok(k) || !t.i0x_host) return -1;
     const int mode = (k.flags & LANCZOS_FLAG_TOLERANCE_1LSB) ? 1 : 0;
     const int C = k.channels, A = k.a, N = k.scale_n, D = k.scale_d;
 #define LZD_CASE(c, a, n, d, id)                                                   \

@@ -35,7 +35,6 @@
 #include <algorithm>
 #include <atomic>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <type_traits>
 #include <cuda.h>
@@ -43,38 +42,14 @@
 #include "../../include/lanczos_b200.h"
 #include "fast_common.cuh"
 
-#ifndef LZB_HROUNDS
-#define LZB_HROUNDS 2     // H rounds (of 32 / MAX_GROUPS = 5 rows) per chunk
-#endif
-#ifndef LZB_MINB
-#define LZB_MINB 16      // resident warps per SM the register allocation aims for
-#endif
-#ifndef LZB_TOL_VU
-#define LZB_TOL_VU 1     // ratio periods per V loop iteration in MODE 1 at D = 1 (2: +2 % on 1080p, -5 % on 4K)
-#endif
-#ifndef LZB_VCOLD_W
-#define LZB_VCOLD_W 4    // byte-columns per pass of the V pass's phase-0 second look (4 or 8)
-#endif
-#ifndef LZB_NOISY_AFTER
-#define LZB_NOISY_AFTER 2   // flagged chunks in a row after which a warp stops filtering phase-0 rows (huge = never)
-#endif
-#ifndef LZB_W
-#define LZB_W 1          // independent warps (strips) per CTA
-#endif
-
 namespace lzb {
 
 namespace {
 
-struct V6Params {
-    uint8_t *out;         // output row `out_row0` of frame 0
-    long long out_pitch, out_frame_stride;
-    int in_w, in_h, out_w, out_h;
-    int out_row0, out_rows, in_row0, in_rows;
-    int sw;               // strip width in output bytes (groups * OUT_B)
-    int groups;           // H-pass thread groups per strip row
-    int seg_periods;      // vertical ratio-periods per segment
-    int vperiod0;         // first vertical period covered by the launch (floor(out_row0 / N))
+// strict_counter leads so that every other field keeps the constant-bank offset mod 16 of the layout the kernel was
+// tuned with: with other orders ptxas gave some instances one register and a few instructions more or less.
+struct V6Params : StripParams {
+    unsigned long long *strict_counter;
     const double *wdx, *wdy;  // per-coordinate double weights (exact recomputation, non-uniform phases)
     float guard_h, guard_v;   // rigorous fp32 error bounds (x1.05) of the two summation orders
     int uniform_x, uniform_y; // double weights identical for all coordinates of a phase -> wdtab usable
@@ -87,17 +62,13 @@ struct V6Params {
     float p0c[5];
     float wtab[32 * 8];       // polyphase table [N][8] (padded to 8 taps), N <= 32, times 2^24
     double wdtab[8 * 8];      // double polyphase table [N][8] for N <= 8 (valid when uniform_*)
-    unsigned long long *strict_counter;
 };
 
-__host__ __device__ constexpr int cdiv6(int a, int b) { return (a + b - 1) / b; }
 __host__ __device__ constexpr int cmax6(int a, int b) { return a > b ? a : b; }
-__host__ __device__ constexpr int lcm2(int d) { return d % 2 == 0 ? d : 2 * d; }
 __host__ __device__ constexpr int gcd6(int a, int b) { return b == 0 ? a : gcd6(b, a % b); }
 
-template <int C, int A, int N, int D, int PH, int W, int MODE>
+template <int C, int A, int N, int D, int PH, int MODE>
 struct Geo6 {
-    static constexpr int THREADS = 32 * W;              // W independent warps per CTA, one strip each
     static constexpr int VB = 8;                        // byte-columns per V thread
     static constexpr int TAPS = 2 * A;
     static constexpr int IN_B = PH * D * C;             // input bytes owned by one H item
@@ -121,23 +92,19 @@ struct Geo6 {
     // (+7 % on uniform noise in that mode, measured; +-0 on image-like content)
     static constexpr int SWV = (MODE == 1) ? 5 * OUT_B : 32 * VB;
     static constexpr int VOFF_MAX = OUT_B - gcd6(SWV, OUT_B);     // largest offset of a strip inside its first H item
-    static constexpr int MAX_GROUPS = cdiv6(VOFF_MAX + SWV, OUT_B);   // H items per row of a warp's strip (6 for 48-byte items)
+    static constexpr int MAX_GROUPS = cdiv(VOFF_MAX + SWV, OUT_B);   // H items per row of a warp's strip (6 for 48-byte items)
     static constexpr int SW_MAX = MAX_GROUPS * OUT_B;             // ring pitch in bytes (288)
     // a TMA box must start on a 16-byte boundary of the row: strips whose input starts 8 bytes off get a box
     // that starts 8 bytes early (XSHIFT_MAX extra bytes per row)
     static constexpr int XSHIFT_MAX = (IN_B % 16 != 0) ? 8 : 0;   // H items start at multiples of IN_B input bytes
-    static constexpr int BOX_B = 16 * cdiv6(XSHIFT_MAX + cmax6(PAD_L + MAX_GROUPS * IN_B + HALO_R, WIN0 + (MAX_GROUPS - 1) * IN_B + 8 * NW2), 16);
+    static constexpr int BOX_B = 16 * cdiv(XSHIFT_MAX + cmax6(PAD_L + MAX_GROUPS * IN_B + HALO_R, WIN0 + (MAX_GROUPS - 1) * IN_B + 8 * NW2), 16);
     static constexpr int HB = 32 / MAX_GROUPS;                    // rows one round of H items covers (one item per lane)
-    static constexpr int HROUNDS = LZB_HROUNDS;                   // H rounds per chunk
+    static constexpr int HROUNDS = 2;                             // H rounds per chunk
     static constexpr int RB = HB * HROUNDS;                       // input rows per chunk
     static constexpr int REGIONS = 2;                             // ring regions of RB rows: V(c) reads region c and the tail of c-1
     static constexpr int RING = REGIONS * RB;                     // intermediate rows kept in smem
     static constexpr int STAGE_B = 128 * ((RB * BOX_B + 127) / 128);  // TMA destinations must be 128-byte aligned
-#ifdef LZB_STAGES
-    static constexpr int STAGES = LZB_STAGES;
-#else
-    static constexpr int STAGES = HROUNDS > 1 ? 3 : 4;            // TMA stages in flight
-#endif
+    static constexpr int STAGES = 3;                              // TMA stages in flight
     // the first row pushed by a segment is rs = D*pv0 - A + 1, so (row - A) mod D is static per chunk row
     static constexpr int S0 = (((1 - 2 * A) % D) + D) % D;
     static constexpr int U = lcm2(D);                             // rows per V loop iteration (even: filter delay line parity)
@@ -150,31 +117,13 @@ struct Geo6 {
     static_assert(BOX_B / 4 <= 256, "TMA box too wide");
     static_assert(N <= 32, "phase table too large for kernel params");
     static_assert(YROWS + N * (S0 + A + 1) / D + 2 <= 64, "fix mask (bit per output row) too small");
-    static_assert(cdiv6(S0 * N, D) + YROWS <= 32, "rows fixed per chunk must fit 32 bits");
+    static_assert(cdiv(S0 * N, D) + YROWS <= 32, "rows fixed per chunk must fit 32 bits");
     static_assert(ND <= 31, "H fix mask (bit per packed word) too small");
     static_assert(D <= 2, "phase-0 filter delay line assumes the +-2 rows are phase-0 centres themselves");
 };
 
-// residue s of a completing centre (c = D*t + s): its output rows are N*t + [ylo, yhi)
-template <int N, int D> __host__ __device__ constexpr int ylo6(int s) { return cdiv6(s * N, D); }
-template <int N, int D> __host__ __device__ constexpr int yhi6(int s) { return cdiv6((s + 1) * N, D); }
-template <int N, int D> __host__ __device__ constexpr int cnt6(int s) {   // interpolated (phase != 0) rows among them
-    int n = 0;
-    for (int yr = ylo6<N, D>(s); yr < yhi6<N, D>(s); yr++) n += ((yr * D) % N != 0) ? 1 : 0;
-    return n;
-}
-template <int N, int D, int TAPS> __host__ __device__ constexpr int nslot6() {   // partial sums alive while a row is processed
-    int best = 0;
-    for (int s0 = 0; s0 < D; s0++) {
-        int n = 0;
-        for (int dc = 0; dc < TAPS; dc++) n += cnt6<N, D>((s0 + dc) % D);
-        best = n > best ? n : best;
-    }
-    return best;
-}
-
 template <class G>
-struct __align__(128) Smem6 {             // one per warp
+struct __align__(128) Smem6 {             // one per CTA
     uint8_t in[G::STAGES][G::STAGE_B];    // TMA destinations, row lr at lr * BOX_B
     uint8_t ring[G::RING][G::SW_MAX];     // H-pass results (uint8), row r lives in slot (r - rs) % RING
     unsigned long long full[G::STAGES];   // TMA stage filled
@@ -225,12 +174,6 @@ __device__ __forceinline__ uint32_t quantise_f32(float x) {
 
 // summation order of the H-pass chains: outermost (smallest) weights first, the two central taps last
 template <int TAPS> __host__ __device__ constexpr int tap_order6(int i) { return (i & 1) ? TAPS - 1 - i / 2 : i / 2; }
-
-__device__ __forceinline__ uint32_t hfma2_u(uint32_t a, uint32_t b, uint32_t c) {
-    uint32_t d;
-    asm("fma.rn.f16x2 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
-    return d;
-}
 
 // Phase-0 second look (a = 3): the reference's double sum b0*w0 + b1*w1 + v + b3*w3 + b4*w4 (full_TB.h:58-63 /
 // :71-75 at a coordinate that falls on an input sample; ascending taps, tap 5 never changes it) restated in fp32.
@@ -342,7 +285,7 @@ __device__ __forceinline__ uint32_t exact_ring(uint32_t col_e, int slot0, W weig
 // the reference's double arithmetic gives (full_TB.h:71-75), and stores it again (same lane, program order).
 template <int A, int N, int D, int VU, int S0> __host__ __device__ constexpr int viter_interp_rows() {
     int n = 0;
-    for (int u = 0; u < VU; u++) n += cnt6<N, D>((S0 + u) % D);
+    for (int u = 0; u < VU; u++) n += cnt<N, D>((S0 + u) % D);
     return n;
 }
 template <int A, int N, int D, int VU, int S0> __host__ __device__ constexpr int viter_centre_rows() {
@@ -466,7 +409,7 @@ __device__ __noinline__ int v_fix_iter(const V6Params &p, uint32_t col, int slot
     for (int u = 0; u < VU; u++) {
         const int s0 = (S0 + u) % D, tq = (S0 + u) / D;
 #pragma unroll
-        for (int yr = ylo6<N, D>(s0); yr < yhi6<N, D>(s0); yr++) {
+        for (int yr = ylo<N, D>(s0); yr < yhi<N, D>(s0); yr++) {
             if ((yr * D) % N == 0) continue;
             if ((f.dx[qi] | f.dy[qi]) != 0u) {
                 const uint32_t need = (lsb4_to_bits(f.dx[qi]) | (lsb4_to_bits(f.dy[qi]) << 4)) & vmask;
@@ -534,31 +477,29 @@ __device__ __noinline__ void alias_fix(const V6Params &p, const AliasArgs a) {
     }
 }
 
-template <int C, int A, int N, int D, int PH, int KM, int W, int MODE, bool ST64>
-__global__ void __launch_bounds__(32 * W, LZB_MINB / W)
+// one warp per CTA, 16 resident per SM: the register allocation aims for 128 per thread
+template <int C, int A, int N, int D, int PH, int KM, int MODE, bool ST64>
+__global__ void __launch_bounds__(32, 16)
 lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ V6Params p) {
-    using G = Geo6<C, A, N, D, PH, W, MODE>;
+    using G = Geo6<C, A, N, D, PH, MODE>;
     constexpr int TAPS = G::TAPS;
     constexpr int SWM = G::SW_MAX;
     constexpr int VB = G::VB;
     constexpr int CEN = A - 1;                                  // centre tap of a phase-0 sample
-    constexpr int NSLOT = nslot6<N, D, TAPS>();
-    constexpr int CNTMAX = cmax6(1, cmax6(cnt6<N, D>(0), cnt6<N, D>(D - 1)));   // D <= 2
+    constexpr int NSLOT = nslot<N, D, TAPS>();
+    constexpr int CNTMAX = cntmax<N, D>();
 #ifdef LZB_ABL_NOVFILTER     // ablation builds (timing experiments only, results are wrong): see tools/ablate.sh
     constexpr bool FILTER = false;
 #else
     constexpr bool FILTER = (MODE == 0) && (KM != 0);
 #endif
-    // input rows per V loop iteration: one (even) ratio period.  LZB_TOL_VU = 2 lets the plain fp32 V pass of MODE 1
-    // take two of them at D = 1: +2 % on 1080p batches, -5 % on 4K ones (measured), so it stays off.
-    constexpr int VU = (MODE == 1 && D == 1 && G::RB % (LZB_TOL_VU * G::U) == 0) ? LZB_TOL_VU * G::U : G::U;
+    // input rows per V loop iteration: one (even) ratio period (two in MODE 1 at D = 1 measured +2 % on 1080p, -5 % on 4K)
+    constexpr int VU = G::U;
     static_assert(KM == 0 || (A == 3 && KM == 0x11), "phase-0 row filter is written for the +-2 residues of a = 3");
     extern __shared__ __align__(128) uint8_t smem_raw[];
-    // every warp works on its own strip with its own TMA stages, ring and barriers: nothing is shared between
-    // the warps of a CTA, so there is no CTA-wide synchronisation anywhere
-    const int tid = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    Smem6<G> &sm = reinterpret_cast<Smem6<G> *>(smem_raw)[warp];
-    const int strip = blockIdx.x * W + warp, seg = blockIdx.y, frame = blockIdx.z;
+    Smem6<G> &sm = *reinterpret_cast<Smem6<G> *>(smem_raw);
+    const int tid = threadIdx.x;
+    const int strip = blockIdx.x, seg = blockIdx.y, frame = blockIdx.z;
     // programmatic dependent launch: let the next kernel of the stream start as soon as SMs free up; unless the caller
     // declared the frames independent, wait here until everything before this kernel on the stream has completed
     // (both are no-ops for a launch without the attribute)
@@ -842,7 +783,7 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
 #pragma unroll
                 for (int u = 0; u < VU; u++) {
                     const int s0 = (G::S0 + u) % D, tq = (G::S0 + u) / D;   // completing centre = D*(t + tq) + s0
-                    const int cnt0 = cnt6<N, D>(s0);
+                    const int cnt0 = cnt<N, D>(s0);
                     const uint2 w = *reinterpret_cast<const uint2 *>(vit + u * SWM);
                     const uint32_t h0 = __byte_perm(w.x, 0u, 0x4140), h1 = __byte_perm(w.x, 0u, 0x4342);
                     const uint32_t h2 = __byte_perm(w.y, 0u, 0x4140), h3 = __byte_perm(w.y, 0u, 0x4342);
@@ -863,13 +804,12 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
                             const int sdc = (s0 + dc) % D;
                             const int k = TAPS - 1 - dc;
 #pragma unroll
-                            for (int yr = ylo6<N, D>(sdc); yr < yhi6<N, D>(sdc); yr++) {
+                            for (int yr = ylo<N, D>(sdc); yr < yhi<N, D>(sdc); yr++) {
                                 const int ph = (yr * D) % N;
                                 if (ph == 0) continue;
 #ifdef LZB_ABL_TAPS             // ablation: only the first and the last LZB_ABL_TAPS/2 taps are computed
                                 if (dc >= LZB_ABL_TAPS / 2 && dc < TAPS - LZB_ABL_TAPS / 2) { q++; continue; }
 #endif
-#ifndef LZB_V_SCALAR
                                 // two columns per FFMA2 (one issue slot for two FMAs; same rounding as two FFMAs)
                                 const float2 wk2 = make_float2(p.wtab[ph * 8 + k], p.wtab[ph * 8 + k]);
 #pragma unroll
@@ -880,15 +820,6 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
                                     if (dc == 0) { res[q][i] = r2.x; res[q][i + 1] = r2.y; }
                                     else { acc[q - cnt0][i] = r2.x; acc[q - cnt0][i + 1] = r2.y; }
                                 }
-#else
-#pragma unroll
-                                for (int i = 0; i < VB; i++) {
-                                    const float wk = p.wtab[ph * 8 + k];
-                                    if (dc == 0) res[q][i] = fmaf(x[i], wk, acc[q][i]);
-                                    else if (dc < TAPS - 1) acc[q - cnt0][i] = fmaf(x[i], wk, acc[q][i]);
-                                    else acc[q - cnt0][i] = fmaf(x[i], wk, -guard_v);
-                                }
-#endif
                                 q++;
                             }
                         }
@@ -926,8 +857,8 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
                             qv.y = __byte_perm(zA[zs][2], zA[zs][3], 0x6420);
 #pragma unroll
                             for (int i = 0; i < VB / 2; i++) {
-                                zpost |= hfma2_u(hn[i], kR, zA[zs][i]);
-                                zpre |= hfma2_u(zA[zs][i], kR, hn[i]);
+                                zpost |= hfma2(hn[i], kR, zA[zs][i]);
+                                zpre |= hfma2(zA[zs][i], kR, hn[i]);
                                 zA[zs][i] = hn[i];
                             }
                             // (rows outside [ys, ye) -- warm-up rows, rows of the next segment -- are never stored: no second look)
@@ -943,7 +874,7 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
                     {
                         int q = 0;
 #pragma unroll
-                        for (int yr = ylo6<N, D>(s0); yr < yhi6<N, D>(s0); yr++) {
+                        for (int yr = ylo<N, D>(s0); yr < yhi<N, D>(s0); yr++) {
                             const int ph = (yr * D) % N;
                             if (ph == 0) continue;
                             uint2 qv;
@@ -997,6 +928,7 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
     };
 
     // ------------------------------ pipeline ------------------------------
+    constexpr int kNoisyAfter = 2;     // flagged chunks in a row after which a warp stops filtering phase-0 rows
     bool noisy = false;
     int flagged_run = 0;
     for (int chunk = 0; chunk < nchunks; chunk++) {
@@ -1019,7 +951,7 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
         if constexpr (FILTER) {
             if (!noisy) {
                 flagged_run = __any_sync(0xffffffffu, flagged) ? flagged_run + 1 : 0;
-                noisy = flagged_run >= LZB_NOISY_AFTER;
+                noisy = flagged_run >= kNoisyAfter;
             }
         }
 #endif
@@ -1038,88 +970,54 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-template <int C, int A, int N, int D, int PH, int KM, int W, int MODE, bool ST64>
+// Vertical segments of a launch over vperiods ratio periods, cols = strips x frames CTA columns and slots resident CTAs
+// (one warp each) on sms SMs.  Every segment re-runs 2a-1 warm-up rows and works in whole chunks of RB rows, and the
+// time of a chunk depends on how many warps share an SM sub-partition: measured on 1080p->2160p single frames
+// (segment-count sweep, B200) it is ~(1.6 + 1.7 w) us for w = 1..4 resident warps -- two warps already reach 92 % of
+// the issue rate of four.  Small jobs minimise chunks x sum over waves of that time; batches, which run many waves,
+// minimise waves x rows per segment (plan_segments).
+SegPlan plan_v6_segments(int vperiods, int D, int A, int RB, long long cols, long long slots, int sms, bool independent) {
+    constexpr int kMaxSegs = 256;
+    if (cols * 4 > slots) return plan_segments(vperiods, D, A, RB, cols, slots, kMaxSegs);
+    // small job (a frame or a few): everything is resident at once, latency counts
+    const int max_segs = max_segments(vperiods, D, RB);
+    int segs;
+    if (independent) {
+        // LANCZOS_FLAG_INDEPENDENT: successive small launches of a stream overlap like the frames of a batch, so what
+        // counts is throughput, not the latency of one launch: about four launches' worth of warps resident at a time
+        // (measured on 1080p single frames, profiles/r02b_segs_independent.txt: 13 segments 11.6 us per frame,
+        // 27 segments -- what the latency model picks -- 13.3 us, 3 segments 16.2 us)
+        segs = std::max(1, std::min(max_segs, (int)std::lround((double)slots / (4.0 * (double)cols))));
+    } else {
+        auto chunk_time = [&](double warps) { return 1.6 + 1.7 * std::max(1.0, warps / (4.0 * sms)); };
+        segs = cheapest_segments(vperiods, max_segs, kMaxSegs, [&](int per, int sg) {
+            const double chunks = std::ceil((double)(per * D + 2 * A - 1) / RB);
+            const long long ctas = cols * sg;
+            const long long full_waves = ctas / slots, rem = ctas - full_waves * slots;
+            return chunks * ((double)full_waves * chunk_time((double)slots) + (rem > 0 ? chunk_time((double)rem) : 0.0));
+        });
+    }
+    return split_periods(vperiods, segs);
+}
+
+template <int C, int A, int N, int D, int PH, int KM, int MODE, bool ST64>
 int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kernel, cudaStream_t s) {
-    using G = Geo6<C, A, N, D, PH, W, MODE>;
-    EncodeFn encode = get_encode();
-    if (!encode) return -1;
-    const int row_bytes = k.out_w * C;
-    // one strip of SWV = 256 output bytes per warp
-    const int sw = G::SWV;
-    const int strips = (row_bytes + sw - 1) / sw;
+    using G = Geo6<C, A, N, D, PH, MODE>;
+    CUtensorMap map;
+    if (!encode_input_map(&map, k, G::BOX_B, G::RB)) return -1;
+    auto kern = lanczos_v6_kernel<C, A, N, D, PH, KM, MODE, ST64>;
+    const size_t smem = sizeof(Smem6<G>) + 128;
+    static std::atomic<int> ctas_per_sm[64] = {};
+    const Residency res = resident_ctas(ctas_per_sm, kern, smem);
+    if (res.ctas == 0) return -1;
+    const int strips = (k.out_w * C + G::SWV - 1) / G::SWV;   // one strip of SWV = 256 output bytes per warp
+    const long long cols = (long long)strips * k.n_frames;
     const int vperiod0 = k.out_row0 / N;
     const int vperiods = (k.out_row0 + k.out_rows + N - 1) / N - vperiod0;
-    // Vertical segments: every segment re-runs 2a-1 warm-up rows and works in whole chunks of RB rows, and the
-    // time of a chunk depends on how many warps share an SM sub-partition: measured on 1080p->2160p single
-    // frames (LZB_SEGS sweep, B200) it is ~(1.6 + 1.7 w) us for w = 1..4 resident warps -- two warps already
-    // reach 92 % of the issue rate of four.  Small jobs minimise chunks x sum over waves of that time; batches,
-    // which run many waves, minimise waves x rows per segment.
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    auto kern = lanczos_v6_kernel<C, A, N, D, PH, KM, W, MODE, ST64>;
-    const size_t smem = W * sizeof(Smem6<G>) + 128;
-    // per device, set once; the calls are idempotent, so two threads racing here only repeat them
-    static std::atomic<int> ctas_per_sm[64] = {};
-    if (ctas_per_sm[dev & 63].load(std::memory_order_acquire) == 0) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) { cudaGetLastError(); return -1; }   // clear the error state: the caller falls back to another kernel
-        int nb = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, 32 * W, smem) != cudaSuccess || nb < 1) nb = 4;
-        ctas_per_sm[dev & 63].store(nb, std::memory_order_release);
-    }
-    const long long slots = (long long)ctas_per_sm[dev & 63].load(std::memory_order_relaxed) * sms * W;      // resident warps = strips in flight
-    const long long cols = (long long)strips * k.n_frames;
-    const int max_segs = std::max(1, vperiods / std::max(1, (2 * G::RB) / D));
-    int segs = 1;
-    double best_cost = 1e300;
-    static const int force_segs = [] { const char *e = getenv("LZB_SEGS"); return e ? atoi(e) : 0; }();
-    for (int sg = 1; sg <= std::min(max_segs, 256); sg++) {
-        const int per = (vperiods + sg - 1) / sg;
-        const int sg_eff = (vperiods + per - 1) / per;
-        double cost;
-        if (cols * 4 <= slots) {
-            // small job (a frame or a few): everything is resident at once, latency counts
-            const double chunks = std::ceil((double)(per * D + 2 * A - 1) / G::RB);
-            const long long ctas = cols * sg_eff;
-            const long long full_waves = ctas / slots, rem = ctas - full_waves * slots;
-            auto chunk_time = [&](double warps) { return 1.6 + 1.7 * std::max(1.0, warps / (4.0 * sms)); };
-            cost = chunks * ((double)full_waves * chunk_time((double)slots) + (rem > 0 ? chunk_time((double)rem) : 0.0));
-        } else {
-            // batch: (waves) x (rows per segment + warm-up + pipeline fill); a wave that is not full still costs a
-            // full wave unless it is the only one
-            const double rows = (double)per * D + 2 * A - 1 + 0.5 * G::RB;
-            const double waves = std::ceil((double)(cols * sg_eff) / (double)slots);
-            cost = (cols * sg_eff <= slots) ? rows * 1.0 : rows * waves;
-        }
-        if (cost < best_cost - 1e-9) { best_cost = cost; segs = sg_eff; }
-    }
-    // LANCZOS_FLAG_INDEPENDENT: successive small launches of a stream overlap like the frames of a batch, so what counts
-    // is throughput, not the latency of one launch: about four launches' worth of warps resident at a time (measured on
-    // 1080p single frames, profiles/r02b_segs_independent.txt: 13 segments 11.6 us per frame, 27 segments -- what the
-    // latency model picks -- 13.3 us, 3 segments 16.2 us)
-    if ((k.flags & LANCZOS_FLAG_INDEPENDENT) && cols * 4 <= slots)
-        segs = std::max(1, std::min(max_segs, (int)std::lround((double)slots / (4.0 * (double)cols))));
-    if (force_segs > 0) segs = std::min(force_segs, max_segs);
-    int seg_periods = (vperiods + segs - 1) / segs;
-    segs = (vperiods + seg_periods - 1) / seg_periods;
-
-    CUtensorMap map;
-    const cuuint64_t dims[3] = {(cuuint64_t)(k.in_w * C / 4), (cuuint64_t)k.in_rows, (cuuint64_t)k.n_frames};
-    const cuuint64_t strides[2] = {(cuuint64_t)k.in_pitch, (cuuint64_t)(k.n_frames > 1 ? k.in_frame_stride : k.in_pitch * k.in_rows)};
-    const cuuint32_t box[3] = {(cuuint32_t)(G::BOX_B / 4), (cuuint32_t)G::RB, 1};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    if (encode(&map, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, const_cast<uint8_t *>(k.in), dims, strides, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return -1;
+    const SegPlan sp = plan_v6_segments(vperiods, D, A, G::RB, cols, res.ctas, res.sms, (k.flags & LANCZOS_FLAG_INDEPENDENT) != 0);
 
     V6Params p{};
-    p.out = k.out;
-    p.out_pitch = k.out_pitch;
-    p.out_frame_stride = k.out_frame_stride;
-    p.in_w = k.in_w; p.in_h = k.in_h; p.out_w = k.out_w; p.out_h = k.out_h;
-    p.out_row0 = k.out_row0; p.out_rows = k.out_rows; p.in_row0 = k.in_row0; p.in_rows = k.in_rows;
-    p.sw = sw; p.groups = G::MAX_GROUPS; p.seg_periods = seg_periods; p.vperiod0 = vperiod0;
+    set_strip_params(p, k, vperiod0, sp.seg_periods);
     p.wdx = k.wdx; p.wdy = k.wdy;
     p.guard_h = k.guard_outer; p.guard_v = k.guard_asc;
     p.uniform_x = t.uniform_x; p.uniform_y = t.uniform_y;
@@ -1135,18 +1033,17 @@ int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kerne
     }
     for (int i = 0; i < 8; i++) p.align_k[i] = i < 2 * A ? t.align_k[i] : 0.f;
     for (int i = 0; i < 5; i++) p.p0c[i] = t.p0_chain ? t.p0_chain[i] * 16777216.f : 0.f;   // x 2^24, exact
-    for (int ph = 0; ph < N; ph++)
-        for (int q = 0; q < 8; q++) p.wtab[ph * 8 + q] = q < 2 * A ? t.phase_w[ph * 2 * A + q] * 16777216.f : 0.f;  // x 2^24, see kPixUnscale
+    fill_wtab(p.wtab, t, A, N);
     for (int ph = 0; ph < N && ph < 8; ph++)
         for (int q = 0; q < 8; q++) p.wdtab[ph * 8 + q] = q < 2 * A ? t.phase_wd[ph * 2 * A + q] : 0.0;
     p.strict_counter = k.strict_counter;
 
-    dim3 grid((strips + W - 1) / W, segs, k.n_frames);
+    dim3 grid(strips, sp.segs, k.n_frames);
     p.independent = (k.flags & LANCZOS_FLAG_INDEPENDENT) ? 1 : 0;
     if (p.independent) {
         cudaLaunchConfig_t cfg{};
         cfg.gridDim = grid;
-        cfg.blockDim = dim3(32 * W);
+        cfg.blockDim = dim3(32);
         cfg.dynamicSmemBytes = smem;
         cfg.stream = s;
         cudaLaunchAttribute attr{};
@@ -1156,7 +1053,7 @@ int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kerne
         cfg.numAttrs = 1;
         return (int)cudaLaunchKernelEx(&cfg, kern, map, p);
     }
-    kern<<<grid, 32 * W, smem, s>>>(map, p);
+    kern<<<grid, 32, smem, s>>>(map, p);
     return (int)cudaGetLastError();
 }
 
@@ -1164,11 +1061,8 @@ int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kerne
 
 // Returns 0 on launch, >0 cudaError, -1 when no specialised kernel applies (caller falls back).
 int launch_v6(const KParams &k, const FastHostTables &t, int *kernel_id, int *alias_in_kernel, cudaStream_t s) {
-    // layout requirements of the TMA map and of the 32-bit/64-bit/128-bit accesses
-    if ((k.in_w * k.channels) % 4 != 0 || (k.out_w * k.channels) % 4 != 0) return -1;
-    if (k.in_pitch % 16 != 0 || k.out_pitch % 4 != 0) return -1;
-    if ((reinterpret_cast<uintptr_t>(k.in) & 15) != 0 || (reinterpret_cast<uintptr_t>(k.out) & 3) != 0) return -1;
-    if (k.n_frames > 1 && (k.in_frame_stride % 16 != 0 || k.out_frame_stride % 4 != 0)) return -1;
+    if (!strip_layout_ok(k)) return -1;
+    // 64-bit stores of the V pass
     const bool st64 = (k.out_w * k.channels) % 8 == 0 && k.out_pitch % 8 == 0 && (reinterpret_cast<uintptr_t>(k.out) & 7) == 0 &&
                       (k.n_frames <= 1 || k.out_frame_stride % 8 == 0);
     if (!t.exact_x || !t.exact_y) return -1;     // phase-0 coordinates not exactly integral in double: other kernels
@@ -1184,10 +1078,10 @@ int launch_v6(const KParams &k, const FastHostTables &t, int *kernel_id, int *al
 #define LZ6_CASE(c, a, n, d, ph, kmask, id)                                                            \
     if (C == c && A == a && N == n && D == d && km == (kmask)) {                                        \
         *kernel_id = id;                                                                                \
-        if (mode == 0) return st64 ? launch_v6_one<c, a, n, d, ph, kmask, LZB_W, 0, true>(k, t, alias_in_kernel, s)         \
-                                   : launch_v6_one<c, a, n, d, ph, kmask, LZB_W, 0, false>(k, t, alias_in_kernel, s);       \
-        return st64 ? launch_v6_one<c, a, n, d, ph, kmask, LZB_W, 1, true>(k, t, alias_in_kernel, s)                        \
-                    : launch_v6_one<c, a, n, d, ph, kmask, LZB_W, 1, false>(k, t, alias_in_kernel, s);                      \
+        if (mode == 0) return st64 ? launch_v6_one<c, a, n, d, ph, kmask, 0, true>(k, t, alias_in_kernel, s)         \
+                                   : launch_v6_one<c, a, n, d, ph, kmask, 0, false>(k, t, alias_in_kernel, s);       \
+        return st64 ? launch_v6_one<c, a, n, d, ph, kmask, 1, true>(k, t, alias_in_kernel, s)                        \
+                    : launch_v6_one<c, a, n, d, ph, kmask, 1, false>(k, t, alias_in_kernel, s);                      \
     }
     // the phase-0 second look is the exact fp32 chain (phase0_chain2): only with plan.cpp's proof for these weights
     if (km != 0 && !t.p0_chain) return -1;
