@@ -101,9 +101,9 @@ struct HlsGeo {
 // de-ring clamp of worker.cpp:66-74 / :103-111
 __device__ __forceinline__ int dering(int acc, int c0, int c1) { return max(min(c0, c1), min(acc, max(c0, c1))); }
 
-// MASK >= 0: the LUT is known to hold 2^BP at distance 0 and, at the other whole-pixel distances N*k, -1 where bit
-// k of MASK is set and 0 elsewhere (floor of the +-1e-17 residues of L(k), kernel.cpp:40-45): samples that sit on an
-// input sample then need a shift and a subtraction or two instead of 2a multiplications.  MASK < 0: no assumption.
+// The LUT is known to hold 2^BP at distance 0 and, at the other whole-pixel distances N*k, -1 where bit k of MASK is
+// set and 0 elsewhere (floor of the +-1e-17 residues of L(k), kernel.cpp:40-45; launch_hls_tile checks it): samples
+// that sit on an input sample then need a shift and a subtraction or two instead of 2a multiplications.
 template <int C, int A, int N, int MASK>
 __global__ void __launch_bounds__(256) lanczos_hls_tile_kernel(const __grid_constant__ HlsParams p) {
     using G = HlsGeo<C, A, N>;
@@ -145,7 +145,7 @@ __global__ void __launch_bounds__(256) lanczos_hls_tile_kernel(const __grid_cons
                 for (int j = 0; j < TAPS; j++) {
                     const int dist = r - (j - A + 1) * N;           // y - row * N
                     const int k = (j - A + 1) < 0 ? -(j - A + 1) : (j - A + 1);
-                    if (MASK >= 0 && r == 0) {
+                    if (r == 0) {
                         if (k == 0) acc += win[j] << BP;
                         else if ((MASK >> k) & 1) acc -= win[j];
                     } else {
@@ -182,7 +182,7 @@ __global__ void __launch_bounds__(256) lanczos_hls_tile_kernel(const __grid_cons
                 const int dist = r - (j - A + 1) * N;               // x - col * N
                 const int k = (j - A + 1) < 0 ? -(j - A + 1) : (j - A + 1);
                 const int v = mid[(base + j) * C + c];
-                if (MASK >= 0 && r == 0) {
+                if (r == 0) {
                     if (k == 0) acc += v;                           // (2^BP * v) >> BP
                     else if ((MASK >> k) & 1) acc += (-v) >> BP;    // (-1 * v) >> BP, arithmetic shift = floor
                 } else {
@@ -203,15 +203,16 @@ __global__ void __launch_bounds__(256) lanczos_hls_tile_kernel(const __grid_cons
     }
 }
 
+// Returns -1 without launching when the LUT lacks the whole-pixel pattern the MASK instance assumes (the caller then
+// runs lanczos_hls_kernel).  The library's own LUT always has it for the configurations below.
 template <int C, int A, int N, int MASK>
 int launch_hls_tile(const HlsParams &p, int n_frames, cudaStream_t s) {
     using G = HlsGeo<C, A, N>;
-    dim3 grid((p.out_w + G::TW - 1) / G::TW, (p.out_h + G::TH - 1) / G::TH, n_frames);
-    // does the LUT have the whole-pixel pattern the MASK instance assumes?
     bool pattern = p.lut[0] == (1 << 8);
     for (int k = 1; k <= A; k++) pattern = pattern && p.lut[k * N] == (((MASK >> k) & 1) ? -1 : 0);
-    if (pattern) lanczos_hls_tile_kernel<C, A, N, MASK><<<grid, 256, 0, s>>>(p);
-    else lanczos_hls_tile_kernel<C, A, N, -1><<<grid, 256, 0, s>>>(p);
+    if (!pattern) return -1;
+    dim3 grid((p.out_w + G::TW - 1) / G::TW, (p.out_h + G::TH - 1) / G::TH, n_frames);
+    lanczos_hls_tile_kernel<C, A, N, MASK><<<grid, 256, 0, s>>>(p);
     return (int)cudaGetLastError();
 }
 
@@ -227,9 +228,14 @@ int launch_hls(const uint8_t *in, uint8_t *out, long long in_pitch, long long ou
     for (int i = 0; i <= a * n; i++) p.lut[i] = lut[i];
     if (bp == 8) {      // 16-bit intermediates: the tiled kernel (the reference's template BIT_PRECISION is 8)
         // a = 3: floor(L(2) * 2^BP) = -1 (sin(2 pi) < 0 in double), the other whole-pixel entries are 0; a = 2: all 0
-#define HLS_CASE(c, aa, nn, mask) if (channels == c && a == aa && n == nn) { *kernel_id = 101; return launch_hls_tile<c, aa, nn, mask>(p, n_frames, s); }
+        int rc = -1;
+#define HLS_CASE(c, aa, nn, mask) if (channels == c && a == aa && n == nn) rc = launch_hls_tile<c, aa, nn, mask>(p, n_frames, s);
         HLS_CASE(3, 3, 2, 4) HLS_CASE(4, 3, 2, 4) HLS_CASE(1, 3, 2, 4) HLS_CASE(3, 2, 2, 0) HLS_CASE(3, 3, 4, 4) HLS_CASE(3, 2, 4, 0)
 #undef HLS_CASE
+        if (rc >= 0) {
+            *kernel_id = 101;
+            return rc;
+        }
     }
     *kernel_id = 100;
     dim3 grid((out_w + HT_W - 1) / HT_W, (out_h + HT_H - 1) / HT_H, n_frames);

@@ -138,9 +138,10 @@ def axis_tables(out_len, in_len, n, d, a):
     return w, np.clip(idx, 0, in_len - 1), valid
 
 
-def restate_planar(img, out_w, out_h, a, n, d, clean):
+def restate_planar(img, out_w, out_h, a, n, d, clean, parts=False):
     """uint8 [C][H][W] -> [C][out_h][out_w]: sequential double sums in ascending taps over the clipped window, clamp,
-    truncate; rows first, then columns bottom-up in place (clean=False) or from a copy of the row pass (clean=True)."""
+    truncate; rows first, then columns bottom-up in place (clean=False) or from a copy of the row pass (clean=True).
+    parts=True returns (out, row pass [C][H][out_w] uint8, column sums [C][out_h][out_w] before quantisation)."""
     c, h, w = img.shape
     wx, ix, vx = axis_tables(out_w, w, n, d, a)
     wy, iy, vy = axis_tables(out_h, h, n, d, a)
@@ -151,14 +152,17 @@ def restate_planar(img, out_w, out_h, a, n, d, clean):
         term = src[:, :, ix[:, k]] * wx[:, k]
         s = np.where(vx[:, k], s + term, s)
     out[:, :h, :] = NT.quantise(s)
-    mid = out.copy() if clean else out
+    mid = out.copy() if clean or parts else out
+    sums = np.zeros((c, out_h, out_w)) if parts else None
     for yy in range(out_h - 1, -1, -1):
         s = np.zeros((c, out_w))
         for k in range(2 * a):
             if vy[yy, k]:
-                s = s + mid[:, iy[yy, k], :].astype(np.float64) * wy[yy, k]
+                s = s + (mid if clean else out)[:, iy[yy, k], :].astype(np.float64) * wy[yy, k]
         out[:, yy, :] = NT.quantise(s)
-    return out
+        if parts:
+            sums[:, yy, :] = s
+    return (out, mid, sums) if parts else out
 
 
 def to_planar(img):
