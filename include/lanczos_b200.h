@@ -109,6 +109,16 @@ typedef struct lanczos_stats {
     int32_t alias_rows;        /* top rows produced by the in-place emulation */
 } lanczos_stats;
 
+/* Launch shape of the last call on this host thread (for reports and tests), taken from the FIRST main-kernel launch
+ * of the call.  The host-buffer drivers run one device call per frame or band: there it describes the last of them. */
+typedef struct lanczos_launch {
+    int32_t grid_x, grid_y, grid_z;  /* gridDim of the main kernel; grid_z = frames (planes) of its frame group */
+    int32_t seg_periods;             /* ratio periods (N output rows) per vertical segment; 0 for generic and HLS kernels */
+    int32_t chunk_rows;              /* input rows per pipeline chunk of a segment; 0 for generic and HLS kernels */
+    int32_t main_launches;           /* main-kernel launches of the call: one per frame group of at most 65,535 frames */
+    int64_t resident_ctas;           /* resident CTAs of the device the segment plan assumed; 0 for generic and HLS */
+} lanczos_launch;
+
 /* ---- single frame, device buffers.
  * Replaces `void lanczos(stream_t in, stream_t out)` (lanczos.h:121-126) and its software
  * twin `lanczos_expected(byte[C][IN_H][IN_W], byte[C][OUT_H][OUT_W])` (full_TB.h:79-82).
@@ -119,7 +129,8 @@ int lanczos_b200_upscale(const lanczos_desc *desc, const uint8_t *d_in, uint8_t 
 
 /* ---- batch of independent frames with the same descriptor (BASELINE configs 3 and 4).
  * Frame f lives at d_in + f*in_frame_stride / d_out + f*out_frame_stride
- * (0 = in_pitch*in_h / out_pitch*out_h). One launch covers the whole batch. */
+ * (0 = in_pitch*in_h / out_pitch*out_h). One launch covers a group of up to 65,535 frames (CUDA's limit on a grid's
+ * y and z dimensions): larger batches run as consecutive groups on the same stream, each with its own launch. */
 int lanczos_b200_upscale_batch(const lanczos_desc *desc, const uint8_t *d_in, uint8_t *d_out,
                                int32_t n_frames, int64_t in_frame_stride,
                                int64_t out_frame_stride, int device, void *cuda_stream);
@@ -129,7 +140,8 @@ int lanczos_b200_upscale_batch(const lanczos_desc *desc, const uint8_t *d_in, ui
  * `desc->channels` = planes per frame; `in_pitch`/`out_pitch` = row pitch of a plane in bytes (0 = width).
  * Plane q (q = frame*channels + c) lives at d_in + q*in_plane_stride / d_out + q*out_plane_stride
  * (0 = pitch*height). Every plane is resampled as a one-channel image, like the reference's per-channel loops
- * (full_TB.h:83-95); one launch covers all planes of all frames. */
+ * (full_TB.h:83-95); the planes of all frames are one batch of n_frames*channels one-channel frames (grouped like
+ * lanczos_b200_upscale_batch), which must not exceed INT32_MAX (else LANCZOS_ERR_DIMS). */
 int lanczos_b200_upscale_planar(const lanczos_desc *desc, const uint8_t *d_in, uint8_t *d_out,
                                 int32_t n_frames, int64_t in_plane_stride, int64_t out_plane_stride,
                                 int device, void *cuda_stream);
@@ -225,6 +237,7 @@ int lanczos_b200_synchronize(int device);
 
 void lanczos_b200_enable_stats(int on);                 /* count strict samples (slower) */
 int lanczos_b200_get_stats(lanczos_stats *out);
+int lanczos_b200_get_launch(lanczos_launch *out);       /* read only: see lanczos_launch */
 const char *lanczos_b200_strerror(int code);
 const char *lanczos_b200_last_cuda_error(void);
 int lanczos_b200_abi_version(void);

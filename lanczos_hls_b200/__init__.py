@@ -30,6 +30,7 @@ from .api import (  # noqa: F401
     reduce_ratio,
     resolve,
     stats,
+    launch,
     enable_stats,
     upscale,
     upscale_bands_multi_gpu,

@@ -42,6 +42,12 @@ class Stats(C.Structure):
                 ("kernel_id", C.c_int32), ("alias_rows", C.c_int32)]
 
 
+class Launch(C.Structure):
+    """lanczos_launch (include/lanczos_b200.h)."""
+    _fields_ = [("grid_x", C.c_int32), ("grid_y", C.c_int32), ("grid_z", C.c_int32), ("seg_periods", C.c_int32),
+                ("chunk_rows", C.c_int32), ("main_launches", C.c_int32), ("resident_ctas", C.c_int64)]
+
+
 _lib = None
 
 
@@ -93,6 +99,7 @@ def lib():
     L.lanczos_b200_enable_stats.argtypes = [C.c_int]
     L.lanczos_b200_enable_stats.restype = None
     L.lanczos_b200_get_stats.argtypes = [C.POINTER(Stats)]
+    L.lanczos_b200_get_launch.argtypes = [C.POINTER(Launch)]
     L.lanczos_b200_strerror.argtypes = [C.c_int]
     L.lanczos_b200_strerror.restype = C.c_char_p
     L.lanczos_b200_last_cuda_error.restype = C.c_char_p
@@ -162,6 +169,13 @@ def stats():
     lib().lanczos_b200_get_stats(C.byref(s))
     return {"kernel_launches": s.kernel_launches, "strict_samples": s.strict_samples,
             "kernel_id": s.kernel_id, "alias_rows": s.alias_rows}
+
+
+def launch():
+    """Shape of the first main-kernel launch of the last call on this thread, and the number of main launches."""
+    s = Launch()
+    _check(lib().lanczos_b200_get_launch(C.byref(s)))
+    return {f: getattr(s, f) for f, _ in Launch._fields_}
 
 
 class PinnedBuffer:

@@ -28,6 +28,7 @@ namespace {
 
 thread_local std::string g_last_cuda_error;
 thread_local lanczos_stats g_stats{};
+thread_local lanczos_launch g_launch{};
 std::atomic<bool> g_stats_enabled{false};
 
 int cuda_fail(cudaError_t e, const char *what) {
@@ -262,6 +263,18 @@ struct Scratch {  // RAII device buffer from the pool (current device must be `d
 };
 
 // ---- core launch ----------------------------------------------------------------------------
+constexpr int kMaxGridFrames = 65535;
+
+// the first main launch of a call (main_launches is counted by the caller)
+void set_launch(const LaunchShape &sh) {
+    g_launch.grid_x = sh.grid_x;
+    g_launch.grid_y = sh.grid_y;
+    g_launch.grid_z = sh.grid_z;
+    g_launch.seg_periods = sh.seg_periods;
+    g_launch.chunk_rows = sh.chunk_rows;
+    g_launch.resident_ctas = sh.resident_ctas;
+}
+
 int run_device(const DevicePlan &dp, unsigned flags, const uint8_t *d_in, uint8_t *d_out, int n_frames,
                long long in_frame_stride, long long out_frame_stride, int out_row0, int out_rows,
                int in_row0, int in_rows, long long in_pitch, long long out_pitch, cudaStream_t s) {
@@ -289,6 +302,7 @@ int run_device(const DevicePlan &dp, unsigned flags, const uint8_t *d_in, uint8_
     const bool count = g_stats_enabled.load(std::memory_order_relaxed);
     p.strict_counter = count ? dp.strict_counter : nullptr;
     g_stats = lanczos_stats{};
+    g_launch = lanczos_launch{};
     if (n_frames <= 0 || out_rows <= 0) return LANCZOS_OK;
     // counting calls are synchronous and take turns on the plan's counter (several host threads or streams may share a plan)
     std::unique_lock<std::mutex> stats_lock;
@@ -297,31 +311,41 @@ int run_device(const DevicePlan &dp, unsigned flags, const uint8_t *d_in, uint8_
         CU(cudaMemsetAsync(dp.strict_counter, 0, 8, s));
     }
 
-    int kid = 0, alias_done = 0;
-    int frc = -1;
-    if (!(flags & LANCZOS_FLAG_GENERIC_KERNEL)) {
-        FastHostTables t{h.phase_w.data(), h.phase_wd.data(), h.align_k.data(), h.x.aligned_exact ? 1 : 0,
-                         h.y.aligned_exact ? 1 : 0, h.x.uniform_phase ? 1 : 0, h.y.uniform_phase ? 1 : 0, h.x.i0.data(),
-                         h.p0_chain_ok ? h.p0_chain : nullptr};
-        frc = launch_v6(p, t, &kid, &alias_done, s);
-        if (frc < 0) frc = launch_dyn(p, t, &kid, s);
-    }
-    if (frc > 0) return cuda_fail((cudaError_t)frc, "specialised kernel launch");
-    cudaError_t e = cudaSuccess;
-    if (frc < 0) {
-        kid = 0;
-        e = (cudaError_t)launch_generic(p, s);
-    }
-    if (e != cudaSuccess) return cuda_fail(e, "launch_generic");
-    g_stats.kernel_launches++;
-    g_stats.kernel_id = kid;
-    if (h.alias_rows > 0 && out_row0 < h.alias_rows && alias_done) {
-        g_stats.alias_rows = std::min(h.alias_rows, out_row0 + out_rows) - out_row0;
-    } else if (h.alias_rows > 0 && out_row0 < h.alias_rows) {
-        e = (cudaError_t)launch_alias_rows(p, s);
-        if (e != cudaSuccess) return cuda_fail(e, "launch_alias_rows");
+    // CUDA caps a grid's y and z dimensions at 65,535 (frames are gridDim.z of the main kernels and gridDim.y of the
+    // alias-rows kernel): larger batches run as consecutive frame groups, each with its own tensor map and plan
+    for (int g0 = 0; g0 < n_frames; g0 += kMaxGridFrames) {
+        p.in = d_in + (long long)g0 * in_frame_stride;
+        p.out = d_out + (long long)g0 * out_frame_stride;
+        p.n_frames = std::min(kMaxGridFrames, n_frames - g0);
+        int kid = 0, alias_done = 0;
+        int frc = -1;
+        LaunchShape shape;
+        if (!(flags & LANCZOS_FLAG_GENERIC_KERNEL)) {
+            FastHostTables t{h.phase_w.data(), h.phase_wd.data(), h.align_k.data(), h.x.aligned_exact ? 1 : 0,
+                             h.y.aligned_exact ? 1 : 0, h.x.uniform_phase ? 1 : 0, h.y.uniform_phase ? 1 : 0, h.x.i0.data(),
+                             h.p0_chain_ok ? h.p0_chain : nullptr};
+            frc = launch_v6(p, t, &kid, &alias_done, &shape, s);
+            if (frc < 0) frc = launch_dyn(p, t, &kid, &shape, s);
+        }
+        if (frc > 0) return cuda_fail((cudaError_t)frc, "specialised kernel launch");
+        cudaError_t e = cudaSuccess;
+        if (frc < 0) {
+            kid = 0;
+            e = (cudaError_t)launch_generic(p, &shape, s);
+        }
+        if (e != cudaSuccess) return cuda_fail(e, "launch_generic");
         g_stats.kernel_launches++;
-        g_stats.alias_rows = std::min(h.alias_rows, out_row0 + out_rows) - out_row0;
+        g_stats.kernel_id = kid;
+        if (g0 == 0) set_launch(shape);
+        g_launch.main_launches++;
+        if (h.alias_rows > 0 && out_row0 < h.alias_rows && alias_done) {
+            g_stats.alias_rows = std::min(h.alias_rows, out_row0 + out_rows) - out_row0;
+        } else if (h.alias_rows > 0 && out_row0 < h.alias_rows) {
+            e = (cudaError_t)launch_alias_rows(p, s);
+            if (e != cudaSuccess) return cuda_fail(e, "launch_alias_rows");
+            g_stats.kernel_launches++;
+            g_stats.alias_rows = std::min(h.alias_rows, out_row0 + out_rows) - out_row0;
+        }
     }
     if (count) {
         unsigned long long c = 0;
@@ -376,6 +400,12 @@ void lanczos_b200_enable_stats(int on) { g_stats_enabled.store(on != 0, std::mem
 int lanczos_b200_get_stats(lanczos_stats *out) {
     if (!out) return LANCZOS_ERR_NULL;
     *out = g_stats;
+    return LANCZOS_OK;
+}
+
+int lanczos_b200_get_launch(lanczos_launch *out) {
+    if (!out) return LANCZOS_ERR_NULL;
+    *out = g_launch;
     return LANCZOS_OK;
 }
 
@@ -546,10 +576,12 @@ int lanczos_b200_upscale_planar(const lanczos_desc *desc, const uint8_t *d_in, u
     if (!desc || !d_in || !d_out) return LANCZOS_ERR_NULL;
     if (n_frames < 0) return LANCZOS_ERR_DIMS;
     if (desc->channels < 1 || desc->channels > 4) return LANCZOS_ERR_CHANNELS;
+    const int64_t planes = (int64_t)n_frames * desc->channels;
+    if (planes > INT32_MAX) return LANCZOS_ERR_DIMS;
     // a plane is a one-channel frame: the reference's own loop is per channel, rows then columns (full_TB.h:83-95)
     lanczos_desc plane = *desc;
     plane.channels = 1;
-    return lanczos_b200_upscale_batch(&plane, d_in, d_out, n_frames * desc->channels, in_plane_stride, out_plane_stride,
+    return lanczos_b200_upscale_batch(&plane, d_in, d_out, (int32_t)planes, in_plane_stride, out_plane_stride,
                                       device, cuda_stream);
 }
 
@@ -603,14 +635,21 @@ int lanczos_b200_upscale_hls(const lanczos_desc *desc, const uint8_t *d_in, uint
     if (in_frame_stride == 0) in_frame_stride = r.in_pitch * r.in_h;
     if (out_frame_stride == 0) out_frame_stride = r.out_pitch * r.out_h;
     g_stats = lanczos_stats{};
-    if (n_frames == 0) return LANCZOS_OK;
-    int kid = 100;
-    cudaError_t e = (cudaError_t)launch_hls(d_in, d_out, r.in_pitch, r.out_pitch, in_frame_stride, out_frame_stride,
-                                            n_frames, r.in_w, r.in_h, r.out_w, r.out_h, r.channels, r.a, r.scale_n,
-                                            bit_precision, lut, &kid, (cudaStream_t)cuda_stream);
-    if (e != cudaSuccess) return cuda_fail(e, "launch_hls");
-    g_stats.kernel_launches = 1;
-    g_stats.kernel_id = kid;
+    g_launch = lanczos_launch{};
+    for (int g0 = 0; g0 < n_frames; g0 += kMaxGridFrames) {   // frame groups, as in run_device
+        int kid = 100;
+        LaunchShape shape;
+        cudaError_t e = (cudaError_t)launch_hls(d_in + (long long)g0 * in_frame_stride, d_out + (long long)g0 * out_frame_stride,
+                                                r.in_pitch, r.out_pitch, in_frame_stride, out_frame_stride,
+                                                std::min(kMaxGridFrames, n_frames - g0), r.in_w, r.in_h, r.out_w, r.out_h,
+                                                r.channels, r.a, r.scale_n, bit_precision, lut, &kid, &shape,
+                                                (cudaStream_t)cuda_stream);
+        if (e != cudaSuccess) return cuda_fail(e, "launch_hls");
+        g_stats.kernel_launches++;
+        g_stats.kernel_id = kid;
+        if (g0 == 0) set_launch(shape);
+        g_launch.main_launches++;
+    }
     return LANCZOS_OK;
 }
 

@@ -28,8 +28,15 @@ struct KParams {
     unsigned long long *strict_counter;  // may be null
 };
 
+// Shape of one main-kernel launch, handed back by the launchers (lanczos_b200_get_launch reports it).  The segment
+// fields stay 0 for the kernels without vertical segments (generic, HLS).
+struct LaunchShape {
+    int grid_x = 0, grid_y = 0, grid_z = 0;
+    int seg_periods = 0, chunk_rows = 0;
+    long long resident_ctas = 0;
+};
 // Generic kernel: any ratio, any a<=4, channels 1..4. Returns cudaError_t as int.
-int launch_generic(const KParams &p, cudaStream_t s);
+int launch_generic(const KParams &p, LaunchShape *shape, cudaStream_t s);
 // Specialised TMA + register-window kernels (lanczos_v6.cu, lanczos_dyn.cu). Their launchers return 0 when
 // launched, a positive cudaError_t on failure, -1 when no specialisation applies (the caller then falls back).
 struct FastHostTables {            // host-side views of the plan the specialised kernels need
@@ -43,16 +50,17 @@ struct FastHostTables {            // host-side views of the plan the specialise
 };
 // Static-phase kernels (lanczos_v6.cu): 8-byte V columns, PRMT-spliced copies, scalar constant-bank FFMA.
 // *alias_in_kernel = 1 when the kernel also produced the in-place top rows (no launch_alias_rows needed).
-int launch_v6(const KParams &p, const FastHostTables &t, int *kernel_id, int *alias_in_kernel, cudaStream_t s);
+int launch_v6(const KParams &p, const FastHostTables &t, int *kernel_id, int *alias_in_kernel, LaunchShape *shape,
+              cudaStream_t s);
 // Any-ratio member of the second generation (lanczos_dyn.cu): dynamic-phase H pass, static systolic V pass.
-int launch_dyn(const KParams &p, const FastHostTables &t, int *kernel_id, cudaStream_t s);
+int launch_dyn(const KParams &p, const FastHostTables &t, int *kernel_id, LaunchShape *shape, cudaStream_t s);
 // In-place top rows (full_TB.h:67-77 aliasing), exact double arithmetic.
 int launch_alias_rows(const KParams &p, cudaStream_t s);
 // Fixed-point HLS arithmetic (lanczos_hls.cu), integer scales; lut has a*n+1 entries in units of 2^-bp.
 // *kernel_id: 101 = tiled kernel (a, n compile-time, bp = 8), 100 = generic tile kernel.
 int launch_hls(const uint8_t *in, uint8_t *out, long long in_pitch, long long out_pitch, long long in_fs,
                long long out_fs, int n_frames, int in_w, int in_h, int out_w, int out_h, int channels, int a, int n,
-               int bp, const int *lut, int *kernel_id, cudaStream_t s);
+               int bp, const int *lut, int *kernel_id, LaunchShape *shape, cudaStream_t s);
 // Packed 24-bit words <-> interleaved RGB for lanczos_b200_stream.
 int launch_words_to_rgb(const uint32_t *words, uint8_t *rgb, long long n_px, cudaStream_t s);
 int launch_rgb_to_words(const uint8_t *rgb, uint32_t *words, long long n_px, cudaStream_t s);

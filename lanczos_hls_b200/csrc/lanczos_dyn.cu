@@ -482,7 +482,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
 }
 
 template <int C, int A, int N, int D, int MODE>
-int launch_dyn_one(const KParams &k, const FastHostTables &t, cudaStream_t s) {
+int launch_dyn_one(const KParams &k, const FastHostTables &t, LaunchShape *shape, cudaStream_t s) {
     using G = GeoD<C, A, N, D>;
     const int row_bytes = k.out_w * C;
     const int strips = (row_bytes + G::SWB - 1) / G::SWB;
@@ -523,6 +523,7 @@ int launch_dyn_one(const KParams &k, const FastHostTables &t, cudaStream_t s) {
     p.strict_counter = k.strict_counter;
 
     dim3 grid(strips, sp.segs, k.n_frames);
+    *shape = LaunchShape{(int)grid.x, (int)grid.y, (int)grid.z, sp.seg_periods, G::RB, res.ctas};
     kern<<<grid, 32, smem, s>>>(map, p);
     return (int)cudaGetLastError();
 }
@@ -536,10 +537,10 @@ int launch_dyn_one(const KParams &k, const FastHostTables &t, cudaStream_t s) {
 #define LZD_PART 0
 #endif
 #if LZD_PART == 0
-int launch_dyn_part1(const KParams &k, const FastHostTables &t, int *kernel_id, cudaStream_t s);
-int launch_dyn(const KParams &k, const FastHostTables &t, int *kernel_id, cudaStream_t s) {
+int launch_dyn_part1(const KParams &k, const FastHostTables &t, int *kernel_id, LaunchShape *shape, cudaStream_t s);
+int launch_dyn(const KParams &k, const FastHostTables &t, int *kernel_id, LaunchShape *shape, cudaStream_t s) {
 #else
-int launch_dyn_part1(const KParams &k, const FastHostTables &t, int *kernel_id, cudaStream_t s) {
+int launch_dyn_part1(const KParams &k, const FastHostTables &t, int *kernel_id, LaunchShape *shape, cudaStream_t s) {
 #endif
     if (!strip_layout_ok(k) || !t.i0x_host) return -1;
     const int mode = (k.flags & LANCZOS_FLAG_TOLERANCE_1LSB) ? 1 : 0;
@@ -547,7 +548,7 @@ int launch_dyn_part1(const KParams &k, const FastHostTables &t, int *kernel_id, 
 #define LZD_CASE(c, a, n, d, id)                                                   \
     if (C == c && A == a && N == n && D == d) {                                     \
         *kernel_id = id;                                                            \
-        return mode == 0 ? launch_dyn_one<c, a, n, d, 0>(k, t, s) : launch_dyn_one<c, a, n, d, 1>(k, t, s); \
+        return mode == 0 ? launch_dyn_one<c, a, n, d, 0>(k, t, shape, s) : launch_dyn_one<c, a, n, d, 1>(k, t, shape, s); \
     }
 #if LZD_PART == 0
     LZD_CASE(3, 3, 17, 10, 5)
@@ -560,7 +561,7 @@ int launch_dyn_part1(const KParams &k, const FastHostTables &t, int *kernel_id, 
     LZD_CASE(1, 2, 3, 1, 13)
     LZD_CASE(3, 3, 4, 1, 14)
     LZD_CASE(1, 3, 3, 1, 15)
-    return launch_dyn_part1(k, t, kernel_id, s);
+    return launch_dyn_part1(k, t, kernel_id, shape, s);
 #else
     LZD_CASE(3, 3, 5, 3, 16)
     LZD_CASE(3, 3, 7, 4, 17)

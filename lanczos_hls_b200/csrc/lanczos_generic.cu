@@ -186,8 +186,9 @@ __global__ void rgb_to_words_kernel(const uint8_t *rgb, uint32_t *words, long lo
 
 }  // namespace
 
-int launch_generic(const KParams &p, cudaStream_t s) {
+int launch_generic(const KParams &p, LaunchShape *shape, cudaStream_t s) {
     dim3 grid((p.out_w + GT_W - 1) / GT_W, (p.out_rows + GT_H - 1) / GT_H, p.n_frames);
+    *shape = LaunchShape{(int)grid.x, (int)grid.y, (int)grid.z};
     dim3 block(GT_THREADS);
     switch (p.channels) {
         case 1: lanczos_generic_kernel<1><<<grid, block, 0, s>>>(p); break;

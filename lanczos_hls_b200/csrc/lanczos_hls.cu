@@ -206,12 +206,13 @@ __global__ void __launch_bounds__(256) lanczos_hls_tile_kernel(const __grid_cons
 // Returns -1 without launching when the LUT lacks the whole-pixel pattern the MASK instance assumes (the caller then
 // runs lanczos_hls_kernel).  The library's own LUT always has it for the configurations below.
 template <int C, int A, int N, int MASK>
-int launch_hls_tile(const HlsParams &p, int n_frames, cudaStream_t s) {
+int launch_hls_tile(const HlsParams &p, int n_frames, LaunchShape *shape, cudaStream_t s) {
     using G = HlsGeo<C, A, N>;
     bool pattern = p.lut[0] == (1 << 8);
     for (int k = 1; k <= A; k++) pattern = pattern && p.lut[k * N] == (((MASK >> k) & 1) ? -1 : 0);
     if (!pattern) return -1;
     dim3 grid((p.out_w + G::TW - 1) / G::TW, (p.out_h + G::TH - 1) / G::TH, n_frames);
+    *shape = LaunchShape{(int)grid.x, (int)grid.y, (int)grid.z};
     lanczos_hls_tile_kernel<C, A, N, MASK><<<grid, 256, 0, s>>>(p);
     return (int)cudaGetLastError();
 }
@@ -220,7 +221,7 @@ int launch_hls_tile(const HlsParams &p, int n_frames, cudaStream_t s) {
 
 int launch_hls(const uint8_t *in, uint8_t *out, long long in_pitch, long long out_pitch, long long in_fs,
                long long out_fs, int n_frames, int in_w, int in_h, int out_w, int out_h, int channels, int a, int n,
-               int bp, const int *lut, int *kernel_id, cudaStream_t s) {
+               int bp, const int *lut, int *kernel_id, LaunchShape *shape, cudaStream_t s) {
     HlsParams p{};
     p.in = in; p.out = out; p.in_pitch = in_pitch; p.out_pitch = out_pitch;
     p.in_frame_stride = in_fs; p.out_frame_stride = out_fs;
@@ -229,7 +230,7 @@ int launch_hls(const uint8_t *in, uint8_t *out, long long in_pitch, long long ou
     if (bp == 8) {      // 16-bit intermediates: the tiled kernel (the reference's template BIT_PRECISION is 8)
         // a = 3: floor(L(2) * 2^BP) = -1 (sin(2 pi) < 0 in double), the other whole-pixel entries are 0; a = 2: all 0
         int rc = -1;
-#define HLS_CASE(c, aa, nn, mask) if (channels == c && a == aa && n == nn) rc = launch_hls_tile<c, aa, nn, mask>(p, n_frames, s);
+#define HLS_CASE(c, aa, nn, mask) if (channels == c && a == aa && n == nn) rc = launch_hls_tile<c, aa, nn, mask>(p, n_frames, shape, s);
         HLS_CASE(3, 3, 2, 4) HLS_CASE(4, 3, 2, 4) HLS_CASE(1, 3, 2, 4) HLS_CASE(3, 2, 2, 0) HLS_CASE(3, 3, 4, 4) HLS_CASE(3, 2, 4, 0)
 #undef HLS_CASE
         if (rc >= 0) {
@@ -239,6 +240,7 @@ int launch_hls(const uint8_t *in, uint8_t *out, long long in_pitch, long long ou
     }
     *kernel_id = 100;
     dim3 grid((out_w + HT_W - 1) / HT_W, (out_h + HT_H - 1) / HT_H, n_frames);
+    *shape = LaunchShape{(int)grid.x, (int)grid.y, (int)grid.z};
     switch (channels) {
         case 1: lanczos_hls_kernel<1><<<grid, HT_THREADS, 0, s>>>(p); break;
         case 2: lanczos_hls_kernel<2><<<grid, HT_THREADS, 0, s>>>(p); break;

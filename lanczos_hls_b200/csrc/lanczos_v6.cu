@@ -1001,7 +1001,7 @@ SegPlan plan_v6_segments(int vperiods, int D, int A, int RB, long long cols, lon
 }
 
 template <int C, int A, int N, int D, int PH, int KM, int MODE, bool ST64>
-int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kernel, cudaStream_t s) {
+int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kernel, LaunchShape *shape, cudaStream_t s) {
     using G = Geo6<C, A, N, D, PH, MODE>;
     CUtensorMap map;
     if (!encode_input_map(&map, k, G::BOX_B, G::RB)) return -1;
@@ -1039,6 +1039,7 @@ int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kerne
     p.strict_counter = k.strict_counter;
 
     dim3 grid(strips, sp.segs, k.n_frames);
+    *shape = LaunchShape{(int)grid.x, (int)grid.y, (int)grid.z, sp.seg_periods, G::RB, res.ctas};
     p.independent = (k.flags & LANCZOS_FLAG_INDEPENDENT) ? 1 : 0;
     if (p.independent) {
         cudaLaunchConfig_t cfg{};
@@ -1060,7 +1061,8 @@ int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kerne
 }  // namespace
 
 // Returns 0 on launch, >0 cudaError, -1 when no specialised kernel applies (caller falls back).
-int launch_v6(const KParams &k, const FastHostTables &t, int *kernel_id, int *alias_in_kernel, cudaStream_t s) {
+int launch_v6(const KParams &k, const FastHostTables &t, int *kernel_id, int *alias_in_kernel, LaunchShape *shape,
+              cudaStream_t s) {
     if (!strip_layout_ok(k)) return -1;
     // 64-bit stores of the V pass
     const bool st64 = (k.out_w * k.channels) % 8 == 0 && k.out_pitch % 8 == 0 && (reinterpret_cast<uintptr_t>(k.out) & 7) == 0 &&
@@ -1078,10 +1080,10 @@ int launch_v6(const KParams &k, const FastHostTables &t, int *kernel_id, int *al
 #define LZ6_CASE(c, a, n, d, ph, kmask, id)                                                            \
     if (C == c && A == a && N == n && D == d && km == (kmask)) {                                        \
         *kernel_id = id;                                                                                \
-        if (mode == 0) return st64 ? launch_v6_one<c, a, n, d, ph, kmask, 0, true>(k, t, alias_in_kernel, s)         \
-                                   : launch_v6_one<c, a, n, d, ph, kmask, 0, false>(k, t, alias_in_kernel, s);       \
-        return st64 ? launch_v6_one<c, a, n, d, ph, kmask, 1, true>(k, t, alias_in_kernel, s)                        \
-                    : launch_v6_one<c, a, n, d, ph, kmask, 1, false>(k, t, alias_in_kernel, s);                      \
+        if (mode == 0) return st64 ? launch_v6_one<c, a, n, d, ph, kmask, 0, true>(k, t, alias_in_kernel, shape, s)         \
+                                   : launch_v6_one<c, a, n, d, ph, kmask, 0, false>(k, t, alias_in_kernel, shape, s);       \
+        return st64 ? launch_v6_one<c, a, n, d, ph, kmask, 1, true>(k, t, alias_in_kernel, shape, s)                        \
+                    : launch_v6_one<c, a, n, d, ph, kmask, 1, false>(k, t, alias_in_kernel, shape, s);                      \
     }
     // the phase-0 second look is the exact fp32 chain (phase0_chain2): only with plan.cpp's proof for these weights
     if (km != 0 && !t.p0_chain) return -1;

@@ -147,10 +147,15 @@ static coord_t *build_coords(int out_len, int in_len, int a, double scale) {
     return c;
 }
 
-int oracle_expected_planar_fast(const uint8_t *in, uint8_t *out, int channels,
-                                int in_w, int in_h, int out_w, int out_h, int a,
-                                int scale_n, int scale_d, int variant, int threads) {
+/* Output rows [row0, row0 + rows) of the planar result; the other rows of `out` are scratch.  Only the input rows
+ * those rows read go through the horizontal pass.  In place (VERBATIM) a top row reads rows below it that already
+ * hold final output (full_TB.h:67-77), so the vertical pass starts at the first row that reads no row below itself
+ * and walks up from there like the full sweep does: every row the band reads has the value the full sweep gives it. */
+static int expected_planar_rows(const uint8_t *in, uint8_t *out, int channels, int in_w, int in_h, int out_w,
+                                int out_h, int a, int scale_n, int scale_d, int variant, int threads, int row0,
+                                int rows) {
     if (check_args(channels, in_w, in_h, out_w, out_h, a, scale_n, scale_d)) return -1;
+    if (row0 < 0 || rows < 0 || row0 + rows > out_h) return -1;
     if (a > 8) return -1;
     const double scale = (double)scale_n / scale_d;
     const size_t in_plane = (size_t)in_w * in_h, out_plane = (size_t)out_w * out_h;
@@ -168,10 +173,20 @@ int oracle_expected_planar_fast(const uint8_t *in, uint8_t *out, int channels,
     threads = 1;
 #endif
     memset(out, 0, out_plane * channels);
+    if (rows == 0) {
+        free(cx); free(cy); free(tmp);
+        return 0;
+    }
+    /* vertical rows yy_lo..yy_hi (bottom-up), horizontal rows h_lo..h_hi; first/last grow with the output row, so
+     * yy_hi is the first row at or below the band that reads no row below itself */
+    const int yy_lo = row0;
+    int yy_hi = row0 + rows - 1;
+    while (cy[yy_hi].last > yy_hi) yy_hi = cy[yy_hi].last;
+    const int h_lo = cy[yy_lo].first, h_hi = cy[yy_hi].last;
     /* horizontal pass: rows are independent */
 #pragma omp parallel for num_threads(threads) schedule(static) collapse(2)
     for (int j = 0; j < channels; j++) {
-        for (int i = 0; i < in_h; i++) {
+        for (int i = h_lo; i <= h_hi; i++) {
             const uint8_t *src = in + j * in_plane + (size_t)i * in_w;
             uint8_t *dst = out + j * out_plane + (size_t)i * out_w;
             for (int xx = 0; xx < out_w; xx++) {
@@ -195,7 +210,7 @@ int oracle_expected_planar_fast(const uint8_t *in, uint8_t *out, int channels,
             uint8_t *plane = out + j * out_plane;
             const uint8_t *src = tmp ? tmp + j * out_plane : plane;
             double acc[256];
-            for (int xx = out_h - 1; xx >= 0; xx--) {
+            for (int xx = yy_hi; xx >= yy_lo; xx--) {
                 const coord_t *c = &cy[xx];
                 for (int col = c0; col < c1; col++) acc[col - c0] = 0;
                 for (int t = c->first, k = 0; t <= c->last; t++, k++) {
@@ -210,6 +225,13 @@ int oracle_expected_planar_fast(const uint8_t *in, uint8_t *out, int channels,
     }
     free(cx); free(cy); free(tmp);
     return 0;
+}
+
+int oracle_expected_planar_fast(const uint8_t *in, uint8_t *out, int channels,
+                                int in_w, int in_h, int out_w, int out_h, int a,
+                                int scale_n, int scale_d, int variant, int threads) {
+    return expected_planar_rows(in, out, channels, in_w, in_h, out_w, out_h, a, scale_n, scale_d, variant, threads,
+                                0, out_h);
 }
 
 /* ---- interleaved front end (full_TB.h:127-138, :146-165) ------------------ */
@@ -231,8 +253,8 @@ int oracle_upscale_interleaved_rows(const uint8_t *in, int64_t in_pitch,
         for (int x = 0; x < in_w; x++)
             for (int c = 0; c < channels; c++)
                 pin[c * in_plane + (size_t)y * in_w + x] = in[y * in_pitch + (int64_t)x * channels + c];
-    int rc = oracle_expected_planar_fast(pin, pout, channels, in_w, in_h, out_w, out_h, a,
-                                         scale_n, scale_d, variant, threads);
+    int rc = expected_planar_rows(pin, pout, channels, in_w, in_h, out_w, out_h, a, scale_n, scale_d, variant,
+                                  threads, row0, rows);
     if (rc == 0) {
         for (int y = 0; y < rows; y++)
             for (int x = 0; x < out_w; x++)

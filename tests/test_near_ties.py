@@ -84,17 +84,26 @@ def q_table(xx, n, d, a):
     return NT.quantise(NT.seq_sum(np.repeat(np.arange(256)[:, None], 2 * a, axis=1), w))
 
 
-def v_image(oracle, n, d, a, c, seed=0, nblk=24):
+def v_image(oracle, n, d, a, c, seed=0, nblk=24, base=None, place=None):
     """Tall, narrow image with every V window of (n, d, a) planted; returns (img, [(block, channel, X, idx)]).
-    A window goes to one channel of one block; windows whose bytes no q_X of the block reaches are skipped."""
+    A window goes to one channel of one block; windows whose bytes no q_X of the block reaches are skipped.
+    base: plant into a copy of this [H][W][C] image instead; place(idx): the output row of window idx (None: leave it
+    out), by default its stored coordinate when that lies below V_TOP."""
     idx = config_rows(n, d, a)
     taps = 2 * a
     wblk = taps + 4
     p0s = [4 + j * (wblk + BLOCK_GAP) for j in range(nblk)]
-    step = 16 * d
-    in_w = step * ((p0s[-1] + wblk + 4 + step - 1) // step)
-    in_h = max([tap0(int(WIN["coord"][i]), n, d, a) + taps for i in idx] + [64]) + 4
-    img = noise_hwc(oracle, in_h, in_w, c, seed=seed + 1)
+    if base is None:
+        step = 16 * d
+        in_w = step * ((p0s[-1] + wblk + 4 + step - 1) // step)
+        in_h = max([tap0(int(WIN["coord"][i]), n, d, a) + taps for i in idx] + [64]) + 4
+        img = noise_hwc(oracle, in_h, in_w, c, seed=seed + 1)
+    else:
+        img = base.copy()
+        in_w = img.shape[1]
+    if place is None:
+        def place(i):
+            return int(WIN["coord"][i]) if WIN["coord"][i] >= V_TOP else None
     # interior output columns of every block (all taps inside the block) and their q tables
     cols = []
     for p0 in p0s:
@@ -103,8 +112,8 @@ def v_image(oracle, n, d, a, c, seed=0, nblk=24):
     used = {}                                       # (block, channel) -> occupied [lo, hi) input rows
     planted = []
     for i in idx:
-        yy = int(WIN["coord"][i])
-        if yy < V_TOP:
+        yy = place(i)
+        if yy is None:
             continue
         lo = tap0(yy, n, d, a)
         win = WIN["win"][i][:taps]
