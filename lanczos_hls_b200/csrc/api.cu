@@ -100,12 +100,16 @@ long long scratch_pitch(long long row_bytes) { return (row_bytes + 15) / 16 * 16
 // no renormalisation) and every output column is computed independently of the others, so the original columns
 // come out bit for bit; the extra output columns are never copied back.  The reference's own sample size
 // (lanczos.h:13-14: 162 -> 486 pixels, planar) takes the specialised kernels this way.
+// The extra output columns must not change which descriptors are accepted: when one of them fails the reference's
+// float floor (LANCZOS_ERR_RATIO_FLOAT) the image is run at its own widths, as the device entry points would run it.
 lanczos_desc widened(const lanczos_desc &r) {
     lanczos_desc d = r;            // resolved: scale_n / scale_d are explicit, so the ratio does not follow the new widths
-    const int q = d.channels == 4 ? 1 : (d.channels == 2 ? 2 : 4);
-    d.in_w = (r.in_w + q - 1) / q * q;
-    d.out_w = (r.out_w + q - 1) / q * q;
     d.in_pitch = d.out_pitch = 0;
+    const int q = d.channels == 4 ? 1 : (d.channels == 2 ? 2 : 4);
+    const int out_w = (r.out_w + q - 1) / q * q;
+    if (!float_floor_exact(r.out_w, out_w, r.scale_n, r.scale_d)) return d;
+    d.in_w = (r.in_w + q - 1) / q * q;
+    d.out_w = out_w;
     return d;
 }
 cudaError_t copy_rows(void *dst, long long dpitch, const void *src, long long spitch, long long row_bytes, long long rows,

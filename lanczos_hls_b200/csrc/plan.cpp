@@ -137,10 +137,18 @@ int resolve_desc(const lanczos_desc *in, lanczos_desc *out) {
     return LANCZOS_OK;
 }
 
+bool float_floor_exact(int from, int to, int n, int d) {
+    const double scale = (double)n / d;  // lanczos.h:112
+    for (int xx = from; xx < to; xx++)
+        if ((double)((int64_t)xx * d / n) != std::floor((double)xx / scale)) return false;
+    return true;
+}
+
 static int build_axis(AxisTables &t, int out_len, int in_len, int a, int n, int dd,
                       const std::vector<float> &phase_w, const std::vector<double> &phase_wd) {
     const int taps = 2 * a;
     const double scale = (double)n / dd;  // lanczos.h:112
+    if (!float_floor_exact(0, out_len, n, dd)) return LANCZOS_ERR_RATIO_FLOAT;
     t.out_len = out_len;
     t.in_len = in_len;
     t.i0.resize(out_len);
@@ -154,7 +162,6 @@ static int build_axis(AxisTables &t, int out_len, int in_len, int a, int n, int 
         const double x = (double)xx / scale;  // full_TB.h:57,70
         const double fx = std::floor(x);
         const int64_t q = (int64_t)xx * dd / n;
-        if ((double)q != fx) return LANCZOS_ERR_RATIO_FLOAT;
         const int phase = (int)(((int64_t)xx * dd) % n);
         if (phase == 0 && x != fx) t.aligned_exact = false;
         const int first = (int)q - a + 1;

@@ -63,6 +63,10 @@ bool verify_phase0_chain(const double *w, float *W);
 // The reference kernel, full_TB.h:39-53.
 double ref_kernel(double x, int a);
 
+// True when the reference's tap origin floor((double)xx / ((double)n/d)) (full_TB.h:57) equals the exact floor(xx*d/n)
+// for every output coordinate xx in [from, to): the condition behind LANCZOS_ERR_RATIO_FLOAT.
+bool float_floor_exact(int from, int to, int n, int d);
+
 // Input row range needed for a band of output rows (global indices).
 void band_rows(const Plan &p, int out_row0, int out_rows, int *in_row0, int *in_rows);
 

@@ -1,6 +1,8 @@
-"""Generate tests/golden/near_ties.npz: adversarial 2a-byte windows whose reference sums land on or near an integer.
+"""Generate tests/golden/near_ties.npz and tests/golden/near_ties_any_ratio.npz: adversarial 2a-byte windows whose
+reference sums land on or near an integer.
 
-Run once from the repository root: `python tests/golden/make_near_ties.py` (a few minutes on 8 cores).
+Run once from the repository root: `python tests/golden/make_near_ties.py` (a few minutes on 8 cores).  A re-run
+writes both files again byte for byte.
 
 The product's outputs must equal the reference's double-precision software path bit for bit
 (full_TB.h:55-77: x = xx/SCALE, sum += in[i] * lanczos_kernel(x - i) in ascending taps, clamp, truncate).
@@ -21,11 +23,22 @@ stores the window bytes in three classes:
 Weights come from the oracle's oracle_kernel (glibc sin, as in the reference).  Ties are found by a
 meet-in-the-middle search over every window for a <= 3 (a = 4: 2^48 of its 2^64 windows); the other two classes
 by random windows.  The oracle stays the truth: this file only decides what the tests cover.
+
+near_ties_any_ratio.npz holds windows for the generic kernel (lanczos_generic.cu), which serves every ratio and
+(channels, a) without a kernel instance.  Its arithmetic differs from the instances': s = fmaf(b_k, (float)w_k, s) from
+0 in ascending taps, each output coordinate with its own weights.  For every ratio N/D <= 16 the library accepts and
+a = 1..4 (GENERIC_CONFIGS), at one coordinate near the origin and one near 1024, both on edges of the generic kernel's
+64 x 32 output tiles, it stores
+  * wrong side (1): 1e-9 <= distance <= 3e-5 and that chain truncates differently from the reference (flag
+    F_WRONG_GENERIC; F_OFF_INTEGER when the fp32 result is not the integer itself, so that only a guard wider than
+    half an ulp re-evaluates the sample);
+  * near (2): distance <= 1e-6.
 Classes that no window falls into are empty.  For 2/1 the weights of the one interpolated phase are symmetric, so
 a sum is a combination of the pair sums b_k + b_{2a-1-k}: with a = 1 or 2 no window comes within 3e-5 of an integer
 1..255 at all, and with a = 3 or 4 no tie discriminates.  The search found no discriminating tie either for 3/2 and 3/1
 with a = 2 or for 4/1 with a = 3; those ratios keep their wrong-side and near windows.
 """
+import math
 import multiprocessing
 import os
 import sys
@@ -39,6 +52,7 @@ sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import oracle_py as O  # noqa: E402
 
 OUT = os.path.join(HERE, "near_ties.npz")
+OUT_ANY = os.path.join(HERE, "near_ties_any_ratio.npz")
 
 # every (N, D, a) that a specialised kernel instance serves
 CONFIGS = [(2, 1, 1), (2, 1, 2), (2, 1, 3), (2, 1, 4), (3, 2, 2), (3, 2, 3), (17, 10, 3), (3, 1, 2), (3, 1, 3),
@@ -47,6 +61,7 @@ MAGNITUDES = [36, 1024, 12288, 27648]
 TIE, WRONG, NEAR = 0, 1, 2
 # flag bits
 F_PHASE, F_FMA, F_REV, F_INTEGRAL, F_WRONG_OUTER, F_WRONG_ASC = 1, 2, 4, 8, 16, 32
+F_WRONG_GENERIC, F_OFF_INTEGER = 64, 128
 TIE_TOL, WRONG_LO, WRONG_HI, NEAR_TOL = 4e-12, 1e-9, 3e-5, 1e-6
 CAP_TIE_EACH, CAP_INTEGRAL, CAP_WRONG, CAP_NEAR = 4, 2, 4, 3
 
@@ -187,6 +202,58 @@ def coordinates(n, d, a):
     return out
 
 
+def float_floor_ok(xx, n, d):
+    """The reference's tap origin floor((double)xx / ((double)N/D)) equals the exact floor(xx*D/N) (plan.cpp)."""
+    return math.floor(xx / (n / d)) == xx * d // n
+
+
+def first_float_floor_miss(n, d, limit=1 << 12):
+    """The first output coordinate below `limit` at which the library rejects N/D (LANCZOS_ERR_RATIO_FLOAT), or None."""
+    return next((xx for xx in range(limit) if not float_floor_ok(xx, n, d)), None)
+
+
+# every reduced N/D with D < N <= 16 that the library accepts up to 4096 output samples, with a = 1..4
+GENERIC_CONFIGS = [(n, d, a) for n in range(2, 17) for d in range(1, n) if math.gcd(n, d) == 1
+                   and first_float_floor_miss(n, d) is None for a in range(1, 5)]
+GENERIC_BASES = [64, 1024]
+
+
+def generic_coordinates(n, d):
+    """Per base, the first interpolated coordinate among base - 1, base, base + 63, base + 64, ...: the last or first
+    column of a 64-pixel tile and the last or first row of a 32-row tile of the generic kernel."""
+    return [next(xx for j in range(n) for xx in (b + 64 * j - 1, b + 64 * j) if phase(xx, n, d) != 0)
+            for b in GENERIC_BASES]
+
+
+def generic_chain(win, w):
+    """lanczos_generic.cu: s = fmaf((float)b_k, (float)w_k, s) from 0, ascending taps, this coordinate's own weights."""
+    return f32_chain(win, np.asarray(w).astype(np.float32), list(range(len(w))))
+
+
+def classify_generic(win, xx, n, d, a):
+    """(class or -1, flags, nearest integer, distance) of one window for the generic kernel's arithmetic."""
+    taps = 2 * a
+    w, _ = weights(xx, n, d, a)
+    win = np.asarray(win[:taps], dtype=np.int64)
+    s = float(seq_sum(win, w)[0])
+    k = int(np.rint(s))
+    dist = abs(s - k)
+    if k < 1 or k > 255:
+        return -1, 0, k, dist
+    flags = 0
+    if dist >= WRONG_LO:
+        g = generic_chain(win, w)
+        if quantise(g) != quantise(s):
+            flags |= F_WRONG_GENERIC | (F_OFF_INTEGER if g != k else 0)
+    if WRONG_LO <= dist <= WRONG_HI and flags & F_WRONG_GENERIC:
+        cls = WRONG
+    elif dist <= NEAR_TOL:
+        cls = NEAR
+    else:
+        cls = -1
+    return cls, flags, k, dist
+
+
 def half_sums(w, rng, limit):
     """All byte combinations of the taps with weights w (or `limit` random ones): (sums, bytes)."""
     h = len(w)
@@ -275,10 +342,26 @@ def one_coordinate(job):
     return (n, d, a, xx, len(ties), rows)
 
 
-def main():
-    jobs = [(n, d, a, xx) for (n, d, a) in CONFIGS for xx in coordinates(n, d, a)]
-    with multiprocessing.Pool(min(8, os.cpu_count() or 1)) as pool:
-        results = pool.map(one_coordinate, jobs, chunksize=1)
+def one_generic_coordinate(job):
+    n, d, a, xx = job
+    rng = np.random.default_rng(1000003 * n + 1009 * d + 101 * a + xx + 7)
+    w, _ = weights(xx, n, d, a)
+    rows = []
+    n_wrong = n_near = 0
+    for win in random_candidates(w, rng):
+        if n_wrong >= CAP_WRONG and n_near >= CAP_NEAR:
+            break
+        cls, flags, k, dist = classify_generic(win, xx, n, d, a)
+        if cls == WRONG and n_wrong < CAP_WRONG:
+            n_wrong += 1
+            rows.append((WRONG, win, flags, k, dist))
+        elif cls == NEAR and n_near < CAP_NEAR:
+            n_near += 1
+            rows.append((NEAR, win, flags, k, dist))
+    return (n, d, a, xx, 0, rows)
+
+
+def save(path, results):
     cols = {k: [] for k in ("n", "d", "a", "coord", "cls", "flags", "k", "dist", "win")}
     for (n, d, a, xx, n_ties, rows) in results:
         print(f"{n}/{d} a={a} x={xx}: {n_ties} ties found, kept " +
@@ -289,9 +372,17 @@ def main():
             for key, v in (("n", n), ("d", d), ("a", a), ("coord", xx), ("cls", cls), ("flags", flags), ("k", k),
                            ("dist", dist), ("win", padded)):
                 cols[key].append(v)
-    np.savez_compressed(OUT, **{k: np.array(v, dtype=np.float64 if k == "dist" else (np.uint8 if k == "win" else np.int32))
-                                for k, v in cols.items()})
-    print("wrote", OUT, os.path.getsize(OUT), "bytes,", len(cols["n"]), "windows")
+    np.savez_compressed(path, **{k: np.array(v, dtype=np.float64 if k == "dist" else (np.uint8 if k == "win" else np.int32))
+                                 for k, v in cols.items()})
+    print("wrote", path, os.path.getsize(path), "bytes,", len(cols["n"]), "windows")
+
+
+def main():
+    jobs = [(n, d, a, xx) for (n, d, a) in CONFIGS for xx in coordinates(n, d, a)]
+    any_jobs = [(n, d, a, xx) for (n, d, a) in GENERIC_CONFIGS for xx in generic_coordinates(n, d)]
+    with multiprocessing.Pool(min(8, os.cpu_count() or 1)) as pool:
+        save(OUT, pool.map(one_coordinate, jobs, chunksize=1))
+        save(OUT_ANY, pool.map(one_generic_coordinate, any_jobs, chunksize=1))
 
 
 if __name__ == "__main__":

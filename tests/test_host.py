@@ -1,5 +1,6 @@
 """CPU tests of the host logic and the C-ABI surface (no compute calls: there is no GPU here)."""
 import ctypes
+import math
 import os
 import re
 
@@ -46,7 +47,8 @@ def test_descriptor_validation(lz, kw, code):
 
 
 def test_phase_table_matches_oracle_kernel(lz, oracle):
-    for (n, d, a) in [(2, 1, 3), (3, 2, 3), (17, 10, 3), (3, 1, 2), (4, 1, 3), (1, 1, 3)]:
+    sweep = [(n, d, a) for n in range(2, 17) for d in range(1, n) if math.gcd(n, d) == 1 for a in range(1, 5)]
+    for (n, d, a) in [(2, 1, 3), (3, 2, 3), (17, 10, 3), (3, 1, 2), (4, 1, 3), (1, 1, 3), (65, 64, 4)] + sweep:
         t = lz.phase_table(lz.make_desc(d * 8, d * 8, n * 8, n * 8, 3, a, n, d))
         assert t.shape == (n, 2 * a)
         for xx in range(n):

@@ -36,8 +36,8 @@ def windows():
 WIN = windows()
 
 
-def config_rows(n, d, a):
-    return np.nonzero((WIN["n"] == n) & (WIN["d"] == d) & (WIN["a"] == a))[0]
+def config_rows(n, d, a, win=WIN):
+    return np.nonzero((win["n"] == n) & (win["d"] == d) & (win["a"] == a))[0]
 
 
 def tap0(xx, n, d, a):
@@ -50,17 +50,18 @@ def up_len(in_len, n, d):
 
 # ---- the builder -------------------------------------------------------------------------------------
 
-def h_image(oracle, n, d, a, c, seed=0, odd=False):
-    """Wide, short image with every H window of (n, d, a) planted; returns (img, [(row, channel, idx)])."""
-    idx = config_rows(n, d, a)
+def h_image(oracle, n, d, a, c, seed=0, odd=False, win=WIN):
+    """Wide, short image with every H window of (n, d, a) planted; returns (img, [(row, channel, idx)]).
+    win: the windows (default near_ties.npz)."""
+    idx = config_rows(n, d, a, win)
     taps = 2 * a
-    need = max([tap0(int(WIN["coord"][i]), n, d, a) + taps for i in idx] + [64]) + 4
+    need = max([tap0(int(win["coord"][i]), n, d, a) + taps for i in idx] + [64]) + 4
     step = 16 * d
     in_w = step * ((need + step - 1) // step) + (1 if odd else 0)
     slots = []                                      # per (row, channel): occupied [lo, hi) pixel intervals
     planted = []
     for i in idx:
-        lo = tap0(int(WIN["coord"][i]), n, d, a)
+        lo = tap0(int(win["coord"][i]), n, d, a)
         hi = lo + taps
         for s, iv in enumerate(slots):
             if all(hi <= l or lo >= h for (l, h) in iv):
@@ -73,8 +74,8 @@ def h_image(oracle, n, d, a, c, seed=0, odd=False):
     in_h = max(2 * taps, 2 + (len(slots) + c - 1) // c)
     img = noise_hwc(oracle, in_h, in_w, c, seed=seed)
     for (r, ch, i) in planted:
-        lo = tap0(int(WIN["coord"][i]), n, d, a)
-        img[r, lo:lo + taps, ch] = WIN["win"][i][:taps]
+        lo = tap0(int(win["coord"][i]), n, d, a)
+        img[r, lo:lo + taps, ch] = win["win"][i][:taps]
     return img, planted
 
 
@@ -84,26 +85,26 @@ def q_table(xx, n, d, a):
     return NT.quantise(NT.seq_sum(np.repeat(np.arange(256)[:, None], 2 * a, axis=1), w))
 
 
-def v_image(oracle, n, d, a, c, seed=0, nblk=24, base=None, place=None):
+def v_image(oracle, n, d, a, c, seed=0, nblk=24, base=None, place=None, win=WIN):
     """Tall, narrow image with every V window of (n, d, a) planted; returns (img, [(block, channel, X, idx)]).
     A window goes to one channel of one block; windows whose bytes no q_X of the block reaches are skipped.
     base: plant into a copy of this [H][W][C] image instead; place(idx): the output row of window idx (None: leave it
     out), by default its stored coordinate when that lies below V_TOP."""
-    idx = config_rows(n, d, a)
+    idx = config_rows(n, d, a, win)
     taps = 2 * a
     wblk = taps + 4
     p0s = [4 + j * (wblk + BLOCK_GAP) for j in range(nblk)]
     if base is None:
         step = 16 * d
         in_w = step * ((p0s[-1] + wblk + 4 + step - 1) // step)
-        in_h = max([tap0(int(WIN["coord"][i]), n, d, a) + taps for i in idx] + [64]) + 4
+        in_h = max([tap0(int(win["coord"][i]), n, d, a) + taps for i in idx] + [64]) + 4
         img = noise_hwc(oracle, in_h, in_w, c, seed=seed + 1)
     else:
         img = base.copy()
         in_w = img.shape[1]
     if place is None:
         def place(i):
-            return int(WIN["coord"][i]) if WIN["coord"][i] >= V_TOP else None
+            return int(win["coord"][i]) if win["coord"][i] >= V_TOP else None
     # interior output columns of every block (all taps inside the block) and their q tables
     cols = []
     for p0 in p0s:
@@ -116,14 +117,14 @@ def v_image(oracle, n, d, a, c, seed=0, nblk=24, base=None, place=None):
         if yy is None:
             continue
         lo = tap0(yy, n, d, a)
-        win = WIN["win"][i][:taps]
+        bytes_ = win["win"][i][:taps]
         done = False
         for b, p0 in enumerate(p0s):
             for ch in range(c):
                 if done or not all(lo + taps <= l or lo >= h for (l, h) in used.get((b, ch), [])):
                     continue
                 for X, q in cols[b]:
-                    pre = [np.nonzero(q == t)[0] for t in win]
+                    pre = [np.nonzero(q == t)[0] for t in bytes_]
                     if all(len(v) for v in pre):
                         used.setdefault((b, ch), []).append((lo, lo + taps))
                         for k, v in enumerate(pre):
@@ -224,10 +225,10 @@ def test_weights_are_the_oracles(oracle):
             assert w[k] == oracle.lib().oracle_kernel(x - (first + k), a)
 
 
-def planted_counts(planted):
+def planted_counts(planted, win=WIN):
     out = {TIE: 0, WRONG: 0, NEAR: 0}
     for p in planted:
-        out[int(WIN["cls"][p[-1]])] += 1
+        out[int(win["cls"][p[-1]])] += 1
     return out
 
 
@@ -339,9 +340,9 @@ def run_gpu(torch, lz, img, ow, oh, a, n, d, flags=0):
     return d_out.cpu().numpy()
 
 
-def strict_floor(planted):
+def strict_floor(planted, win=WIN):
     """Samples the exact path must have evaluated: the planted near and wrong-side windows."""
-    return sum(1 for p in planted if WIN["cls"][p[-1]] in (NEAR, WRONG))
+    return sum(1 for p in planted if win["cls"][p[-1]] in (NEAR, WRONG))
 
 
 def check_image(torch, lz, oracle, img, planted, a, n, d, kid):
