@@ -1,4 +1,4 @@
-// fast_common.cuh -- device/host helpers shared by the TMA + register-window kernels
+// fast_common.cuh -- the strip pipeline and the device/host helpers shared by the TMA + register-window kernels
 // (lanczos_v6.cu: static-phase H pass for a few ratios; lanczos_dyn.cu: any ratio with N <= 32).
 #pragma once
 #include <algorithm>
@@ -120,9 +120,9 @@ __device__ __forceinline__ uint32_t quantise4(float a, float b, float c, float d
     return r;
 }
 
-// Exact restatement of full_TB.h:58-63 for one sample whose 2a taps are `stride` bytes apart in
-// shared memory (taps outside the image were zero-filled by TMA: 0*w adds +-0, same bits).
-// (double)byte is formed as (2^52 + b) - 2^52 on the FP64 pipe: I2F.F64 runs on the slow XU unit.
+// The reference's exact sum for one sample whose 2a taps are `stride` bytes apart in shared memory (taps outside the
+// image were zero-filled by TMA).  This is exact_add spelled out: with exact_add itself ptxas schedules three kernel
+// instances differently (v6 <1,3,2,1,24,17,0,true> +8 instructions, dyn <1,3,4,1,0> +6 in its chunk loop).
 template <int TAPS, class W>
 __device__ __forceinline__ uint8_t exact_taps(const uint8_t *tap0, int stride, W weight) {
     double sum = 0.0;
@@ -133,6 +133,95 @@ __device__ __forceinline__ uint8_t exact_taps(const uint8_t *tap0, int stride, W
     }
     return quantise_f64(sum);
 }
+
+// ---------------------------------------------------------------------------------------------
+// the strip pipeline both families share
+// ---------------------------------------------------------------------------------------------
+// One warp owns a strip of output byte-columns x one vertical segment.  Chunks of RB input rows are staged by TMA
+// (STAGES stages in flight, BOX_B bytes per staged row), the H pass writes them to a shared-memory ring of RING rows
+// (PITCH bytes each), and the systolic V pass reads them back, VB byte-columns per lane.  A family describes its
+// own choices in F (VB, RB, BOX_B, STAGES, PITCH); StripGeo adds what the pipeline derives from them.
+template <int A, int N, int D, class F>
+struct StripGeo : F {
+    static constexpr int TAPS = 2 * A;
+    static constexpr int U = lcm2(D);                             // input rows per V loop iteration (one ratio period, even)
+    static constexpr int REGIONS = 2;                             // ring regions of RB rows: V(c) reads region c and the tail of c-1
+    static constexpr int RING = REGIONS * F::RB;                  // intermediate rows kept in smem
+    static constexpr int STAGE_B = 128 * cdiv(F::RB * F::BOX_B, 128);   // TMA destinations must be 128-byte aligned
+    // the first row pushed by a segment is rs = D*pv0 - A + 1, so (row - A) mod D is static per chunk row
+    static constexpr int S0 = (((1 - 2 * A) % D) + D) % D;
+    static constexpr int YROWS = N * F::RB / D;                   // output rows completed per chunk
+    static_assert(F::RB % U == 0, "chunk must be a whole number of V loop iterations");
+    static_assert(TAPS - 1 <= F::RB, "tap rows must not reach further back than one ring region");
+    static_assert(F::BOX_B / 4 <= 256, "TMA box too wide");
+    static_assert(N <= 32, "phase table too large for kernel params");
+    static_assert(cdiv(S0 * N, D) + YROWS <= 32, "rows fixed per chunk must fit 32 bits");
+};
+
+template <class G>
+struct __align__(128) StripSmem {         // one per warp (a CTA is one warp)
+    uint8_t in[G::STAGES][G::STAGE_B];    // TMA destinations, row lr at lr * BOX_B
+    uint8_t ring[G::RING][G::PITCH];      // H-pass results (uint8), row r lives in slot (r - rs) % RING
+    unsigned long long full[G::STAGES];   // TMA stage filled
+};
+template <class G> constexpr size_t strip_smem_bytes() { return sizeof(StripSmem<G>) + 128; }
+
+// The rows of segment `seg`: ratio periods [pv0, pv1) -> output rows [ys, ye) (N*pv0 .. N*pv1 clipped to the band),
+// from the intermediate rows rs .. rs + 2a - 2 + D*(pv1 - pv0) pushed in nchunks chunks of RB rows.
+struct SegRows {
+    int ys, ye, rs, nchunks;
+};
+// false when the segment has no rows in the band (the CTA has nothing to do)
+template <int A, int N, int D, int RB>
+__device__ __forceinline__ bool segment_rows(const StripParams &p, int seg, SegRows &r) {
+    const int pv0 = p.vperiod0 + seg * p.seg_periods;
+    const int y_end_band = p.out_row0 + p.out_rows;
+    const int pv1 = min(pv0 + p.seg_periods, (y_end_band + N - 1) / N);
+    r.ys = max(N * pv0, p.out_row0);
+    r.ye = min(N * pv1, y_end_band);
+    if (r.ys >= r.ye) return false;
+    r.rs = D * pv0 - A + 1;                                   // first intermediate row pushed
+    const int nrows = D * (pv1 - pv0) + 2 * A - 1;            // rows to push
+    r.nchunks = (nrows + RB - 1) / RB;
+    return true;
+}
+
+// Systolic step of the V pass: every pending output row of the lane's VB byte-columns takes its next tap from the
+// converted ring row x, whose completing centre has residue s0 (c = D*t + s0).  acc[j - cnt0] = fma(x, w, acc[j]): the
+// FFMA's destination does the window shift, so a V loop iteration is one ratio period of straight-line code.  A row
+// takes its first tap from -guard_v; the rows that take their last tap land in res, in the order they complete.
+// Two columns per FFMA2 (one issue slot for two FMAs; same rounding as two FFMAs).
+// cnt0 = cnt<N, D>(s0), computed by the caller before it loads the ring row: computed here, it moves ptxas's
+// schedule of the V loop (headline kernel: 8104 -> 8112 instructions, one V loop 214 -> 221).
+template <int N, int D, int TAPS, int VB, int NSLOT, int CNTMAX>
+__device__ __forceinline__ void systolic_step(const float (&x)[VB], float (&acc)[NSLOT][VB], float (&res)[CNTMAX][VB], int s0,
+                                              int cnt0, float guard_v, const float *wtab) {
+    int q = 0;
+#pragma unroll
+    for (int dc = 0; dc < TAPS; dc++) {
+        const int sdc = (s0 + dc) % D;
+        const int k = TAPS - 1 - dc;
+#pragma unroll
+        for (int yr = ylo<N, D>(sdc); yr < yhi<N, D>(sdc); yr++) {
+            const int ph = (yr * D) % N;
+            if (ph == 0) continue;
+#ifdef LZB_ABL_TAPS     // ablation: only the first and the last LZB_ABL_TAPS/2 taps are computed
+            if (dc >= LZB_ABL_TAPS / 2 && dc < TAPS - LZB_ABL_TAPS / 2) { q++; continue; }
+#endif
+            const float2 wk2 = make_float2(wtab[ph * 8 + k], wtab[ph * 8 + k]);
+#pragma unroll
+            for (int i = 0; i < VB; i += 2) {
+                const float2 x2 = make_float2(x[i], x[i + 1]);
+                const float2 a2 = (dc < TAPS - 1) ? make_float2(acc[q][i], acc[q][i + 1]) : make_float2(-guard_v, -guard_v);
+                const float2 r2 = __ffma2_rn(x2, wk2, a2);
+                if (dc == 0) { res[q][i] = r2.x; res[q][i + 1] = r2.y; }
+                else { acc[q - cnt0][i] = r2.x; acc[q - cnt0][i + 1] = r2.y; }
+            }
+            q++;
+        }
+    }
+}
+
 using EncodeFn = CUresult (*)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                               const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                               CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -258,6 +347,30 @@ inline void set_strip_params(StripParams &p, const KParams &k, int vperiod0, int
 inline void fill_wtab(float *wtab, const FastHostTables &t, int A, int N) {
     for (int ph = 0; ph < N; ph++)
         for (int q = 0; q < 8; q++) wtab[ph * 8 + q] = q < 2 * A ? t.phase_w[ph * 2 * A + q] * 16777216.f : 0.f;
+}
+
+// The tail of a launch of either family: p arrives with the family's own fields set; this fills the fields every strip
+// kernel has, reports the shape and launches kern over strips x segments x frames, one warp per CTA.  `programmatic`:
+// the kernel may start before the previous kernel of the stream has finished (programmatic dependent launch).
+template <class G, class P, class Kernel>
+int launch_strips(Kernel kern, const CUtensorMap &map, P &p, const KParams &k, const FastHostTables &t, int strips,
+                  int vperiod0, SegPlan sp, long long ctas, bool programmatic, LaunchShape *shape, cudaStream_t s) {
+    set_strip_params(p, k, vperiod0, sp.seg_periods);
+    fill_wtab(p.wtab, t, k.a, k.scale_n);
+    p.strict_counter = k.strict_counter;
+    const dim3 grid(strips, sp.segs, k.n_frames);
+    *shape = LaunchShape{(int)grid.x, (int)grid.y, (int)grid.z, sp.seg_periods, G::RB, ctas};
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = grid;
+    cfg.blockDim = dim3(32);
+    cfg.dynamicSmemBytes = strip_smem_bytes<G>();
+    cfg.stream = s;
+    cudaLaunchAttribute attr{};
+    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr.val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = &attr;
+    cfg.numAttrs = programmatic ? 1 : 0;
+    return (int)cudaLaunchKernelEx(&cfg, kern, map, p);
 }
 
 }  // namespace

@@ -21,7 +21,7 @@ struct KParams {
     const int32_t *i0x; const float *wfx; const double *wdx;
     const int32_t *i0y; const float *wfy; const double *wdy;
     const float *phase_w;          // [scale_n][taps]
-    float guard;                   // ascending taps, |.|-sum bound (generic + first-generation kernels)
+    float guard;                   // ascending taps, |.|-sum bound (generic kernel)
     float guard_asc, guard_outer;  // sign-aware bounds: ascending order / outermost taps first (lanczos_v6.cu)
     int alias_rows, alias_top_row, alias_in_rows;
     unsigned flags;
@@ -71,13 +71,29 @@ __device__ __forceinline__ uint8_t quantise_f64(double x) {
     if (x < 0.0) return 0;
     return (uint8_t)(int)x;
 }
+// The same on one fp32 value, as F2I does it: truncate toward zero, then clamp to [0,255] (same result).
+__device__ __forceinline__ uint8_t quantise_f32(float x) {
+    const int i = __float2int_rz(x);
+    return (uint8_t)min(max(i, 0), 255);
+}
 
-// Exact restatement of the reference inner loop (full_TB.h:58-63): plain double multiply then add,
-// ascending tap order, no FMA contraction. Taps outside the image hold 0 (0*w adds +-0: same bits).
+// The reference's exact sum (full_TB.h:58-63 horizontal, :71-75 vertical): from 0.0, taps in ascending order, each a
+// plain double multiply then add, no FMA contraction.  The exact paths add their taps with exact_add (exact_taps in
+// fast_common.cuh spells the same step out, see there).
+// Taps outside the image hold 0 (0*w adds +-0: same bits).
+// (double)byte is formed as (2^52 + b) - 2^52 on the FP64 pipe: I2F.F64 runs on the slow XU unit.
+__device__ __forceinline__ double byte_to_double(int b) {
+    return __hiloint2double(0x43300000, b) - 4503599627370496.0;
+}
+__device__ __forceinline__ double exact_add(double sum, int byte, double w) {
+    return __dadd_rn(sum, __dmul_rn(byte_to_double(byte), w));
+}
+
+// One sample of the reference with `taps` weights w and tap(k) the k-th input byte.
 template <typename LoadTap>
 __device__ __forceinline__ uint8_t strict_sample(const double *w, int taps, LoadTap tap) {
     double sum = 0.0;
-    for (int k = 0; k < taps; k++) sum = __dadd_rn(sum, __dmul_rn((double)tap(k), w[k]));
+    for (int k = 0; k < taps; k++) sum = exact_add(sum, tap(k), w[k]);
     return quantise_f64(sum);
 }
 

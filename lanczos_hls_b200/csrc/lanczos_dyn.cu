@@ -1,22 +1,18 @@
 // lanczos_dyn.cu -- any-ratio member of the second-generation kernels (ratio period N <= 32, e.g. 17/10).
 //
-// Same structure as lanczos_v6.cu (see there for what each piece replaces in the reference): every warp owns one
-// strip of 128 output byte-columns, its own TMA stages, its own shared-memory ring of horizontal results and
-// its own mbarriers; rows stream through in chunks of RB input rows.  What differs:
+// The strip pipeline of lanczos_v6.cu (fast_common.cuh: TMA stages, ring, systolic V step), with strips of 128
+// output bytes, 4 per lane.  What differs:
 //   * H pass: a lane owns one 32-bit word of the strip (the same 4 byte-columns it owns in the V pass).  Its
 //     tap offsets and its 4 x 2a phase weights are fixed for the whole strip, so they are looked up once
 //     (plan tables i0x / polyphase table) and kept in registers; per row it does 4 x 2a byte loads from the
-//     staged input row, FHADD conversions and FFMAs.  No compile-time knowledge of the horizontal phase
-//     pattern is needed (17/10 RGB has a 51-byte period that fits no vector width).
-//   * V pass: the systolic scheme of lanczos_v6.cu with 4-byte columns; the vertical phase pattern is static
-//     (template N, D), the loop body is one ratio period (lcm(D,2) input rows).
+//     staged input row and FFMAs on the bytes read as fp32 denormals.  No compile-time knowledge of the horizontal
+//     phase pattern is needed (17/10 RGB has a 51-byte period that fits no vector width).
 //   * Phase-0 samples (output coordinate on an input sample) are always evaluated with the reference's double
 //     arithmetic: for ratios like 17/10 the coordinate xx/SCALE is not exactly integral in double, so the
 //     reference's weights there are 1-eps and +-1e-13 and its result is v or v-1 depending on all six taps.
 //     In the H pass these samples sit in fixed byte columns of the strip: one lane per (column, row) after the
 //     row loop.  In the V pass they are whole output rows (every N-th): v_fix_dyn.
-// Exactness of everything else: fp32 chains from -guard, truncation compared at +guard, exact double
-// re-evaluation (full_TB.h:58-63 / :71-75) when they differ.  MODE 1 = LANCZOS_FLAG_TOLERANCE_1LSB (V pass plain fp32).
+// MODE 1 = LANCZOS_FLAG_TOLERANCE_1LSB (V pass plain fp32).
 #include <algorithm>
 #include <atomic>
 #include <cmath>
@@ -42,27 +38,20 @@ struct DynParams : StripParams {
     unsigned long long *strict_counter;
 };
 
+// The dyn choices of the strip pipeline (StripGeo): strips of 128 output bytes, 4 per lane.
 template <int C, int A, int N, int D>
-struct GeoD {
+struct DynItems {
     static constexpr int VB = 4;                         // byte-columns per lane
-    static constexpr int SWB = 32 * VB;                  // strip width in output bytes = ring pitch
-    static constexpr int TAPS = 2 * A;
-    static constexpr int U = lcm2(D);                    // input rows per V loop iteration (one ratio period, even)
-    static constexpr int RB = U * cdiv(TAPS > 6 ? TAPS : 6, U);    // input rows per chunk (>= 2a - 1: see the ring)
-    static constexpr int REGIONS = 2;
-    static constexpr int RING = REGIONS * RB;
+    static constexpr int SWB = 32 * VB;                  // strip width in output bytes
+    static constexpr int PITCH = SWB;                    // ring pitch
+    static constexpr int RB = lcm2(D) * cdiv(2 * A > 6 ? 2 * A : 6, lcm2(D));   // input rows per chunk: whole V loop iterations, >= 6
     static constexpr int STAGES = 4;
     // input pixels a strip can touch: its (SWB/C + 2) output pixels span that many * D/N input pixels, plus taps
-    static constexpr int IN_PX = ((SWB / C + 2) * D) / N + 2 + TAPS;
+    static constexpr int IN_PX = ((SWB / C + 2) * D) / N + 2 + 2 * A;
     static constexpr int BOX_B = 16 * cdiv(IN_PX * C + 15, 16);   // + 15: the box starts on a 16-byte boundary
-    static constexpr int STAGE_B = 128 * cdiv(RB * BOX_B, 128);
-    static constexpr int S0 = (((1 - 2 * A) % D) + D) % D;
-    static constexpr int YROWS = N * RB / D;             // output rows completed per chunk
-    static_assert(TAPS - 1 <= RB, "tap rows must not reach further back than one ring region");
-    static_assert(BOX_B / 4 <= 256, "TMA box too wide");
-    static_assert(N <= 32, "phase table too large for kernel params");
-    static_assert(cdiv(S0 * N, D) + YROWS <= 32, "fix mask (bit per output row) too small");
 };
+template <int C, int A, int N, int D>
+using GeoD = StripGeo<A, N, D, DynItems<C, A, N, D>>;
 
 // fma.rn.f32 WITHOUT .ftz whatever the compilation flags say (-use_fast_math would flush the denormal operand)
 __device__ __forceinline__ float fma_keep_denormals(float a, float b, float c) {
@@ -78,14 +67,6 @@ __device__ __forceinline__ float2 ffma2_keep_denormals(float2 a, float2 b, float
         : "=f"(d.x), "=f"(d.y) : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y), "f"(c.x), "f"(c.y));
     return d;
 }
-
-template <class G>
-struct __align__(128) SmemD {             // one per warp
-    uint8_t in[G::STAGES][G::STAGE_B];    // TMA destinations, row lr at lr * BOX_B
-    uint8_t ring[G::RING][G::SWB];        // H-pass results (uint8), row r lives in slot (r - rs) % RING
-    unsigned long long full[G::STAGES];
-};
-
 
 // exact evaluation of the bytes of one output row whose fp32 truncation is in doubt, and of whole phase-0 rows
 struct VFixD {
@@ -141,10 +122,7 @@ __device__ __noinline__ int v_fix_dyn(const DynParams &p, const VFixD a) {
             if (!((need >> e) & 1u)) continue;
             double sum = 0.0;
 #pragma unroll
-            for (int k = 0; k < TAPS; k++) {
-                const double v = __hiloint2double(0x43300000, (int)((tw[k] >> (8 * e)) & 0xffu)) - 4503599627370496.0;
-                sum = __dadd_rn(sum, __dmul_rn(v, w[k]));
-            }
+            for (int k = 0; k < TAPS; k++) sum = exact_add(sum, (tw[k] >> (8 * e)) & 0xffu, w[k]);
             orow[e] = quantise_f64(sum);
             n_strict++;
         }
@@ -160,7 +138,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
     constexpr int NSLOT = nslot<N, D, TAPS>();
     constexpr int CNTMAX = cntmax<N, D>();
     extern __shared__ __align__(128) uint8_t smem_raw[];
-    SmemD<G> &sm = *reinterpret_cast<SmemD<G> *>(smem_raw);
+    StripSmem<G> &sm = *reinterpret_cast<StripSmem<G> *>(smem_raw);
 
     const int lane = threadIdx.x;
     const int strip = blockIdx.x, seg = blockIdx.y, frame = blockIdx.z;
@@ -171,15 +149,9 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
     const int row_bytes = p.out_w * C;
     const int valid_bytes = min(SWB, row_bytes - obyte0);     // > 0 by construction of the grid, multiple of 4
     const int xbyte0 = ((p.i0x[obyte0 / C] * C) >> 4) << 4;   // staged rows start here (16-byte aligned, may be < 0)
-    // vertical extent: periods [pv0, pv1) -> output rows [N*pv0, N*pv1), clipped to the band
-    const int pv0 = p.vperiod0 + seg * p.seg_periods;
-    const int y_end_band = p.out_row0 + p.out_rows;
-    const int pv1 = min(pv0 + p.seg_periods, (y_end_band + N - 1) / N);
-    const int ys = max(N * pv0, p.out_row0), ye = min(N * pv1, y_end_band);
-    if (ys >= ye) return;
-    const int rs = D * pv0 - A + 1;                           // first intermediate row pushed
-    const int nrows = D * (pv1 - pv0) + TAPS - 1;             // rows to push
-    const int nchunks = (nrows + RB - 1) / RB;
+    SegRows sr;
+    if (!segment_rows<A, N, D, RB>(p, seg, sr)) return;
+    const int ys = sr.ys, ye = sr.ye, rs = sr.rs, nchunks = sr.nchunks;
 
     uint32_t full0 = smem_u32(&sm.full[0]);
     asm volatile("" : "+r"(full0));
@@ -380,31 +352,8 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
                     const uint32_t w = *reinterpret_cast<const uint32_t *>(vit + u * SWB);
                     float x[VB];
                     word_to_f32x4(w, x[0], x[1], x[2], x[3]);
-                    // ---- systolic step: every pending output row takes its next tap from this row ----
                     float res[CNTMAX][VB];
-                    {
-                        int q = 0;
-#pragma unroll
-                        for (int dc = 0; dc < TAPS; dc++) {
-                            const int sdc = (s0 + dc) % D;
-                            const int k = TAPS - 1 - dc;
-#pragma unroll
-                            for (int yr = ylo<N, D>(sdc); yr < yhi<N, D>(sdc); yr++) {
-                                const int ph = (yr * D) % N;
-                                if (ph == 0) continue;
-                                const float2 wk2 = make_float2(p.wtab[ph * 8 + k], p.wtab[ph * 8 + k]);
-#pragma unroll
-                                for (int i = 0; i < VB; i += 2) {
-                                    const float2 x2 = make_float2(x[i], x[i + 1]);
-                                    const float2 a2 = (dc < TAPS - 1) ? make_float2(acc[q][i], acc[q][i + 1]) : make_float2(-guard_v, -guard_v);
-                                    const float2 r2 = __ffma2_rn(x2, wk2, a2);
-                                    if (dc == 0) { res[q][i] = r2.x; res[q][i + 1] = r2.y; }
-                                    else { acc[q - cnt0][i] = r2.x; acc[q - cnt0][i + 1] = r2.y; }
-                                }
-                                q++;
-                            }
-                        }
-                    }
+                    systolic_step<N, D, TAPS>(x, acc, res, s0, cnt0, guard_v, p.wtab);
                     // ---- rows that received their last tap ----
                     {
                         int q = 0;
@@ -496,16 +445,14 @@ int launch_dyn_one(const KParams &k, const FastHostTables &t, LaunchShape *shape
     CUtensorMap map;
     if (!encode_input_map(&map, k, G::BOX_B, G::RB)) return -1;
     auto kern = lanczos_dyn_kernel<C, A, N, D, MODE>;
-    const size_t smem = sizeof(SmemD<G>) + 128;
     static std::atomic<int> ctas_per_sm[64] = {};
-    const Residency res = resident_ctas(ctas_per_sm, kern, smem);
+    const Residency res = resident_ctas(ctas_per_sm, kern, strip_smem_bytes<G>());
     if (res.ctas == 0) return -1;
     const int vperiod0 = k.out_row0 / N;
     const int vperiods = (k.out_row0 + k.out_rows + N - 1) / N - vperiod0;
     const SegPlan sp = plan_segments(vperiods, D, A, G::RB, (long long)strips * k.n_frames, res.ctas, 512);
 
     DynParams p{};
-    set_strip_params(p, k, vperiod0, sp.seg_periods);
     p.i0x = k.i0x; p.wdx = k.wdx; p.wdy = k.wdy;
     p.guard = k.guard_asc;
     // the cheap phase-0 test needs: coordinates exactly integral in double on both axes (then the weights there are
@@ -519,13 +466,8 @@ int launch_dyn_one(const KParams &k, const FastHostTables &t, LaunchShape *shape
         }
         p.p0_filter = (A == 3 && km == 0x11 && small && t.exact_x && t.exact_y) ? 1 : 0;
     }
-    fill_wtab(p.wtab, t, A, N);
-    p.strict_counter = k.strict_counter;
-
-    dim3 grid(strips, sp.segs, k.n_frames);
-    *shape = LaunchShape{(int)grid.x, (int)grid.y, (int)grid.z, sp.seg_periods, G::RB, res.ctas};
-    kern<<<grid, 32, smem, s>>>(map, p);
-    return (int)cudaGetLastError();
+    // stream order: the kernel is not written for programmatic dependent launch (no griddepcontrol)
+    return launch_strips<G>(kern, map, p, k, t, strips, vperiod0, sp, res.ctas, false, shape, s);
 }
 
 }  // namespace

@@ -11,7 +11,7 @@
 // Arithmetic: fp32 FMA with per-coordinate float weights.  Whenever the fp32 sum lies within
 // `guard` (a rigorous bound on the fp32-vs-double error, plan.cpp) of an integer 1..255, the
 // sample is re-evaluated exactly like the reference does (double multiply, double add, ascending
-// taps, kernels.cuh strict_sample) so the truncated result is bit-identical.
+// taps, kernels.cuh exact_add) so the truncated result is bit-identical.
 #include "kernels.cuh"
 
 namespace lzb {
@@ -27,11 +27,6 @@ constexpr int GT_IN_COLS = GT_W + 8;
 __device__ __forceinline__ bool near_integer(float s, float guard) {
     const float r = rintf(s);
     return fabsf(s - r) < guard && r >= 1.f && r <= 255.f;
-}
-
-__device__ __forceinline__ uint8_t quantise_f32(float s) {
-    s = fminf(fmaxf(s, 0.f), 255.f);  // full_TB.h:30-33
-    return (uint8_t)(int)s;           // full_TB.h:35 truncation
 }
 
 template <int C>
@@ -159,7 +154,7 @@ __global__ void __launch_bounds__(128) lanczos_alias_rows_kernel(const KParams p
             const int i = first + k;
             if (i < 0 || i >= p.in_h) continue;  // full_TB.h:72 clips the window
             const uint8_t v = (i > yy) ? fin[i & 7] : (cached ? T[i] : mid(i));
-            sum = __dadd_rn(sum, __dmul_rn((double)v, wy[k]));
+            sum = exact_add(sum, v, wy[k]);
         }
         const uint8_t q = quantise_f64(sum);
         fin[yy & 7] = q;

@@ -67,10 +67,10 @@ struct V6Params : StripParams {
 __host__ __device__ constexpr int cmax6(int a, int b) { return a > b ? a : b; }
 __host__ __device__ constexpr int gcd6(int a, int b) { return b == 0 ? a : gcd6(b, a % b); }
 
+// The v6 choices of the strip pipeline (StripGeo): H items of PH ratio periods, strips of SWV output bytes.
 template <int C, int A, int N, int D, int PH, int MODE>
-struct Geo6 {
+struct V6Items {
     static constexpr int VB = 8;                        // byte-columns per V thread
-    static constexpr int TAPS = 2 * A;
     static constexpr int IN_B = PH * D * C;             // input bytes owned by one H item
     static constexpr int OUT_B = PH * N * C;            // output bytes produced by one H item
     static constexpr int NI = PH * (N - 1) * C;         // interpolated (phase != 0) samples per H item
@@ -93,7 +93,7 @@ struct Geo6 {
     static constexpr int SWV = (MODE == 1) ? 5 * OUT_B : 32 * VB;
     static constexpr int VOFF_MAX = OUT_B - gcd6(SWV, OUT_B);     // largest offset of a strip inside its first H item
     static constexpr int MAX_GROUPS = cdiv(VOFF_MAX + SWV, OUT_B);   // H items per row of a warp's strip (6 for 48-byte items)
-    static constexpr int SW_MAX = MAX_GROUPS * OUT_B;             // ring pitch in bytes (288)
+    static constexpr int PITCH = MAX_GROUPS * OUT_B;              // ring pitch in bytes (288)
     // a TMA box must start on a 16-byte boundary of the row: strips whose input starts 8 bytes off get a box
     // that starts 8 bytes early (XSHIFT_MAX extra bytes per row)
     static constexpr int XSHIFT_MAX = (IN_B % 16 != 0) ? 8 : 0;   // H items start at multiples of IN_B input bytes
@@ -101,33 +101,15 @@ struct Geo6 {
     static constexpr int HB = 32 / MAX_GROUPS;                    // rows one round of H items covers (one item per lane)
     static constexpr int HROUNDS = 2;                             // H rounds per chunk
     static constexpr int RB = HB * HROUNDS;                       // input rows per chunk
-    static constexpr int REGIONS = 2;                             // ring regions of RB rows: V(c) reads region c and the tail of c-1
-    static constexpr int RING = REGIONS * RB;                     // intermediate rows kept in smem
-    static constexpr int STAGE_B = 128 * ((RB * BOX_B + 127) / 128);  // TMA destinations must be 128-byte aligned
     static constexpr int STAGES = 3;                              // TMA stages in flight
-    // the first row pushed by a segment is rs = D*pv0 - A + 1, so (row - A) mod D is static per chunk row
-    static constexpr int S0 = (((1 - 2 * A) % D) + D) % D;
-    static constexpr int U = lcm2(D);                             // rows per V loop iteration (even: filter delay line parity)
-    static constexpr int YROWS = N * RB / D;                      // output rows completed per chunk
     static_assert(IN_B % 8 == 0, "H item input must be 8-byte aligned");
     static_assert(OUT_B % 16 == 0, "H item output must be 16-byte aligned");
     static_assert(OUT_B % VB == 0 && HB * MAX_GROUPS <= 32 && HB >= 1, "one H item per lane and round, one V column per lane");
-    static_assert(RB % U == 0, "chunk must be a whole number of V loop iterations");
-    static_assert(TAPS - 1 <= RB, "tap rows must not reach further back than one ring region");
-    static_assert(BOX_B / 4 <= 256, "TMA box too wide");
-    static_assert(N <= 32, "phase table too large for kernel params");
-    static_assert(YROWS + N * (S0 + A + 1) / D + 2 <= 64, "fix mask (bit per output row) too small");
-    static_assert(cdiv(S0 * N, D) + YROWS <= 32, "rows fixed per chunk must fit 32 bits");
     static_assert(ND <= 31, "H fix mask (bit per packed word) too small");
     static_assert(D <= 2, "phase-0 filter delay line assumes the +-2 rows are phase-0 centres themselves");
 };
-
-template <class G>
-struct __align__(128) Smem6 {             // one per CTA
-    uint8_t in[G::STAGES][G::STAGE_B];    // TMA destinations, row lr at lr * BOX_B
-    uint8_t ring[G::RING][G::SW_MAX];     // H-pass results (uint8), row r lives in slot (r - rs) % RING
-    unsigned long long full[G::STAGES];   // TMA stage filled
-};
+template <int C, int A, int N, int D, int PH, int MODE>
+using Geo6 = StripGeo<A, N, D, V6Items<C, A, N, D, PH, MODE>>;
 
 // Four bytes from up to four source words, positions known at compile time after unrolling: one PRMT for
 // the first two distinct sources, one more per further source.
@@ -166,12 +148,6 @@ __device__ __forceinline__ uint32_t gather4(const uint32_t (&arr)[NSRC], const i
     return res;
 }
 
-// double_to_uint8 (full_TB.h:29-37) on one fp32 value, as F2IP does it: clamp to [0,255], truncate toward zero
-__device__ __forceinline__ uint32_t quantise_f32(float x) {
-    const int i = __float2int_rz(x);
-    return (uint32_t)min(max(i, 0), 255);
-}
-
 // summation order of the H-pass chains: outermost (smallest) weights first, the two central taps last
 template <int TAPS> __host__ __device__ constexpr int tap_order6(int i) { return (i & 1) ? TAPS - 1 - i / 2 : i / 2; }
 
@@ -205,7 +181,7 @@ __device__ __forceinline__ uint32_t lds_u8(uint32_t a) {
 
 // ---------------------------------------------------------------------------------------------
 // slow paths: executed by the thread that found a sample in doubt, kept out of line so that the hot loop
-// stays small.  Both restate full_TB.h:58-63 / :71-75 exactly (exact_taps).
+// stays small.  Both restate full_TB.h:58-63 / :71-75 exactly (exact_add).
 // ---------------------------------------------------------------------------------------------
 struct HFixArgs {
     const uint8_t *in_row;    // staged input row of the item (byte 0 = ibyte0 - PAD_L)
@@ -271,8 +247,7 @@ __device__ __forceinline__ uint32_t exact_ring(uint32_t col_e, int slot0, W weig
     for (int k = 0; k < NT; k++) {
         int sl = slot0 + k;
         if (sl >= RING) sl -= RING;
-        const double v = __hiloint2double(0x43300000, (int)lds_u8(col_e + sl * SWM)) - 4503599627370496.0;
-        sum = __dadd_rn(sum, __dmul_rn(v, weight(k)));
+        sum = exact_add(sum, lds_u8(col_e + sl * SWM), weight(k));
     }
     return quantise_f64(sum);
 }
@@ -458,11 +433,7 @@ __device__ __noinline__ void alias_fix(const V6Params &p, const AliasArgs a) {
             const uint2 v = (i > yy) ? fin[i] : *reinterpret_cast<const uint2 *>(a.col + (i + A - 1) * SWM);
             const double w = (p.uniform_y && N <= 8) ? p.wdtab[ph * 8 + k] : p.wdy[(long long)yy * TAPS + k];
 #pragma unroll
-            for (int e = 0; e < VB; e++) {
-                const uint32_t word = e < 4 ? v.x : v.y;
-                const double vd = __hiloint2double(0x43300000, (int)((word >> (8 * (e & 3))) & 0xffu)) - 4503599627370496.0;
-                sum[e] = __dadd_rn(sum[e], __dmul_rn(vd, w));
-            }
+            for (int e = 0; e < VB; e++) sum[e] = exact_add(sum[e], ((e < 4 ? v.x : v.y) >> (8 * (e & 3))) & 0xffu, w);
         }
         uint32_t q[VB];
 #pragma unroll
@@ -483,7 +454,7 @@ __global__ void __launch_bounds__(32, 16)
 lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ V6Params p) {
     using G = Geo6<C, A, N, D, PH, MODE>;
     constexpr int TAPS = G::TAPS;
-    constexpr int SWM = G::SW_MAX;
+    constexpr int SWM = G::PITCH;
     constexpr int VB = G::VB;
     constexpr int CEN = A - 1;                                  // centre tap of a phase-0 sample
     constexpr int NSLOT = nslot<N, D, TAPS>();
@@ -497,7 +468,7 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
     constexpr int VU = G::U;
     static_assert(KM == 0 || (A == 3 && KM == 0x11), "phase-0 row filter is written for the +-2 residues of a = 3");
     extern __shared__ __align__(128) uint8_t smem_raw[];
-    Smem6<G> &sm = *reinterpret_cast<Smem6<G> *>(smem_raw);
+    StripSmem<G> &sm = *reinterpret_cast<StripSmem<G> *>(smem_raw);
     const int tid = threadIdx.x;
     const int strip = blockIdx.x, seg = blockIdx.y, frame = blockIdx.z;
     // programmatic dependent launch: let the next kernel of the stream start as soon as SMs free up; unless the caller
@@ -518,15 +489,9 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
     const int hvalid = min(groups * G::OUT_B, row_bytes - obyte0);   // bytes of the H items inside the image
     const int ibyte0 = (obyte0 / (N * C)) * (D * C);          // first input byte column of the H items
     const int xshift = (ibyte0 - G::PAD_L) & 15;              // 0 or 8: the TMA box starts that many bytes early
-    // vertical extent: periods [pv0, pv1) -> output rows [N*pv0, N*pv1), clipped to the band
-    const int pv0 = p.vperiod0 + seg * p.seg_periods;
-    const int y_end_band = p.out_row0 + p.out_rows;
-    const int pv1 = min(pv0 + p.seg_periods, (y_end_band + N - 1) / N);
-    const int ys = max(N * pv0, p.out_row0), ye = min(N * pv1, y_end_band);
-    if (ys >= ye) return;
-    const int rs = D * pv0 - A + 1;                           // first intermediate row pushed
-    const int nrows = D * (pv1 - pv0) + TAPS - 1;             // rows to push
-    const int nchunks = (nrows + G::RB - 1) / G::RB;
+    SegRows sr;
+    if (!segment_rows<A, N, D, G::RB>(p, seg, sr)) return;
+    const int ys = sr.ys, ye = sr.ye, rs = sr.rs, nchunks = sr.nchunks;
 
     uint32_t full0 = smem_u32(&sm.full[0]);
     // keep the address in a register: without this it is re-derived from the CTA's shared window at every use
@@ -795,35 +760,8 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
                     x[0] = h2_lo_to_f32(h0); x[1] = h2_hi_to_f32(h0); x[2] = h2_lo_to_f32(h1); x[3] = h2_hi_to_f32(h1);
                     x[4] = h2_lo_to_f32(h2); x[5] = h2_hi_to_f32(h2); x[6] = h2_lo_to_f32(h3); x[7] = h2_hi_to_f32(h3);
 #endif
-                    // ---- systolic step: every pending output row takes its next tap from this row ----
                     float res[CNTMAX][VB];
-                    {
-                        int q = 0;
-#pragma unroll
-                        for (int dc = 0; dc < TAPS; dc++) {
-                            const int sdc = (s0 + dc) % D;
-                            const int k = TAPS - 1 - dc;
-#pragma unroll
-                            for (int yr = ylo<N, D>(sdc); yr < yhi<N, D>(sdc); yr++) {
-                                const int ph = (yr * D) % N;
-                                if (ph == 0) continue;
-#ifdef LZB_ABL_TAPS             // ablation: only the first and the last LZB_ABL_TAPS/2 taps are computed
-                                if (dc >= LZB_ABL_TAPS / 2 && dc < TAPS - LZB_ABL_TAPS / 2) { q++; continue; }
-#endif
-                                // two columns per FFMA2 (one issue slot for two FMAs; same rounding as two FFMAs)
-                                const float2 wk2 = make_float2(p.wtab[ph * 8 + k], p.wtab[ph * 8 + k]);
-#pragma unroll
-                                for (int i = 0; i < VB; i += 2) {
-                                    const float2 x2 = make_float2(x[i], x[i + 1]);
-                                    const float2 a2 = (dc < TAPS - 1) ? make_float2(acc[q][i], acc[q][i + 1]) : make_float2(-guard_v, -guard_v);
-                                    const float2 r2 = __ffma2_rn(x2, wk2, a2);
-                                    if (dc == 0) { res[q][i] = r2.x; res[q][i + 1] = r2.y; }
-                                    else { acc[q - cnt0][i] = r2.x; acc[q - cnt0][i + 1] = r2.y; }
-                                }
-                                q++;
-                            }
-                        }
-                    }
+                    systolic_step<N, D, TAPS>(x, acc, res, s0, cnt0, guard_v, p.wtab);
                     auto store_row = [&](int yoff, const uint2 qv) {
 #ifdef LZB_ABL_NOSTORE
                         if (qv.x != 0x12345678u) return;
@@ -1006,18 +944,18 @@ int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kerne
     CUtensorMap map;
     if (!encode_input_map(&map, k, G::BOX_B, G::RB)) return -1;
     auto kern = lanczos_v6_kernel<C, A, N, D, PH, KM, MODE, ST64>;
-    const size_t smem = sizeof(Smem6<G>) + 128;
     static std::atomic<int> ctas_per_sm[64] = {};
-    const Residency res = resident_ctas(ctas_per_sm, kern, smem);
+    const Residency res = resident_ctas(ctas_per_sm, kern, strip_smem_bytes<G>());
     if (res.ctas == 0) return -1;
     const int strips = (k.out_w * C + G::SWV - 1) / G::SWV;   // one strip of SWV = 256 output bytes per warp
     const long long cols = (long long)strips * k.n_frames;
     const int vperiod0 = k.out_row0 / N;
     const int vperiods = (k.out_row0 + k.out_rows + N - 1) / N - vperiod0;
-    const SegPlan sp = plan_v6_segments(vperiods, D, A, G::RB, cols, res.ctas, res.sms, (k.flags & LANCZOS_FLAG_INDEPENDENT) != 0);
+    const bool independent = (k.flags & LANCZOS_FLAG_INDEPENDENT) != 0;
+    const SegPlan sp = plan_v6_segments(vperiods, D, A, G::RB, cols, res.ctas, res.sms, independent);
 
     V6Params p{};
-    set_strip_params(p, k, vperiod0, sp.seg_periods);
+    p.independent = independent ? 1 : 0;
     p.wdx = k.wdx; p.wdy = k.wdy;
     p.guard_h = k.guard_outer; p.guard_v = k.guard_asc;
     p.uniform_x = t.uniform_x; p.uniform_y = t.uniform_y;
@@ -1033,29 +971,9 @@ int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kerne
     }
     for (int i = 0; i < 8; i++) p.align_k[i] = i < 2 * A ? t.align_k[i] : 0.f;
     for (int i = 0; i < 5; i++) p.p0c[i] = t.p0_chain ? t.p0_chain[i] * 16777216.f : 0.f;   // x 2^24, exact
-    fill_wtab(p.wtab, t, A, N);
     for (int ph = 0; ph < N && ph < 8; ph++)
         for (int q = 0; q < 8; q++) p.wdtab[ph * 8 + q] = q < 2 * A ? t.phase_wd[ph * 2 * A + q] : 0.0;
-    p.strict_counter = k.strict_counter;
-
-    dim3 grid(strips, sp.segs, k.n_frames);
-    *shape = LaunchShape{(int)grid.x, (int)grid.y, (int)grid.z, sp.seg_periods, G::RB, res.ctas};
-    p.independent = (k.flags & LANCZOS_FLAG_INDEPENDENT) ? 1 : 0;
-    if (p.independent) {
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = grid;
-        cfg.blockDim = dim3(32);
-        cfg.dynamicSmemBytes = smem;
-        cfg.stream = s;
-        cudaLaunchAttribute attr{};
-        attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr.val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = &attr;
-        cfg.numAttrs = 1;
-        return (int)cudaLaunchKernelEx(&cfg, kern, map, p);
-    }
-    kern<<<grid, 32, smem, s>>>(map, p);
-    return (int)cudaGetLastError();
+    return launch_strips<G>(kern, map, p, k, t, strips, vperiod0, sp, res.ctas, independent, shape, s);
 }
 
 }  // namespace
