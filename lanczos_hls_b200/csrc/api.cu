@@ -52,6 +52,10 @@ struct DeviceGuard {
         if (prev >= 0) cudaSetDevice(prev);
     }
 };
+// `dev` is the current device until the end of the enclosing scope, or the function returns LANCZOS_ERR_CUDA
+#define SET_DEVICE(dev)                     \
+    DeviceGuard device_guard__(dev);        \
+    if (!device_guard__.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice")
 
 // Non-blocking streams of the host drivers, kept per device between calls (creating and destroying a stream
 // costs tens of microseconds).  A lease synchronises its stream before handing it back, on every exit path,
@@ -120,16 +124,23 @@ cudaError_t copy_rows(void *dst, long long dpitch, const void *src, long long sp
 }
 
 // ---- host plans (tables only, no device memory), cached per geometry ---------------------------
+// Plans are shared by callers with different row pitches: the key has none, and nothing may read the pitches of the
+// caller that built a plan.  Device plans are cached per (geometry, device).
 using HostKey = std::tuple<int, int, int, int, int, int, int, int, unsigned>;
+using PlanKey = std::pair<HostKey, int>;
+constexpr unsigned kPlanFlagMask = LANCZOS_FLAG_NO_ALIAS;  // flags that change the tables
+HostKey plan_key(const lanczos_desc &r) {
+    return {r.in_w, r.in_h, r.out_w, r.out_h, r.channels, r.a, r.scale_n, r.scale_d, r.flags & kPlanFlagMask};
+}
+
 std::mutex g_host_plan_mutex;
 std::map<HostKey, std::shared_ptr<const Plan>> g_host_plans;
-constexpr unsigned kPlanFlagMask = LANCZOS_FLAG_NO_ALIAS;  // flags that change the tables
 
 int get_host_plan(const lanczos_desc *desc, std::shared_ptr<const Plan> *out) {
     lanczos_desc r;
     int rc = resolve_desc(desc, &r);
     if (rc != LANCZOS_OK) return rc;
-    HostKey key{r.in_w, r.in_h, r.out_w, r.out_h, r.channels, r.a, r.scale_n, r.scale_d, r.flags & kPlanFlagMask};
+    HostKey key = plan_key(r);
     {
         std::lock_guard<std::mutex> lock(g_host_plan_mutex);
         auto it = g_host_plans.find(key);
@@ -141,7 +152,6 @@ int get_host_plan(const lanczos_desc *desc, std::shared_ptr<const Plan> *out) {
     auto p = std::make_shared<Plan>();
     rc = build_plan(&r, p.get());   // O(out_w + out_h) libm calls: outside the lock
     if (rc != LANCZOS_OK) return rc;
-    // plans are shared by callers with different row pitches: nothing may read the pitches of the first caller
     p->d.in_pitch = p->d.out_pitch = 0;
     std::lock_guard<std::mutex> lock(g_host_plan_mutex);
     auto ins = g_host_plans.emplace(key, p);
@@ -153,13 +163,12 @@ int get_host_plan(const lanczos_desc *desc, std::shared_ptr<const Plan> *out) {
 struct DevicePlan {
     std::shared_ptr<const Plan> host_ref;
     const Plan &host() const { return *host_ref; }
-    std::mutex stats_mutex;   // the strict-sample counter is one per plan: calls that count take turns
+    mutable std::mutex stats_mutex;   // the strict-sample counter is one per plan: calls that count take turns
     int device = 0;
     void *blob = nullptr;  // one allocation holding every table
-    const int32_t *i0x = nullptr, *i0y = nullptr;
-    const float *wfx = nullptr, *wfy = nullptr, *phase_w = nullptr;
-    const double *wdx = nullptr, *wdy = nullptr;
     unsigned long long *strict_counter = nullptr;
+    KParams launch{};      // every launch parameter that depends on the plan alone
+    FastHostTables fast{};
     ~DevicePlan() {
         if (blob) {
             DeviceGuard g(device);
@@ -168,18 +177,16 @@ struct DevicePlan {
     }
 };
 
-using PlanKey = std::tuple<int, int, int, int, int, int, int, int, unsigned, int>;
 std::mutex g_plan_mutex;
 std::map<PlanKey, std::shared_ptr<DevicePlan>> g_plans;
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-int get_plan(const lanczos_desc *desc, int device, std::shared_ptr<DevicePlan> *out) {
-    lanczos_desc r;
-    int rc = resolve_desc(desc, &r);
+// The plan of *desc on `device`, and *r = *desc resolved: the caller's pitches, which plans do not carry.
+int get_plan(const lanczos_desc *desc, int device, lanczos_desc *r, std::shared_ptr<DevicePlan> *out) {
+    int rc = resolve_desc(desc, r);
     if (rc != LANCZOS_OK) return rc;
-    PlanKey key{r.in_w, r.in_h, r.out_w, r.out_h, r.channels, r.a, r.scale_n, r.scale_d,
-                r.flags & kPlanFlagMask, device};
+    const PlanKey key{plan_key(*r), device};
     std::lock_guard<std::mutex> lock(g_plan_mutex);
     auto it = g_plans.find(key);
     if (it != g_plans.end()) {
@@ -188,7 +195,7 @@ int get_plan(const lanczos_desc *desc, int device, std::shared_ptr<DevicePlan> *
     }
     auto dp = std::make_shared<DevicePlan>();
     dp->device = device;
-    rc = get_host_plan(&r, &dp->host_ref);
+    rc = get_host_plan(r, &dp->host_ref);
     if (rc != LANCZOS_OK) return rc;
     const Plan &h = dp->host();
     // layout of the single device blob (each table 256-byte aligned)
@@ -209,14 +216,21 @@ int get_plan(const lanczos_desc *desc, int device, std::shared_ptr<DevicePlan> *
     CU(cudaMalloc(&dp->blob, off));
     CU(cudaMemcpy(dp->blob, stage.data(), off, cudaMemcpyHostToDevice));
     auto *b = (uint8_t *)dp->blob;
-    dp->wdx = (const double *)(b + o_wdx);
-    dp->wdy = (const double *)(b + o_wdy);
-    dp->wfx = (const float *)(b + o_wfx);
-    dp->wfy = (const float *)(b + o_wfy);
-    dp->i0x = (const int32_t *)(b + o_i0x);
-    dp->i0y = (const int32_t *)(b + o_i0y);
-    dp->phase_w = (const float *)(b + o_ph);
     dp->strict_counter = (unsigned long long *)(b + o_cnt);
+    KParams &k = dp->launch;
+    k.in_w = h.d.in_w; k.in_h = h.d.in_h; k.out_w = h.d.out_w; k.out_h = h.d.out_h;
+    k.channels = h.d.channels; k.a = h.d.a; k.taps = h.taps;
+    k.scale_n = h.d.scale_n; k.scale_d = h.d.scale_d;
+    k.i0x = (const int32_t *)(b + o_i0x); k.wfx = (const float *)(b + o_wfx); k.wdx = (const double *)(b + o_wdx);
+    k.i0y = (const int32_t *)(b + o_i0y); k.wfy = (const float *)(b + o_wfy); k.wdy = (const double *)(b + o_wdy);
+    k.phase_w = (const float *)(b + o_ph);
+    k.guard = h.guard;
+    k.guard_asc = h.guard_asc;
+    k.guard_outer = h.guard_outer;
+    k.alias_rows = h.alias_rows; k.alias_top_row = h.alias_top_row; k.alias_in_rows = h.alias_in_rows;
+    dp->fast = FastHostTables{h.phase_w.data(), h.phase_wd.data(), h.align_k.data(), h.x.aligned_exact ? 1 : 0,
+                              h.y.aligned_exact ? 1 : 0, h.x.uniform_phase ? 1 : 0, h.y.uniform_phase ? 1 : 0,
+                              h.x.i0.data(), h.p0_chain_ok ? h.p0_chain : nullptr};
     g_plans[key] = dp;
     *out = dp;
     return LANCZOS_OK;
@@ -269,106 +283,154 @@ struct Scratch {  // RAII device buffer from the pool (current device must be `d
 // ---- core launch ----------------------------------------------------------------------------
 constexpr int kMaxGridFrames = 65535;
 
-// the first main launch of a call (main_launches is counted by the caller)
-void set_launch(const LaunchShape &sh) {
-    g_launch.grid_x = sh.grid_x;
-    g_launch.grid_y = sh.grid_y;
-    g_launch.grid_z = sh.grid_z;
-    g_launch.seg_periods = sh.seg_periods;
-    g_launch.chunk_rows = sh.chunk_rows;
-    g_launch.resident_ctas = sh.resident_ctas;
+// CUDA caps a grid's y and z dimensions at 65,535 (frames are gridDim.z of the main kernels and gridDim.y of the
+// alias-rows kernel): larger batches run as consecutive frame groups, each with its own tensor map and plan.
+// main(g0, frames, &kernel_id, &shape) launches the main kernel of frames [g0, g0 + frames), then() what else the group
+// needs; both return LANCZOS_OK or an error code.  The counters of the main launches are kept here.
+template <typename Main, typename Then>
+int launch_frame_groups(int n_frames, Main main, Then then) {
+    for (int g0 = 0; g0 < n_frames; g0 += kMaxGridFrames) {
+        int kid = 0;
+        LaunchShape shape;
+        int rc = main(g0, std::min(kMaxGridFrames, n_frames - g0), &kid, &shape);
+        if (rc != LANCZOS_OK) return rc;
+        g_stats.kernel_launches++;
+        g_stats.kernel_id = kid;
+        if (g0 == 0)   // lanczos_launch describes the first main launch of a call
+            g_launch = lanczos_launch{shape.grid_x, shape.grid_y, shape.grid_z, shape.seg_periods, shape.chunk_rows, 0,
+                                      shape.resident_ctas};
+        g_launch.main_launches++;
+        rc = then();
+        if (rc != LANCZOS_OK) return rc;
+    }
+    return LANCZOS_OK;
 }
 
-int run_device(const DevicePlan &dp, unsigned flags, const uint8_t *d_in, uint8_t *d_out, int n_frames,
-               long long in_frame_stride, long long out_frame_stride, int out_row0, int out_rows,
-               int in_row0, int in_rows, long long in_pitch, long long out_pitch, cudaStream_t s) {
+// Output rows [out_row0, out_row0 + out_rows) of a frame, computed from its input rows [in_row0, in_row0 + in_rows).
+struct Band {
+    int out_row0, out_rows, in_row0, in_rows;
+};
+Band whole_frame(const Plan &h) { return {0, h.d.out_h, 0, h.d.in_h}; }
+
+// One call of the kernels: `band` of n_frames frames; in and out point at the band's first rows in frame 0.
+struct DeviceCall {
+    const uint8_t *in;
+    uint8_t *out;
+    long long in_pitch, out_pitch;
+    Band band;
+    int n_frames = 1;
+    long long in_frame_stride = 0, out_frame_stride = 0;
+};
+
+int run_device(const DevicePlan &dp, unsigned flags, const DeviceCall &c, cudaStream_t s) {
     const Plan &h = dp.host();
-    KParams p{};
-    p.in = d_in;
-    p.out = d_out;
-    p.in_pitch = in_pitch;
-    p.out_pitch = out_pitch;
-    p.in_frame_stride = in_frame_stride;
-    p.out_frame_stride = out_frame_stride;
-    p.n_frames = n_frames;
-    p.in_w = h.d.in_w; p.in_h = h.d.in_h; p.out_w = h.d.out_w; p.out_h = h.d.out_h;
-    p.channels = h.d.channels; p.a = h.d.a; p.taps = h.taps;
-    p.scale_n = h.d.scale_n; p.scale_d = h.d.scale_d;
-    p.out_row0 = out_row0; p.out_rows = out_rows; p.in_row0 = in_row0; p.in_rows = in_rows;
-    p.i0x = dp.i0x; p.wfx = dp.wfx; p.wdx = dp.wdx;
-    p.i0y = dp.i0y; p.wfy = dp.wfy; p.wdy = dp.wdy;
-    p.phase_w = dp.phase_w;
-    p.guard = h.guard;
-    p.guard_asc = h.guard_asc;
-    p.guard_outer = h.guard_outer;
-    p.alias_rows = h.alias_rows; p.alias_top_row = h.alias_top_row; p.alias_in_rows = h.alias_in_rows;
+    const Band &b = c.band;
+    KParams p = dp.launch;
+    p.in_pitch = c.in_pitch;
+    p.out_pitch = c.out_pitch;
+    p.in_frame_stride = c.in_frame_stride;
+    p.out_frame_stride = c.out_frame_stride;
+    p.out_row0 = b.out_row0; p.out_rows = b.out_rows; p.in_row0 = b.in_row0; p.in_rows = b.in_rows;
     p.flags = flags;
     const bool count = g_stats_enabled.load(std::memory_order_relaxed);
     p.strict_counter = count ? dp.strict_counter : nullptr;
     g_stats = lanczos_stats{};
     g_launch = lanczos_launch{};
-    if (n_frames <= 0 || out_rows <= 0) return LANCZOS_OK;
+    if (c.n_frames <= 0 || b.out_rows <= 0) return LANCZOS_OK;
     // counting calls are synchronous and take turns on the plan's counter (several host threads or streams may share a plan)
     std::unique_lock<std::mutex> stats_lock;
     if (count) {
-        stats_lock = std::unique_lock<std::mutex>(const_cast<DevicePlan &>(dp).stats_mutex);
+        stats_lock = std::unique_lock<std::mutex>(dp.stats_mutex);
         CU(cudaMemsetAsync(dp.strict_counter, 0, 8, s));
     }
-
-    // CUDA caps a grid's y and z dimensions at 65,535 (frames are gridDim.z of the main kernels and gridDim.y of the
-    // alias-rows kernel): larger batches run as consecutive frame groups, each with its own tensor map and plan
-    for (int g0 = 0; g0 < n_frames; g0 += kMaxGridFrames) {
-        p.in = d_in + (long long)g0 * in_frame_stride;
-        p.out = d_out + (long long)g0 * out_frame_stride;
-        p.n_frames = std::min(kMaxGridFrames, n_frames - g0);
-        int kid = 0, alias_done = 0;
-        int frc = -1;
-        LaunchShape shape;
-        if (!(flags & LANCZOS_FLAG_GENERIC_KERNEL)) {
-            FastHostTables t{h.phase_w.data(), h.phase_wd.data(), h.align_k.data(), h.x.aligned_exact ? 1 : 0,
-                             h.y.aligned_exact ? 1 : 0, h.x.uniform_phase ? 1 : 0, h.y.uniform_phase ? 1 : 0, h.x.i0.data(),
-                             h.p0_chain_ok ? h.p0_chain : nullptr};
-            frc = launch_v6(p, t, &kid, &alias_done, &shape, s);
-            if (frc < 0) frc = launch_dyn(p, t, &kid, &shape, s);
-        }
-        if (frc > 0) return cuda_fail((cudaError_t)frc, "specialised kernel launch");
-        cudaError_t e = cudaSuccess;
-        if (frc < 0) {
-            kid = 0;
-            e = (cudaError_t)launch_generic(p, &shape, s);
-        }
-        if (e != cudaSuccess) return cuda_fail(e, "launch_generic");
-        g_stats.kernel_launches++;
-        g_stats.kernel_id = kid;
-        if (g0 == 0) set_launch(shape);
-        g_launch.main_launches++;
-        if (h.alias_rows > 0 && out_row0 < h.alias_rows && alias_done) {
-            g_stats.alias_rows = std::min(h.alias_rows, out_row0 + out_rows) - out_row0;
-        } else if (h.alias_rows > 0 && out_row0 < h.alias_rows) {
-            e = (cudaError_t)launch_alias_rows(p, s);
-            if (e != cudaSuccess) return cuda_fail(e, "launch_alias_rows");
-            g_stats.kernel_launches++;
-            g_stats.alias_rows = std::min(h.alias_rows, out_row0 + out_rows) - out_row0;
-        }
-    }
+    int alias_done = 0;
+    int rc = launch_frame_groups(
+        c.n_frames,
+        [&](int g0, int frames, int *kid, LaunchShape *shape) {
+            p.in = c.in + (long long)g0 * c.in_frame_stride;
+            p.out = c.out + (long long)g0 * c.out_frame_stride;
+            p.n_frames = frames;
+            alias_done = 0;
+            int frc = -1;
+            if (!(flags & LANCZOS_FLAG_GENERIC_KERNEL)) {
+                frc = launch_v6(p, dp.fast, kid, &alias_done, shape, s);
+                if (frc < 0) frc = launch_dyn(p, dp.fast, kid, shape, s);
+            }
+            if (frc > 0) return cuda_fail((cudaError_t)frc, "specialised kernel launch");
+            if (frc == 0) return (int)LANCZOS_OK;
+            *kid = 0;
+            const cudaError_t e = (cudaError_t)launch_generic(p, shape, s);
+            return e == cudaSuccess ? (int)LANCZOS_OK : cuda_fail(e, "launch_generic");
+        },
+        [&]() {
+            if (b.out_row0 >= h.alias_rows) return (int)LANCZOS_OK;   // out_row0 >= 0
+            if (!alias_done) {
+                const cudaError_t e = (cudaError_t)launch_alias_rows(p, s);
+                if (e != cudaSuccess) return cuda_fail(e, "launch_alias_rows");
+                g_stats.kernel_launches++;
+            }
+            g_stats.alias_rows = std::min(h.alias_rows, b.out_row0 + b.out_rows) - b.out_row0;
+            return (int)LANCZOS_OK;
+        });
+    if (rc != LANCZOS_OK) return rc;
     if (count) {
-        unsigned long long c = 0;
-        CU(cudaMemcpyAsync(&c, dp.strict_counter, 8, cudaMemcpyDeviceToHost, s));
+        unsigned long long n = 0;
+        CU(cudaMemcpyAsync(&n, dp.strict_counter, 8, cudaMemcpyDeviceToHost, s));
         CU(cudaStreamSynchronize(s));
-        g_stats.strict_samples = (int64_t)c;
+        g_stats.strict_samples = (int64_t)n;
     }
     return LANCZOS_OK;
 }
 
-int check_band(const Plan &h, int out_row0, int out_rows, int in_row0, int in_rows) {
-    if (out_row0 < 0 || out_rows < 0 || out_row0 + out_rows > h.d.out_h) return LANCZOS_ERR_BAND;
-    if (out_rows == 0) return LANCZOS_OK;
+int check_band(const Plan &h, const Band &b) {
+    if (b.out_row0 < 0 || b.out_rows < 0 || b.out_row0 + b.out_rows > h.d.out_h) return LANCZOS_ERR_BAND;
+    if (b.out_rows == 0) return LANCZOS_OK;
     // the supplied rows must be rows of the image: a kernel indexes them as (row - in_row0) * pitch
-    if (in_row0 < 0 || in_rows < 0 || in_row0 + in_rows > h.d.in_h) return LANCZOS_ERR_BAND;
+    if (b.in_row0 < 0 || b.in_rows < 0 || b.in_row0 + b.in_rows > h.d.in_h) return LANCZOS_ERR_BAND;
     int need0, needn;
-    band_rows(h, out_row0, out_rows, &need0, &needn);
-    if (in_row0 > need0 || in_row0 + in_rows < need0 + needn) return LANCZOS_ERR_BAND;
+    band_rows(h, b.out_row0, b.out_rows, &need0, &needn);
+    if (b.in_row0 > need0 || b.in_row0 + b.in_rows < need0 + needn) return LANCZOS_ERR_BAND;
     return LANCZOS_OK;
+}
+
+// ---- host drivers: the kernels run on scratch copies of the caller's rows ---------------------
+struct Staging {
+    lanczos_desc user, wide;            // the caller's descriptor, resolved, and the one the kernels run (see widened)
+    bool is_wide;
+    long long d_in_pitch, d_out_pitch;  // row pitches of the scratch images
+};
+Staging staging(const lanczos_desc &user) {
+    const lanczos_desc wide = widened(user);
+    return {user, wide, wide.in_w != user.in_w || wide.out_w != user.out_w,
+            scratch_pitch((long long)wide.in_w * wide.channels), scratch_pitch((long long)wide.out_w * wide.channels)};
+}
+
+// `band` of n_frames host frames through the scratch buffers d_in, d_out on stream s: copy the input rows in, run the
+// kernels, copy the output rows out.  src and dst point at the band's first rows; several frames are whole frames, back
+// to back in the caller's buffers as in the scratch buffers.
+int run_staged(const DevicePlan &dp, unsigned flags, const Staging &g, const uint8_t *src, uint8_t *dst, const Band &b,
+               int n_frames, void *d_in, void *d_out, cudaStream_t s) {
+    const lanczos_desc &u = g.user;
+    CU(copy_rows(d_in, g.d_in_pitch, src, u.in_pitch, (long long)u.in_w * u.channels, (long long)b.in_rows * n_frames,
+                 cudaMemcpyHostToDevice, s));
+    const int rc = run_device(dp, flags, {(const uint8_t *)d_in, (uint8_t *)d_out, g.d_in_pitch, g.d_out_pitch, b,
+                                          n_frames, g.d_in_pitch * b.in_rows, g.d_out_pitch * b.out_rows}, s);
+    if (rc != LANCZOS_OK) return rc;
+    CU(copy_rows(dst, u.out_pitch, d_out, g.d_out_pitch, (long long)u.out_w * u.channels,
+                 (long long)b.out_rows * n_frames, cudaMemcpyDeviceToHost, s));
+    return LANCZOS_OK;
+}
+
+// The plan of one period of the ratio (D input, N output pixels per side): the polyphase tables without the large
+// per-coordinate ones.
+int period_plan(const lanczos_desc *desc, Plan *p) {
+    lanczos_desc d;
+    int rc = resolve_desc(desc, &d);
+    if (rc != LANCZOS_OK) return rc;
+    d.in_w = d.in_h = d.scale_d;
+    d.out_w = d.out_h = d.scale_n;
+    d.in_pitch = d.out_pitch = 0;
+    return build_plan(&d, p);
 }
 
 }  // namespace
@@ -448,35 +510,20 @@ double lanczos_b200_kernel(double x, int32_t a) { return ref_kernel(x, a); }
 int lanczos_b200_phase_table(const lanczos_desc *desc, float *weights, int32_t capacity_floats) {
     if (!desc) return LANCZOS_ERR_NULL;
     Plan p;
-    // only the table is wanted: shrink the image so the per-coordinate tables stay tiny
-    lanczos_desc d = *desc;
-    int rc = resolve_desc(desc, &d);
+    int rc = period_plan(desc, &p);
     if (rc != LANCZOS_OK) return rc;
-    lanczos_desc small = d;
-    small.in_w = small.in_h = d.scale_d;
-    small.out_w = small.out_h = d.scale_n;
-    small.in_pitch = small.out_pitch = 0;
-    rc = build_plan(&small, &p);
-    if (rc != LANCZOS_OK) return rc;
-    const int need = d.scale_n * 2 * d.a;
+    const int need = p.d.scale_n * 2 * p.d.a;
     if (weights) {
         if (capacity_floats < need) return LANCZOS_ERR_DIMS;
         memcpy(weights, p.phase_w.data(), sizeof(float) * need);
     }
-    return d.scale_n;
+    return p.d.scale_n;
 }
 
 int lanczos_b200_phase0_chain(const lanczos_desc *desc, float *consts) {
     if (!desc || !consts) return LANCZOS_ERR_NULL;
-    lanczos_desc d = *desc;
-    int rc = resolve_desc(desc, &d);
-    if (rc != LANCZOS_OK) return rc;
-    lanczos_desc small = d;
-    small.in_w = small.in_h = d.scale_d;
-    small.out_w = small.out_h = d.scale_n;
-    small.in_pitch = small.out_pitch = 0;
     Plan p;
-    rc = build_plan(&small, &p);
+    int rc = period_plan(desc, &p);
     if (rc != LANCZOS_OK) return rc;
     memcpy(consts, p.p0_chain, sizeof(p.p0_chain));
     return p.p0_chain_ok ? 1 : 0;
@@ -531,20 +578,17 @@ void lanczos_b200_device_free(int device, void *p) {
     cudaFree(p);
 }
 int lanczos_b200_memcpy_h2d(int device, void *d_dst, const void *h_src, size_t bytes) {
-    DeviceGuard g(device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
+    SET_DEVICE(device);
     CU(cudaMemcpy(d_dst, h_src, bytes, cudaMemcpyHostToDevice));
     return LANCZOS_OK;
 }
 int lanczos_b200_memcpy_d2h(int device, void *h_dst, const void *d_src, size_t bytes) {
-    DeviceGuard g(device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
+    SET_DEVICE(device);
     CU(cudaMemcpy(h_dst, d_src, bytes, cudaMemcpyDeviceToHost));
     return LANCZOS_OK;
 }
 int lanczos_b200_synchronize(int device) {
-    DeviceGuard g(device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
+    SET_DEVICE(device);
     CU(cudaDeviceSynchronize());
     return LANCZOS_OK;
 }
@@ -556,18 +600,15 @@ int lanczos_b200_upscale_batch(const lanczos_desc *desc, const uint8_t *d_in, ui
                                int device, void *cuda_stream) {
     if (!desc || !d_in || !d_out) return LANCZOS_ERR_NULL;
     if (n_frames < 0) return LANCZOS_ERR_DIMS;
-    DeviceGuard g(device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
+    SET_DEVICE(device);
+    lanczos_desc r;
     std::shared_ptr<DevicePlan> dp;
-    int rc = get_plan(desc, device, &dp);
+    int rc = get_plan(desc, device, &r, &dp);
     if (rc != LANCZOS_OK) return rc;
-    const lanczos_desc &r = dp->host().d;
-    lanczos_desc user;
-    resolve_desc(desc, &user);  // user pitches (plans are shared across pitches)
-    if (in_frame_stride == 0) in_frame_stride = user.in_pitch * r.in_h;
-    if (out_frame_stride == 0) out_frame_stride = user.out_pitch * r.out_h;
-    return run_device(*dp, desc->flags, d_in, d_out, n_frames, in_frame_stride, out_frame_stride, 0,
-                      r.out_h, 0, r.in_h, user.in_pitch, user.out_pitch, (cudaStream_t)cuda_stream);
+    if (in_frame_stride == 0) in_frame_stride = r.in_pitch * r.in_h;
+    if (out_frame_stride == 0) out_frame_stride = r.out_pitch * r.out_h;
+    return run_device(*dp, desc->flags, {d_in, d_out, r.in_pitch, r.out_pitch, whole_frame(dp->host()), n_frames,
+                                         in_frame_stride, out_frame_stride}, (cudaStream_t)cuda_stream);
 }
 
 int lanczos_b200_upscale(const lanczos_desc *desc, const uint8_t *d_in, uint8_t *d_out, int device,
@@ -593,17 +634,15 @@ int lanczos_b200_upscale_band(const lanczos_desc *desc, const uint8_t *d_in_band
                               int32_t out_row0, int32_t out_rows, int32_t in_row0, int32_t in_rows,
                               int device, void *cuda_stream) {
     if (!desc || !d_in_band || !d_out_band) return LANCZOS_ERR_NULL;
-    DeviceGuard g(device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
+    SET_DEVICE(device);
+    lanczos_desc r;
     std::shared_ptr<DevicePlan> dp;
-    int rc = get_plan(desc, device, &dp);
+    int rc = get_plan(desc, device, &r, &dp);
     if (rc != LANCZOS_OK) return rc;
-    rc = check_band(dp->host(), out_row0, out_rows, in_row0, in_rows);
+    const Band band{out_row0, out_rows, in_row0, in_rows};
+    rc = check_band(dp->host(), band);
     if (rc != LANCZOS_OK) return rc;
-    lanczos_desc user;
-    resolve_desc(desc, &user);
-    return run_device(*dp, desc->flags, d_in_band, d_out_band, 1, 0, 0, out_row0, out_rows, in_row0,
-                      in_rows, user.in_pitch, user.out_pitch, (cudaStream_t)cuda_stream);
+    return run_device(*dp, desc->flags, {d_in_band, d_out_band, r.in_pitch, r.out_pitch, band}, (cudaStream_t)cuda_stream);
 }
 
 // ---- fixed-point HLS mode --------------------------------------------------------------------
@@ -634,27 +673,21 @@ int lanczos_b200_upscale_hls(const lanczos_desc *desc, const uint8_t *d_in, uint
     int32_t lut[128];
     rc = lanczos_b200_hls_lut(r.a, r.scale_n, bit_precision, lut, 128);
     if (rc != LANCZOS_OK) return rc;
-    DeviceGuard g(device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
+    SET_DEVICE(device);
     if (in_frame_stride == 0) in_frame_stride = r.in_pitch * r.in_h;
     if (out_frame_stride == 0) out_frame_stride = r.out_pitch * r.out_h;
     g_stats = lanczos_stats{};
     g_launch = lanczos_launch{};
-    for (int g0 = 0; g0 < n_frames; g0 += kMaxGridFrames) {   // frame groups, as in run_device
-        int kid = 100;
-        LaunchShape shape;
-        cudaError_t e = (cudaError_t)launch_hls(d_in + (long long)g0 * in_frame_stride, d_out + (long long)g0 * out_frame_stride,
-                                                r.in_pitch, r.out_pitch, in_frame_stride, out_frame_stride,
-                                                std::min(kMaxGridFrames, n_frames - g0), r.in_w, r.in_h, r.out_w, r.out_h,
-                                                r.channels, r.a, r.scale_n, bit_precision, lut, &kid, &shape,
-                                                (cudaStream_t)cuda_stream);
-        if (e != cudaSuccess) return cuda_fail(e, "launch_hls");
-        g_stats.kernel_launches++;
-        g_stats.kernel_id = kid;
-        if (g0 == 0) set_launch(shape);
-        g_launch.main_launches++;
-    }
-    return LANCZOS_OK;
+    return launch_frame_groups(
+        n_frames,
+        [&](int g0, int frames, int *kid, LaunchShape *shape) {
+            const cudaError_t e = (cudaError_t)launch_hls(
+                d_in + (long long)g0 * in_frame_stride, d_out + (long long)g0 * out_frame_stride, r.in_pitch,
+                r.out_pitch, in_frame_stride, out_frame_stride, frames, r.in_w, r.in_h, r.out_w, r.out_h, r.channels,
+                r.a, r.scale_n, bit_precision, lut, kid, shape, (cudaStream_t)cuda_stream);
+            return e == cudaSuccess ? (int)LANCZOS_OK : cuda_fail(e, "launch_hls");
+        },
+        [] { return (int)LANCZOS_OK; });
 }
 
 // ---- host-buffer drivers --------------------------------------------------------------------
@@ -664,19 +697,15 @@ int lanczos_b200_upscale_host(const lanczos_desc *desc, const uint8_t *h_in, uin
                               int device, int32_t n_streams) {
     if (!desc || !h_in || !h_out) return LANCZOS_ERR_NULL;
     if (n_frames < 0) return LANCZOS_ERR_DIMS;
-    DeviceGuard g(device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
-    lanczos_desc user;
+    SET_DEVICE(device);
+    lanczos_desc user, r;
     int rc = resolve_desc(desc, &user);
     if (rc != LANCZOS_OK) return rc;
-    const lanczos_desc wide = widened(user);
-    const bool is_wide = wide.in_w != user.in_w || wide.out_w != user.out_w;
+    const Staging sg = staging(user);
     std::shared_ptr<DevicePlan> dp;
-    rc = get_plan(&wide, device, &dp);
+    rc = get_plan(&sg.wide, device, &r, &dp);
     if (rc != LANCZOS_OK) return rc;
     const Plan &h = dp->host();
-    const long long in_row = (long long)user.in_w * user.channels, out_row = (long long)user.out_w * user.channels;
-    const long long d_in_pitch = scratch_pitch((long long)wide.in_w * wide.channels), d_out_pitch = scratch_pitch((long long)wide.out_w * wide.channels);
     if (in_frame_stride == 0) in_frame_stride = user.in_pitch * h.d.in_h;
     if (out_frame_stride == 0) out_frame_stride = user.out_pitch * h.d.out_h;
     if (n_streams < 1) n_streams = 3;
@@ -684,25 +713,25 @@ int lanczos_b200_upscale_host(const lanczos_desc *desc, const uint8_t *h_in, uin
 
     // Work items: whole frames when there are several, otherwise row bands of the single frame,
     // so that host->device, kernel and device->host of different items overlap.
-    struct Item { int frame, out_row0, out_rows, in_row0, in_rows; };
+    struct Item { int frame; Band band; };
     std::vector<Item> items;
     if (n_frames >= 2 * n_streams) {
-        for (int f = 0; f < n_frames; f++) items.push_back({f, 0, h.d.out_h, 0, h.d.in_h});
+        for (int f = 0; f < n_frames; f++) items.push_back({f, whole_frame(h)});
     } else {
         const int bands = std::max(1, std::min(h.d.out_h / 64, 2 * n_streams));
         for (int f = 0; f < n_frames; f++)
             for (int b = 0; b < bands; b++) {
                 const int r0 = (int)((long long)h.d.out_h * b / bands), r1 = (int)((long long)h.d.out_h * (b + 1) / bands);
                 if (r1 <= r0) continue;
-                Item it{f, r0, r1 - r0, 0, 0};
-                band_rows(h, r0, r1 - r0, &it.in_row0, &it.in_rows);
+                Item it{f, {r0, r1 - r0, 0, 0}};
+                band_rows(h, r0, r1 - r0, &it.band.in_row0, &it.band.in_rows);
                 items.push_back(it);
             }
     }
     size_t max_in = 0, max_out = 0;
     for (auto &it : items) {
-        max_in = std::max(max_in, (size_t)(it.in_rows * d_in_pitch));
-        max_out = std::max(max_out, (size_t)(it.out_rows * d_out_pitch));
+        max_in = std::max(max_in, (size_t)(it.band.in_rows * sg.d_in_pitch));
+        max_out = std::max(max_out, (size_t)(it.band.out_rows * sg.d_out_pitch));
     }
     n_streams = std::max(1, std::min<int>(n_streams, (int)items.size()));
     // declaration order matters: the leases are destroyed (= synchronised) before the scratch buffers are released
@@ -713,21 +742,17 @@ int lanczos_b200_upscale_host(const lanczos_desc *desc, const uint8_t *h_in, uin
         bin[i].reset(new Scratch(device, max_in));
         bout[i].reset(new Scratch(device, max_out));
         if (!bin[i]->p || !bout[i]->p) return LANCZOS_ERR_NOMEM;
-        if (is_wide) CU(cudaMemsetAsync(bin[i]->p, 0, max_in, streams[i].s));   // the extra columns stay zero: only pixels are copied in
+        if (sg.is_wide) CU(cudaMemsetAsync(bin[i]->p, 0, max_in, streams[i].s));   // the extra columns stay zero: only pixels are copied in
     }
     int64_t launches = 0;
     for (size_t k = 0; k < items.size(); k++) {
-        const Item &it = items[k];
-        const int si = (int)(k % n_streams);
-        cudaStream_t s = streams[si].s;
-        const uint8_t *src = h_in + it.frame * in_frame_stride + (long long)it.in_row0 * user.in_pitch;
-        uint8_t *dst = h_out + it.frame * out_frame_stride + (long long)it.out_row0 * user.out_pitch;
-        CU(copy_rows(bin[si]->p, d_in_pitch, src, user.in_pitch, in_row, it.in_rows, cudaMemcpyHostToDevice, s));
-        rc = run_device(*dp, desc->flags, (const uint8_t *)bin[si]->p, (uint8_t *)bout[si]->p, 1, 0, 0,
-                        it.out_row0, it.out_rows, it.in_row0, it.in_rows, d_in_pitch, d_out_pitch, s);
+        const Band &b = items[k].band;
+        const int f = items[k].frame, si = (int)(k % n_streams);
+        rc = run_staged(*dp, desc->flags, sg, h_in + f * in_frame_stride + (long long)b.in_row0 * user.in_pitch,
+                        h_out + f * out_frame_stride + (long long)b.out_row0 * user.out_pitch, b, 1, bin[si]->p,
+                        bout[si]->p, streams[si].s);
         launches += g_stats.kernel_launches;
         if (rc != LANCZOS_OK) return rc;
-        CU(copy_rows(dst, user.out_pitch, bout[si]->p, d_out_pitch, out_row, it.out_rows, cudaMemcpyDeviceToHost, s));
     }
     for (int i = 0; i < n_streams; i++) CU(streams[i].sync());
     g_stats.kernel_launches = launches;
@@ -741,10 +766,7 @@ int lanczos_b200_upscale_host_bands(const lanczos_desc *desc, const uint8_t *h_i
     lanczos_desc user;
     int rc = resolve_desc(desc, &user);
     if (rc != LANCZOS_OK) return rc;
-    const lanczos_desc wide = widened(user);
-    const bool is_wide = wide.in_w != user.in_w || wide.out_w != user.out_w;
-    const long long in_row = (long long)user.in_w * user.channels, out_row = (long long)user.out_w * user.channels;
-    const long long d_in_pitch = scratch_pitch((long long)wide.in_w * wide.channels), d_out_pitch = scratch_pitch((long long)wide.out_w * wide.channels);
+    const Staging sg = staging(user);
     std::vector<int> rcs(n_devices, LANCZOS_OK);
     std::vector<std::string> errs(n_devices);
     std::vector<int64_t> launches(n_devices, 0);
@@ -756,26 +778,22 @@ int lanczos_b200_upscale_host_bands(const lanczos_desc *desc, const uint8_t *h_i
             const int r1 = (int)((long long)user.out_h * (gidx + 1) / n_devices);
             if (r1 <= r0) return;
             auto body = [&]() -> int {
-                DeviceGuard g(dev);
-                if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
+                SET_DEVICE(dev);
+                lanczos_desc r;
                 std::shared_ptr<DevicePlan> dp;
-                int rc2 = get_plan(&wide, dev, &dp);
+                int rc2 = get_plan(&sg.wide, dev, &r, &dp);
                 if (rc2 != LANCZOS_OK) return rc2;
-                int in0, inn;
-                band_rows(dp->host(), r0, r1 - r0, &in0, &inn);
-                Scratch bin(dev, (size_t)(inn * d_in_pitch)), bout(dev, (size_t)((r1 - r0) * d_out_pitch));
+                Band b{r0, r1 - r0, 0, 0};
+                band_rows(dp->host(), r0, r1 - r0, &b.in_row0, &b.in_rows);
+                Scratch bin(dev, (size_t)(b.in_rows * sg.d_in_pitch)), bout(dev, (size_t)(b.out_rows * sg.d_out_pitch));
                 if (!bin.p || !bout.p) return LANCZOS_ERR_NOMEM;
                 StreamLease st;   // after the scratch buffers: synchronised before they are released
                 CU(st.acquire(dev));
-                if (is_wide) CU(cudaMemsetAsync(bin.p, 0, (size_t)(inn * d_in_pitch), st.s));
-                CU(copy_rows(bin.p, d_in_pitch, h_in + (long long)in0 * user.in_pitch, user.in_pitch, in_row, inn,
-                             cudaMemcpyHostToDevice, st.s));
-                rc2 = run_device(*dp, desc->flags, (const uint8_t *)bin.p, (uint8_t *)bout.p, 1, 0, 0, r0,
-                                 r1 - r0, in0, inn, d_in_pitch, d_out_pitch, st.s);
+                if (sg.is_wide) CU(cudaMemsetAsync(bin.p, 0, (size_t)(b.in_rows * sg.d_in_pitch), st.s));
+                rc2 = run_staged(*dp, desc->flags, sg, h_in + (long long)b.in_row0 * user.in_pitch,
+                                 h_out + (long long)r0 * user.out_pitch, b, 1, bin.p, bout.p, st.s);
                 launches[gidx] = g_stats.kernel_launches;
                 if (rc2 != LANCZOS_OK) return rc2;
-                CU(copy_rows(h_out + (long long)r0 * user.out_pitch, user.out_pitch, bout.p, d_out_pitch, out_row, r1 - r0,
-                             cudaMemcpyDeviceToHost, st.s));
                 CU(st.sync());
                 return LANCZOS_OK;
             };
@@ -803,28 +821,26 @@ int lanczos_b200_expected(const lanczos_desc *desc, const uint8_t *h_in_planar, 
     lanczos_desc r;
     int rc = resolve_desc(&d, &r);
     if (rc != LANCZOS_OK) return rc;
-    DeviceGuard g(device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
-    // planes stay planes: each one is upscaled as a one-channel frame (no interleaving round trip); on the device
-    // the rows of a plane are padded to 16 bytes so that odd widths keep the TMA kernels
-    const long long planes = r.channels;
-    lanczos_desc plane = r;
-    plane.channels = 1;
-    const lanczos_desc wide = widened(plane);               // one-channel planes: widths rounded up to 4 pixels
-    const long long d_in_pitch = scratch_pitch(wide.in_w), d_out_pitch = scratch_pitch(wide.out_w);
-    d = wide;
-    d.channels = r.channels;
-    d.in_pitch = d_in_pitch;
-    d.out_pitch = d_out_pitch;
-    Scratch pin(device, (size_t)(d_in_pitch * r.in_h * planes)), pout(device, (size_t)(d_out_pitch * r.out_h * planes));
+    SET_DEVICE(device);
+    // planes stay planes: each one is upscaled as a one-channel frame of one call (no interleaving round trip); on the
+    // device the rows of a plane are padded to 16 bytes so that odd widths keep the TMA kernels
+    const int planes = r.channels;
+    r.channels = 1;
+    r.in_pitch = r.in_w;
+    r.out_pitch = r.out_w;
+    const Staging sg = staging(r);    // one-channel planes: widths rounded up to 4 pixels
+    const size_t in_bytes = (size_t)(sg.d_in_pitch * r.in_h * planes);
+    Scratch pin(device, in_bytes), pout(device, (size_t)(sg.d_out_pitch * r.out_h * planes));
     if (!pin.p || !pout.p) return LANCZOS_ERR_NOMEM;
     StreamLease st;
     CU(st.acquire(device));
-    if (wide.in_w != r.in_w) CU(cudaMemsetAsync(pin.p, 0, (size_t)(d_in_pitch * r.in_h * planes), st.s));
-    CU(copy_rows(pin.p, d_in_pitch, h_in_planar, r.in_w, r.in_w, (long long)r.in_h * planes, cudaMemcpyHostToDevice, st.s));
-    rc = lanczos_b200_upscale_planar(&d, (const uint8_t *)pin.p, (uint8_t *)pout.p, 1, 0, 0, device, st.s);
+    if (sg.wide.in_w != r.in_w) CU(cudaMemsetAsync(pin.p, 0, in_bytes, st.s));
+    std::shared_ptr<DevicePlan> dp;
+    rc = get_plan(&sg.wide, device, &d, &dp);
     if (rc != LANCZOS_OK) return rc;
-    CU(copy_rows(h_out_planar, r.out_w, pout.p, d_out_pitch, r.out_w, (long long)r.out_h * planes, cudaMemcpyDeviceToHost, st.s));
+    rc = run_staged(*dp, desc->flags, sg, h_in_planar, h_out_planar, whole_frame(dp->host()), planes, pin.p, pout.p,
+                    st.s);
+    if (rc != LANCZOS_OK) return rc;
     CU(st.sync());
     return LANCZOS_OK;
 }
@@ -834,13 +850,11 @@ int lanczos_b200_stream(const lanczos_desc *desc, const uint32_t *h_in_words, ui
     if (desc->channels != 3) return LANCZOS_ERR_ALIGN;
     lanczos_desc d = *desc;
     d.in_pitch = d.out_pitch = 0;   // a stream has no row padding (lanczos.cpp:56-62)
-    DeviceGuard g(device);
-    if (!g.ok) return cuda_fail(cudaErrorInvalidDevice, "cudaSetDevice");
-    std::shared_ptr<DevicePlan> dp;
-    int rc = get_plan(&d, device, &dp);
-    if (rc != LANCZOS_OK) return rc;
+    SET_DEVICE(device);
     lanczos_desc r;
-    resolve_desc(&d, &r);           // dense pitches of THIS call: cached plans carry none
+    std::shared_ptr<DevicePlan> dp;
+    int rc = get_plan(&d, device, &r, &dp);
+    if (rc != LANCZOS_OK) return rc;
     const long long n_in = (long long)r.in_w * r.in_h, n_out = (long long)r.out_w * r.out_h;
     Scratch win(device, n_in * 4), iin(device, n_in * 3), iout(device, n_out * 3), wout(device, n_out * 4);
     if (!win.p || !iin.p || !iout.p || !wout.p) return LANCZOS_ERR_NOMEM;
@@ -848,8 +862,8 @@ int lanczos_b200_stream(const lanczos_desc *desc, const uint32_t *h_in_words, ui
     CU(st.acquire(device));
     CU(cudaMemcpyAsync(win.p, h_in_words, n_in * 4, cudaMemcpyHostToDevice, st.s));
     CU((cudaError_t)launch_words_to_rgb((const uint32_t *)win.p, (uint8_t *)iin.p, n_in, st.s));
-    rc = run_device(*dp, d.flags, (const uint8_t *)iin.p, (uint8_t *)iout.p, 1, 0, 0, 0, r.out_h, 0, r.in_h,
-                    r.in_pitch, r.out_pitch, st.s);
+    rc = run_device(*dp, d.flags, {(const uint8_t *)iin.p, (uint8_t *)iout.p, r.in_pitch, r.out_pitch,
+                                   whole_frame(dp->host())}, st.s);
     if (rc != LANCZOS_OK) return rc;
     const int64_t launches = g_stats.kernel_launches + 2;
     CU((cudaError_t)launch_rgb_to_words((const uint8_t *)iout.p, (uint32_t *)wout.p, n_out, st.s));
