@@ -49,7 +49,7 @@ enum {
                                      reduction, or a downscale (worker.cpp:140 assumes 1/SCALE < 1) */
     LANCZOS_ERR_RATIO_FLOAT = -6, /* floor((double)xx/SCALE) != floor(xx*D/N) for some output
                                      coordinate: the reference itself picks a shifted window there */
-    LANCZOS_ERR_BAND        = -7, /* row band outside the image or its input rows not supplied */
+    LANCZOS_ERR_BAND        = -7, /* row band or window outside the image or its input pixels not supplied */
     LANCZOS_ERR_CUDA        = -8, /* CUDA runtime/driver error (see lanczos_b200_last_cuda_error) */
     LANCZOS_ERR_NOMEM       = -9,
     LANCZOS_ERR_ALIGN       = -10 /* packed-word stream shim only supports 3 channels */
@@ -160,6 +160,41 @@ int lanczos_b200_upscale_band(const lanczos_desc *desc, const uint8_t *d_in_band
  * band that contains the in-place top rows. */
 int lanczos_b200_band_input_rows(const lanczos_desc *desc, int32_t out_row0, int32_t out_rows,
                                  int32_t *in_row0, int32_t *in_rows);
+
+/* ---- any rectangle (window) of the output image: a viewport, a tile, part of each video frame.
+ * Every pixel of a window equals the pixel at the same coordinates of the whole-image result, bit for bit (phases
+ * and weights follow the global column and row), and only the input pixels the window reads are needed: the
+ * rectangle of lanczos_b200_region_input_rect.  A row band is the full-width window.
+ *
+ * lanczos_b200_region_input_rect: the input rect [*in_x0, *in_x0+*in_w) x [*in_y0, *in_y0+*in_h) that the output
+ * window [out_x0, out_x0+out_w) x [out_y0, out_y0+out_h) reads.  Rows are lanczos_b200_band_input_rows of the
+ * window's rows (widened for a window that contains the in-place top rows); columns are the same rule on the x-axis,
+ * clipped to the image, with *in_x0 then moved left until in_x0*channels is a multiple of 16 (a view into a
+ * 16-byte-aligned image with a 16-byte pitch keeps the alignment the fast kernels need).
+ * LANCZOS_ERR_BAND when the window is empty or not inside the output image. */
+int lanczos_b200_region_input_rect(const lanczos_desc *desc, int32_t out_x0, int32_t out_y0, int32_t out_w,
+                                   int32_t out_h, int32_t *in_x0, int32_t *in_y0, int32_t *in_w, int32_t *in_h);
+
+/* lanczos_b200_upscale_region: device buffers, asynchronous on `cuda_stream`.  `d_in_rect` points at input pixel
+ * (in_x0, in_y0) and holds in_w x in_h pixels; `d_out_window` points at the window's first pixel.  desc->in_pitch and
+ * desc->out_pitch are the row pitches of these two buffers (0 = dense rows of the rect and of the window), so a view
+ * into a full image passes the full image's pitch.  Frames as in lanczos_b200_upscale_batch (stride 0 = pitch x rows
+ * of the rect / window; groups of at most 65,535 frames); planar images pass channels = 1 and plane strides.
+ * LANCZOS_ERR_BAND when the window or the rect lies outside the image, or the rect does not contain the columns and
+ * rows the window reads (region_input_rect's rect before the 16-byte rounding of in_x0).  An empty window is a no-op.
+ * The fast kernels need what they need for whole images, applied to the rect and the window; the static-phase kernels
+ * also need (out_x0*channels) on their H-item grid (16 bytes for RGB in exact mode) and fall back otherwise. */
+int lanczos_b200_upscale_region(const lanczos_desc *desc, const uint8_t *d_in_rect, uint8_t *d_out_window,
+                                int32_t out_x0, int32_t out_y0, int32_t out_w, int32_t out_h, int32_t in_x0,
+                                int32_t in_y0, int32_t in_w, int32_t in_h, int32_t n_frames, int64_t in_frame_stride,
+                                int64_t out_frame_stride, int device, void *cuda_stream);
+
+/* lanczos_b200_upscale_host_region: a window of a HOST image.  `h_in` is the whole image (desc->in_pitch its pitch,
+ * 0 = dense); only the input rect is copied to the device and only the window back, to `h_out_window` with row pitch
+ * out_window_pitch (0 = dense).  Synchronous: returns when `h_out_window` is complete. */
+int lanczos_b200_upscale_host_region(const lanczos_desc *desc, const uint8_t *h_in, uint8_t *h_out_window,
+                                     int32_t out_x0, int32_t out_y0, int32_t out_w, int32_t out_h,
+                                     int64_t out_window_pitch, int device);
 
 /* ---- end to end with HOST buffers: what sim_tb does around the two calls
  * (full_TB.h:127-165) minus the PNG codec.  Frames are split into chunks that are copied

@@ -28,6 +28,7 @@ from .api import (  # noqa: F401
     phase_table,
     phase0_chain,
     reduce_ratio,
+    region_input_rect,
     resolve,
     stats,
     launch,
@@ -37,6 +38,8 @@ from .api import (  # noqa: F401
     upscale_device,
     upscale_batch_device,
     upscale_band_device,
+    upscale_region,
+    upscale_region_device,
     upscale_planar_device,
     PinnedBuffer,
     hls_lut,

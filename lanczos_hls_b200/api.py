@@ -72,6 +72,9 @@ def lib():
     L.lanczos_b200_upscale_planar.argtypes = [dp, u8p, u8p, i32, i64, i64, C.c_int, vp]
     L.lanczos_b200_upscale_band.argtypes = [dp, u8p, u8p, i32, i32, i32, i32, C.c_int, vp]
     L.lanczos_b200_band_input_rows.argtypes = [dp, i32, i32, C.POINTER(i32), C.POINTER(i32)]
+    L.lanczos_b200_region_input_rect.argtypes = [dp, i32, i32, i32, i32] + [C.POINTER(i32)] * 4
+    L.lanczos_b200_upscale_region.argtypes = [dp, u8p, u8p] + [i32] * 9 + [i64, i64, C.c_int, vp]
+    L.lanczos_b200_upscale_host_region.argtypes = [dp, u8p, u8p, i32, i32, i32, i32, i64, C.c_int]
     L.lanczos_b200_upscale_host.argtypes = [dp, u8p, u8p, i32, i64, i64, C.c_int, i32]
     L.lanczos_b200_upscale_host_bands.argtypes = [dp, u8p, u8p, C.POINTER(i32), i32]
     L.lanczos_b200_expected.argtypes = [dp, u8p, u8p, C.c_int]
@@ -158,6 +161,13 @@ def band_input_rows(desc, out_row0, out_rows):
     a, b = C.c_int32(), C.c_int32()
     _check(lib().lanczos_b200_band_input_rows(C.byref(desc), out_row0, out_rows, C.byref(a), C.byref(b)))
     return a.value, b.value
+
+
+def region_input_rect(desc, x0, y0, w, h):
+    """(in_x0, in_y0, in_w, in_h): the input pixels the output window [x0, x0+w) x [y0, y0+h) reads."""
+    r = [C.c_int32() for _ in range(4)]
+    _check(lib().lanczos_b200_region_input_rect(C.byref(desc), x0, y0, w, h, *[C.byref(v) for v in r]))
+    return tuple(v.value for v in r)
 
 
 def enable_stats(on=True):
@@ -333,6 +343,37 @@ def upscale_band_device(desc, d_in_band, d_out_band, out_row0, out_rows, in_row0
                                            C.c_void_p(d_out_band.data_ptr()), out_row0, out_rows, in_row0, in_rows,
                                            d_in_band.device.index or 0, _stream_ptr(d_in_band)))
     return d_out_band
+
+
+def upscale_region_device(desc, d_in_rect, d_out, x0, y0, in_x0, in_y0, flags=None):
+    """Output window of the image described by `desc` (its sizes, ratio, a and flags; its pitches are not used):
+    torch uint8 CUDA tensors [h][w][C] or [F][h][w][C].  d_in_rect holds the input pixels from (in_x0, in_y0) and
+    d_out receives the window whose first pixel is (x0, y0); sizes come from the shapes, row pitches from stride(-3)
+    and frame strides from stride(0), so a slice of a full image works without a copy.  `flags` replaces desc.flags."""
+    batched = d_in_rect.dim() == 4
+    f = d_in_rect.shape[0] if batched else 1
+    in_h, in_w = d_in_rect.shape[-3:-1]
+    h, w = d_out.shape[-3:-1]
+    d = Desc.from_buffer_copy(desc)
+    d.in_pitch, d.out_pitch = d_in_rect.stride(-3), d_out.stride(-3)
+    if flags is not None:
+        d.flags = flags
+    _check(lib().lanczos_b200_upscale_region(C.byref(d), C.c_void_p(d_in_rect.data_ptr()), C.c_void_p(d_out.data_ptr()),
+                                             x0, y0, w, h, in_x0, in_y0, in_w, in_h, f,
+                                             d_in_rect.stride(0) if batched else 0, d_out.stride(0) if batched else 0,
+                                             d_in_rect.device.index or 0, _stream_ptr(d_in_rect)))
+    return d_out
+
+
+def upscale_region(img, out_w, out_h, x0, y0, w, h, a=3, scale_n=0, scale_d=0, flags=0, device=0):
+    """Window [x0, x0+w) x [y0, y0+h) of the upscaled uint8 [H][W][C] host image: only the input pixels it reads go to
+    the device, only the window comes back."""
+    img = np.ascontiguousarray(img, dtype=np.uint8)
+    ih, iw, c = img.shape
+    desc = make_desc(iw, ih, out_w, out_h, c, a, scale_n, scale_d, flags=flags)
+    out = np.empty((h, w, c), dtype=np.uint8)
+    _check(lib().lanczos_b200_upscale_host_region(C.byref(desc), _np_ptr(img), _np_ptr(out), x0, y0, w, h, 0, device))
+    return out
 
 
 # ---- fixed-point "HLS mode" (the reference's lanczos() arithmetic, parity unpinned) ------------

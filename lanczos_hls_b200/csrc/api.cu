@@ -12,6 +12,7 @@
 #include <map>
 #include <memory>
 #include <mutex>
+#include <numeric>
 #include <string>
 #include <thread>
 #include <tuple>
@@ -306,37 +307,50 @@ int launch_frame_groups(int n_frames, Main main, Then then) {
     return LANCZOS_OK;
 }
 
-// Output rows [out_row0, out_row0 + out_rows) of a frame, computed from its input rows [in_row0, in_row0 + in_rows).
-struct Band {
+// The output window [out_col0, out_col0 + out_cols) x [out_row0, out_row0 + out_rows) of a frame, computed from its
+// input rect [in_col0, in_col0 + in_cols) x [in_row0, in_row0 + in_rows); global coordinates.  Whole frames and row
+// bands are the full-width windows.
+struct Window {
     int out_row0, out_rows, in_row0, in_rows;
+    int out_col0, out_cols, in_col0, in_cols;
 };
-Band whole_frame(const Plan &h) { return {0, h.d.out_h, 0, h.d.in_h}; }
+Window full_width(const Plan &h, int out_row0, int out_rows, int in_row0, int in_rows) {
+    return {out_row0, out_rows, in_row0, in_rows, 0, h.d.out_w, 0, h.d.in_w};
+}
+Window whole_frame(const Plan &h) { return full_width(h, 0, h.d.out_h, 0, h.d.in_h); }
+// The full-width band of output rows [out_row0, out_row0 + out_rows) with the input rows it reads
+Window row_band(const Plan &h, int out_row0, int out_rows) {
+    Window b = full_width(h, out_row0, out_rows, 0, 0);
+    band_rows(h, out_row0, out_rows, &b.in_row0, &b.in_rows);
+    return b;
+}
 
-// One call of the kernels: `band` of n_frames frames; in and out point at the band's first rows in frame 0.
+// One call of the kernels: window `win` of n_frames frames; in and out point at the window's first pixels in frame 0.
 struct DeviceCall {
     const uint8_t *in;
     uint8_t *out;
     long long in_pitch, out_pitch;
-    Band band;
+    Window win;
     int n_frames = 1;
     long long in_frame_stride = 0, out_frame_stride = 0;
 };
 
 int run_device(const DevicePlan &dp, unsigned flags, const DeviceCall &c, cudaStream_t s) {
     const Plan &h = dp.host();
-    const Band &b = c.band;
+    const Window &b = c.win;
     KParams p = dp.launch;
     p.in_pitch = c.in_pitch;
     p.out_pitch = c.out_pitch;
     p.in_frame_stride = c.in_frame_stride;
     p.out_frame_stride = c.out_frame_stride;
     p.out_row0 = b.out_row0; p.out_rows = b.out_rows; p.in_row0 = b.in_row0; p.in_rows = b.in_rows;
+    p.out_col0 = b.out_col0; p.out_cols = b.out_cols; p.in_col0 = b.in_col0; p.in_cols = b.in_cols;
     p.flags = flags;
     const bool count = g_stats_enabled.load(std::memory_order_relaxed);
     p.strict_counter = count ? dp.strict_counter : nullptr;
     g_stats = lanczos_stats{};
     g_launch = lanczos_launch{};
-    if (c.n_frames <= 0 || b.out_rows <= 0) return LANCZOS_OK;
+    if (c.n_frames <= 0 || b.out_rows <= 0 || b.out_cols <= 0) return LANCZOS_OK;
     // counting calls are synchronous and take turns on the plan's counter (several host threads or streams may share a plan)
     std::unique_lock<std::mutex> stats_lock;
     if (count) {
@@ -382,14 +396,33 @@ int run_device(const DevicePlan &dp, unsigned flags, const DeviceCall &c, cudaSt
     return LANCZOS_OK;
 }
 
-int check_band(const Plan &h, const Band &b) {
-    if (b.out_row0 < 0 || b.out_rows < 0 || b.out_row0 + b.out_rows > h.d.out_h) return LANCZOS_ERR_BAND;
-    if (b.out_rows == 0) return LANCZOS_OK;
-    // the supplied rows must be rows of the image: a kernel indexes them as (row - in_row0) * pitch
-    if (b.in_row0 < 0 || b.in_rows < 0 || b.in_row0 + b.in_rows > h.d.in_h) return LANCZOS_ERR_BAND;
+bool inside(int x0, int n, int len) { return x0 >= 0 && n >= 0 && n <= len - x0; }
+bool covers(int x0, int n, int need0, int needn) { return x0 <= need0 && (long long)x0 + n >= (long long)need0 + needn; }
+
+// The non-empty window [out_x0, out_x0 + out_w) x [out_y0, out_y0 + out_h) of the image with the input rect it reads:
+// band_rows and band_cols, then the rect's first column moved left until it starts on the image's 16-byte grid, so that
+// a view into a 16-byte-aligned image with a 16-byte pitch keeps the alignment the TMA kernels need.
+Window region(const Plan &h, int out_x0, int out_y0, int out_w, int out_h) {
+    Window b{out_y0, out_h, 0, 0, out_x0, out_w, 0, 0};
+    band_rows(h, out_y0, out_h, &b.in_row0, &b.in_rows);
+    band_cols(h, out_x0, out_w, &b.in_col0, &b.in_cols);
+    const int step = 16 / std::gcd(16, h.d.channels);   // pixels per 16 bytes, or 16 for C = 3
+    const int x0 = b.in_col0 / step * step;
+    b.in_cols += b.in_col0 - x0;
+    b.in_col0 = x0;
+    return b;
+}
+
+int check_window(const Plan &h, const Window &b) {
+    if (!inside(b.out_row0, b.out_rows, h.d.out_h) || !inside(b.out_col0, b.out_cols, h.d.out_w)) return LANCZOS_ERR_BAND;
+    if (b.out_rows == 0 || b.out_cols == 0) return LANCZOS_OK;
+    // the supplied rect must lie in the image: a kernel indexes it as (row - in_row0) * pitch + (column - in_col0) * C
+    if (!inside(b.in_row0, b.in_rows, h.d.in_h) || !inside(b.in_col0, b.in_cols, h.d.in_w)) return LANCZOS_ERR_BAND;
     int need0, needn;
     band_rows(h, b.out_row0, b.out_rows, &need0, &needn);
-    if (b.in_row0 > need0 || b.in_row0 + b.in_rows < need0 + needn) return LANCZOS_ERR_BAND;
+    if (!covers(b.in_row0, b.in_rows, need0, needn)) return LANCZOS_ERR_BAND;
+    band_cols(h, b.out_col0, b.out_cols, &need0, &needn);
+    if (!covers(b.in_col0, b.in_cols, need0, needn)) return LANCZOS_ERR_BAND;
     return LANCZOS_OK;
 }
 
@@ -405,19 +438,24 @@ Staging staging(const lanczos_desc &user) {
             scratch_pitch((long long)wide.in_w * wide.channels), scratch_pitch((long long)wide.out_w * wide.channels)};
 }
 
-// `band` of n_frames host frames through the scratch buffers d_in, d_out on stream s: copy the input rows in, run the
-// kernels, copy the output rows out.  src and dst point at the band's first rows; several frames are whole frames, back
-// to back in the caller's buffers as in the scratch buffers.
-int run_staged(const DevicePlan &dp, unsigned flags, const Staging &g, const uint8_t *src, uint8_t *dst, const Band &b,
+// The window `b` of n_frames host frames through the scratch buffers d_in, d_out on stream s: copy the input rect in,
+// run the kernels, copy the window out.  src and dst point at the rect's and the window's first pixels, with the row
+// pitches of g.user; several frames are whole frames, back to back in the caller's buffers as in the scratch buffers.
+// The scratch rows are the rect's and the window's rows padded to 16 bytes; only the caller's columns are copied (the
+// widened columns of a whole frame stay as the caller's memset left them).
+int run_staged(const DevicePlan &dp, unsigned flags, const Staging &g, const uint8_t *src, uint8_t *dst, const Window &b,
                int n_frames, void *d_in, void *d_out, cudaStream_t s) {
     const lanczos_desc &u = g.user;
-    CU(copy_rows(d_in, g.d_in_pitch, src, u.in_pitch, (long long)u.in_w * u.channels, (long long)b.in_rows * n_frames,
+    const long long ip = scratch_pitch((long long)b.in_cols * u.channels), op = scratch_pitch((long long)b.out_cols * u.channels);
+    const int in_cols = std::min(b.in_col0 + b.in_cols, u.in_w) - b.in_col0;
+    const int out_cols = std::min(b.out_col0 + b.out_cols, u.out_w) - b.out_col0;
+    CU(copy_rows(d_in, ip, src, u.in_pitch, (long long)in_cols * u.channels, (long long)b.in_rows * n_frames,
                  cudaMemcpyHostToDevice, s));
-    const int rc = run_device(dp, flags, {(const uint8_t *)d_in, (uint8_t *)d_out, g.d_in_pitch, g.d_out_pitch, b,
-                                          n_frames, g.d_in_pitch * b.in_rows, g.d_out_pitch * b.out_rows}, s);
+    const int rc = run_device(dp, flags, {(const uint8_t *)d_in, (uint8_t *)d_out, ip, op, b, n_frames, ip * b.in_rows,
+                                          op * b.out_rows}, s);
     if (rc != LANCZOS_OK) return rc;
-    CU(copy_rows(dst, u.out_pitch, d_out, g.d_out_pitch, (long long)u.out_w * u.channels,
-                 (long long)b.out_rows * n_frames, cudaMemcpyDeviceToHost, s));
+    CU(copy_rows(dst, u.out_pitch, d_out, op, (long long)out_cols * u.channels, (long long)b.out_rows * n_frames,
+                 cudaMemcpyDeviceToHost, s));
     return LANCZOS_OK;
 }
 
@@ -551,6 +589,22 @@ int lanczos_b200_band_input_rows(const lanczos_desc *desc, int32_t out_row0, int
     return LANCZOS_OK;
 }
 
+int lanczos_b200_region_input_rect(const lanczos_desc *desc, int32_t out_x0, int32_t out_y0, int32_t out_w, int32_t out_h,
+                                   int32_t *in_x0, int32_t *in_y0, int32_t *in_w, int32_t *in_h) {
+    if (!desc || !in_x0 || !in_y0 || !in_w || !in_h) return LANCZOS_ERR_NULL;
+    std::shared_ptr<const Plan> p;
+    int rc = get_host_plan(desc, &p);
+    if (rc != LANCZOS_OK) return rc;
+    if (out_w < 1 || out_h < 1 || !inside(out_x0, out_w, p->d.out_w) || !inside(out_y0, out_h, p->d.out_h))
+        return LANCZOS_ERR_BAND;
+    Window b = region(*p, out_x0, out_y0, out_w, out_h);
+    *in_x0 = b.in_col0;
+    *in_y0 = b.in_row0;
+    *in_w = b.in_cols;
+    *in_h = b.in_rows;
+    return LANCZOS_OK;
+}
+
 int lanczos_b200_device_count(void) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess) return 0;
@@ -639,10 +693,35 @@ int lanczos_b200_upscale_band(const lanczos_desc *desc, const uint8_t *d_in_band
     std::shared_ptr<DevicePlan> dp;
     int rc = get_plan(desc, device, &r, &dp);
     if (rc != LANCZOS_OK) return rc;
-    const Band band{out_row0, out_rows, in_row0, in_rows};
-    rc = check_band(dp->host(), band);
+    const Window band = full_width(dp->host(), out_row0, out_rows, in_row0, in_rows);
+    rc = check_window(dp->host(), band);
     if (rc != LANCZOS_OK) return rc;
     return run_device(*dp, desc->flags, {d_in_band, d_out_band, r.in_pitch, r.out_pitch, band}, (cudaStream_t)cuda_stream);
+}
+
+int lanczos_b200_upscale_region(const lanczos_desc *desc, const uint8_t *d_in_rect, uint8_t *d_out_window,
+                                int32_t out_x0, int32_t out_y0, int32_t out_w, int32_t out_h, int32_t in_x0,
+                                int32_t in_y0, int32_t in_w, int32_t in_h, int32_t n_frames, int64_t in_frame_stride,
+                                int64_t out_frame_stride, int device, void *cuda_stream) {
+    if (!desc || !d_in_rect || !d_out_window) return LANCZOS_ERR_NULL;
+    if (n_frames < 0) return LANCZOS_ERR_DIMS;
+    SET_DEVICE(device);
+    // the pitches are those of the rect and the window: the plan is looked up without them
+    lanczos_desc d = *desc, r;
+    d.in_pitch = d.out_pitch = 0;
+    std::shared_ptr<DevicePlan> dp;
+    int rc = get_plan(&d, device, &r, &dp);
+    if (rc != LANCZOS_OK) return rc;
+    const Window b{out_y0, out_h, in_y0, in_h, out_x0, out_w, in_x0, in_w};
+    rc = check_window(dp->host(), b);
+    if (rc != LANCZOS_OK) return rc;
+    const long long in_row = (long long)in_w * r.channels, out_row = (long long)out_w * r.channels;
+    const long long in_pitch = desc->in_pitch ? desc->in_pitch : in_row, out_pitch = desc->out_pitch ? desc->out_pitch : out_row;
+    if (in_pitch < in_row || out_pitch < out_row) return LANCZOS_ERR_DIMS;
+    if (in_frame_stride == 0) in_frame_stride = in_pitch * in_h;
+    if (out_frame_stride == 0) out_frame_stride = out_pitch * out_h;
+    return run_device(*dp, desc->flags, {d_in_rect, d_out_window, in_pitch, out_pitch, b, n_frames, in_frame_stride,
+                                         out_frame_stride}, (cudaStream_t)cuda_stream);
 }
 
 // ---- fixed-point HLS mode --------------------------------------------------------------------
@@ -713,7 +792,7 @@ int lanczos_b200_upscale_host(const lanczos_desc *desc, const uint8_t *h_in, uin
 
     // Work items: whole frames when there are several, otherwise row bands of the single frame,
     // so that host->device, kernel and device->host of different items overlap.
-    struct Item { int frame; Band band; };
+    struct Item { int frame; Window band; };
     std::vector<Item> items;
     if (n_frames >= 2 * n_streams) {
         for (int f = 0; f < n_frames; f++) items.push_back({f, whole_frame(h)});
@@ -723,9 +802,7 @@ int lanczos_b200_upscale_host(const lanczos_desc *desc, const uint8_t *h_in, uin
             for (int b = 0; b < bands; b++) {
                 const int r0 = (int)((long long)h.d.out_h * b / bands), r1 = (int)((long long)h.d.out_h * (b + 1) / bands);
                 if (r1 <= r0) continue;
-                Item it{f, {r0, r1 - r0, 0, 0}};
-                band_rows(h, r0, r1 - r0, &it.band.in_row0, &it.band.in_rows);
-                items.push_back(it);
+                items.push_back({f, row_band(h, r0, r1 - r0)});
             }
     }
     size_t max_in = 0, max_out = 0;
@@ -746,7 +823,7 @@ int lanczos_b200_upscale_host(const lanczos_desc *desc, const uint8_t *h_in, uin
     }
     int64_t launches = 0;
     for (size_t k = 0; k < items.size(); k++) {
-        const Band &b = items[k].band;
+        const Window &b = items[k].band;
         const int f = items[k].frame, si = (int)(k % n_streams);
         rc = run_staged(*dp, desc->flags, sg, h_in + f * in_frame_stride + (long long)b.in_row0 * user.in_pitch,
                         h_out + f * out_frame_stride + (long long)b.out_row0 * user.out_pitch, b, 1, bin[si]->p,
@@ -783,8 +860,7 @@ int lanczos_b200_upscale_host_bands(const lanczos_desc *desc, const uint8_t *h_i
                 std::shared_ptr<DevicePlan> dp;
                 int rc2 = get_plan(&sg.wide, dev, &r, &dp);
                 if (rc2 != LANCZOS_OK) return rc2;
-                Band b{r0, r1 - r0, 0, 0};
-                band_rows(dp->host(), r0, r1 - r0, &b.in_row0, &b.in_rows);
+                const Window b = row_band(dp->host(), r0, r1 - r0);
                 Scratch bin(dev, (size_t)(b.in_rows * sg.d_in_pitch)), bout(dev, (size_t)(b.out_rows * sg.d_out_pitch));
                 if (!bin.p || !bout.p) return LANCZOS_ERR_NOMEM;
                 StreamLease st;   // after the scratch buffers: synchronised before they are released
@@ -810,6 +886,36 @@ int lanczos_b200_upscale_host_bands(const lanczos_desc *desc, const uint8_t *h_i
             return rcs[i];
         }
     }
+    return LANCZOS_OK;
+}
+
+int lanczos_b200_upscale_host_region(const lanczos_desc *desc, const uint8_t *h_in, uint8_t *h_out_window, int32_t out_x0,
+                                     int32_t out_y0, int32_t out_w, int32_t out_h, int64_t out_window_pitch, int device) {
+    if (!desc || !h_in || !h_out_window) return LANCZOS_ERR_NULL;
+    SET_DEVICE(device);
+    lanczos_desc d = *desc, user;   // desc->out_pitch is not read: the window's pitch is out_window_pitch
+    d.out_pitch = 0;
+    std::shared_ptr<DevicePlan> dp;
+    int rc = get_plan(&d, device, &user, &dp);
+    if (rc != LANCZOS_OK) return rc;
+    const Plan &h = dp->host();
+    if (!inside(out_x0, out_w, h.d.out_w) || !inside(out_y0, out_h, h.d.out_h)) return LANCZOS_ERR_BAND;
+    if (out_w == 0 || out_h == 0) return run_device(*dp, desc->flags, {h_in, h_out_window, 0, 0, Window{}, 0}, nullptr);   // no-op
+    // the kernels run on the caller's geometry (no widening: the window is not a whole row); the host side of the copies
+    // is the caller's image and the caller's window
+    user.out_pitch = out_window_pitch ? out_window_pitch : (long long)out_w * user.channels;
+    if (user.out_pitch < (long long)out_w * user.channels) return LANCZOS_ERR_DIMS;
+    const Window b = region(h, out_x0, out_y0, out_w, out_h);
+    const Staging sg{user, user, false, scratch_pitch((long long)b.in_cols * user.channels),
+                     scratch_pitch((long long)b.out_cols * user.channels)};
+    Scratch bin(device, (size_t)(b.in_rows * sg.d_in_pitch)), bout(device, (size_t)(b.out_rows * sg.d_out_pitch));
+    if (!bin.p || !bout.p) return LANCZOS_ERR_NOMEM;
+    StreamLease st;   // after the scratch buffers: synchronised before they are released
+    CU(st.acquire(device));
+    rc = run_staged(*dp, desc->flags, sg, h_in + (long long)b.in_row0 * user.in_pitch + (long long)b.in_col0 * user.channels,
+                    h_out_window, b, 1, bin.p, bout.p, st.s);
+    if (rc != LANCZOS_OK) return rc;
+    CU(st.sync());
     return LANCZOS_OK;
 }
 

@@ -16,15 +16,19 @@ namespace {
 // ---------------------------------------------------------------------------------------------
 // kernel parameters and the static vertical phase pattern
 // ---------------------------------------------------------------------------------------------
-// What both kernel families know about a launch: the output band and how it is cut into vertical segments.  The
+// What both kernel families know about a launch: the output window and how it is cut into vertical segments.  The
 // kernels read out_row0 + out_rows and vperiod0 + seg_periods together: each pair shares one 8-byte word.
+// Columns are byte columns: the window is output bytes [out_byte0, out_byte0 + out_bytes) of a row, and the input rect
+// starts at input byte in_byte0 of a row (both global: KParams out_col0 * C and in_col0 * C).  out_byte0 and in_byte0
+// are the LAST fields of each family's parameter struct (V6Params, DynParams), set by launch_strips: placed here they
+// moved the constant-bank offsets of every other field, and bench.py measured the headline kernel 0.6 % slower.
 struct StripParams {
-    uint8_t *out;         // output row `out_row0` of frame 0
+    uint8_t *out;         // output pixel (out_col0, out_row0) of frame 0
     long long out_pitch, out_frame_stride;
     int out_row0, out_rows;
     int seg_periods;      // vertical ratio-periods per segment
     int vperiod0;         // first vertical period covered by the launch (floor(out_row0 / N))
-    int out_w, in_row0;
+    int out_bytes, in_row0;
 };
 
 __host__ __device__ constexpr int cdiv(int a, int b) { return (a + b - 1) / b; }
@@ -243,22 +247,24 @@ EncodeFn get_encode() {
 // ---------------------------------------------------------------------------------------------
 // host side of a launch
 // ---------------------------------------------------------------------------------------------
-// Layout requirements of the TMA map and of the 32-bit accesses: input and output row bytes %4, input pitch %16,
-// output pitch %4, 16-byte aligned input base, 4-byte aligned output base, and the same for the frame strides.
+// Layout requirements of the TMA map and of the 32-bit accesses: input rect and output window row bytes %4, input
+// pitch %16, output pitch %4, 16-byte aligned input base, 4-byte aligned output base, and the same for the frame strides.
 inline bool strip_layout_ok(const KParams &k) {
-    if ((k.in_w * k.channels) % 4 != 0 || (k.out_w * k.channels) % 4 != 0) return false;
+    if ((k.in_cols * k.channels) % 4 != 0 || (k.out_cols * k.channels) % 4 != 0) return false;
     if (k.in_pitch % 16 != 0 || k.out_pitch % 4 != 0) return false;
     if ((reinterpret_cast<uintptr_t>(k.in) & 15) != 0 || (reinterpret_cast<uintptr_t>(k.out) & 3) != 0) return false;
     if (k.n_frames > 1 && (k.in_frame_stride % 16 != 0 || k.out_frame_stride % 4 != 0)) return false;
     return true;
 }
 
-// The input frames as a 3-D tensor of 32-bit words (x, row, frame), read in boxes of box_bytes x box_rows; TMA fills
-// what lies outside the image with zeros, which are the reference's dropped taps.
+// The input rect of the frames as a 3-D tensor of 32-bit words (x, row, frame), read in boxes of box_bytes x box_rows;
+// TMA fills what lies outside the rect with zeros.  At the image's edges those are the reference's dropped taps; inside
+// the image no window pixel has a tap outside the rect (the caller's rect covers them), so the zeros there only reach
+// samples outside the window, which are never stored.
 inline bool encode_input_map(CUtensorMap *map, const KParams &k, int box_bytes, int box_rows) {
     EncodeFn encode = get_encode();
     if (!encode) return false;
-    const cuuint64_t dims[3] = {(cuuint64_t)(k.in_w * k.channels / 4), (cuuint64_t)k.in_rows, (cuuint64_t)k.n_frames};
+    const cuuint64_t dims[3] = {(cuuint64_t)(k.in_cols * k.channels / 4), (cuuint64_t)k.in_rows, (cuuint64_t)k.n_frames};
     const cuuint64_t strides[2] = {(cuuint64_t)k.in_pitch, (cuuint64_t)(k.n_frames > 1 ? k.in_frame_stride : k.in_pitch * k.in_rows)};
     const cuuint32_t box[3] = {(cuuint32_t)(box_bytes / 4), (cuuint32_t)box_rows, 1};
     const cuuint32_t estr[3] = {1, 1, 1};
@@ -333,12 +339,12 @@ inline SegPlan plan_segments(int vperiods, int D, int A, int RB, long long cols,
     return split_periods(vperiods, segs);
 }
 
-// The StripParams of a launch over the band [out_row0, out_row0 + out_rows) of k
+// The StripParams of a launch over the window of k
 inline void set_strip_params(StripParams &p, const KParams &k, int vperiod0, int seg_periods) {
     p.out = k.out;
     p.out_pitch = k.out_pitch;
     p.out_frame_stride = k.out_frame_stride;
-    p.out_w = k.out_w;
+    p.out_bytes = k.out_cols * k.channels;
     p.out_row0 = k.out_row0; p.out_rows = k.out_rows; p.in_row0 = k.in_row0;
     p.seg_periods = seg_periods; p.vperiod0 = vperiod0;
 }
@@ -356,6 +362,8 @@ template <class G, class P, class Kernel>
 int launch_strips(Kernel kern, const CUtensorMap &map, P &p, const KParams &k, const FastHostTables &t, int strips,
                   int vperiod0, SegPlan sp, long long ctas, bool programmatic, LaunchShape *shape, cudaStream_t s) {
     set_strip_params(p, k, vperiod0, sp.seg_periods);
+    p.out_byte0 = k.out_col0 * k.channels;
+    p.in_byte0 = k.in_col0 * k.channels;
     fill_wtab(p.wtab, t, k.a, k.scale_n);
     p.strict_counter = k.strict_counter;
     const dim3 grid(strips, sp.segs, k.n_frames);

@@ -7,16 +7,18 @@ namespace lzb {
 
 // Everything a kernel needs about one launch. Device pointers unless noted.
 struct KParams {
-    const uint8_t *in;   // points at input row `in_row0` of frame 0
-    uint8_t *out;        // points at output row `out_row0` of frame 0
+    const uint8_t *in;   // points at input pixel (in_col0, in_row0) of frame 0
+    uint8_t *out;        // points at output pixel (out_col0, out_row0) of frame 0
     long long in_pitch, out_pitch;               // bytes
     long long in_frame_stride, out_frame_stride; // bytes
     int n_frames;
     int in_w, in_h, out_w, out_h;  // full image (global coordinates)
     int channels, a, taps;         // taps = 2a
     int scale_n, scale_d;
-    int out_row0, out_rows;        // band of output rows to produce
-    int in_row0, in_rows;          // input rows present in `in`
+    int out_row0, out_rows;        // window of output pixels to produce: rows ...
+    int out_col0, out_cols;        // ... and columns (global indices; phases follow them)
+    int in_row0, in_rows;          // input pixels present in `in`: rows ...
+    int in_col0, in_cols;          // ... and columns
     // per-coordinate tables (plan.h AxisTables)
     const int32_t *i0x; const float *wfx; const double *wdx;
     const int32_t *i0y; const float *wfy; const double *wdy;

@@ -36,6 +36,7 @@ struct DynParams : StripParams {
                               //    so the "cannot flip" test of lanczos_v6.cu (K = 3/8) decides most phase-0 samples
     float wtab[32 * 8];       // polyphase table [N][8] (padded to 8 taps), times 2^24
     unsigned long long *strict_counter;
+    int out_byte0, in_byte0;  // window columns of StripParams (last: see there)
 };
 
 // The dyn choices of the strip pipeline (StripGeo): strips of 128 output bytes, 4 per lane.
@@ -145,10 +146,12 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
     uint8_t *out_frame = p.out + (long long)frame * p.out_frame_stride;
 
     // horizontal extent
-    const int obyte0 = strip * SWB;
-    const int row_bytes = p.out_w * C;
+    const int obyte0 = p.out_byte0 + strip * SWB;             // global output byte column of the strip
+    const int row_bytes = p.out_byte0 + p.out_bytes;          // ... and the window's end
     const int valid_bytes = min(SWB, row_bytes - obyte0);     // > 0 by construction of the grid, multiple of 4
-    const int xbyte0 = ((p.i0x[obyte0 / C] * C) >> 4) << 4;   // staged rows start here (16-byte aligned, may be < 0)
+    // staged rows start at rect byte xbyte0 (16-byte aligned in the rect, may be < 0), which is global byte xbyte0g
+    const int xbyte0 = ((p.i0x[obyte0 / C] * C - p.in_byte0) >> 4) << 4;
+    const int xbyte0g = xbyte0 + p.in_byte0;
     SegRows sr;
     if (!segment_rows<A, N, D, RB>(p, seg, sr)) return;
     const int ys = sr.ys, ye = sr.ye, rs = sr.rs, nchunks = sr.nchunks;
@@ -188,7 +191,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
         const int ob = min(obyte0 + VB * lane + e, row_bytes - 1);
         const int xx = ob / C, c = ob - xx * C;
         const int ph = (xx * D) % N;
-        off[e] = p.i0x[xx] * C + c - xbyte0;
+        off[e] = p.i0x[xx] * C + c - xbyte0g;
 #pragma unroll
         for (int k = 0; k < TAPS; k++) wq[e][k] = p.wtab[ph * 8 + k] * kDenScale;   // exact: a power of two
         if (ph == 0) p0mask |= 0xffu << (8 * e);
@@ -236,7 +239,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
         p0_item[i] = -1;
         if (ob >= 0) {
             const int xx = ob / C, c = ob - xx * C;
-            p0_item[i] = (lr << 20) | ((ob - obyte0) << 12) | (p.i0x[xx] * C + c - xbyte0);
+            p0_item[i] = (lr << 20) | ((ob - obyte0) << 12) | (p.i0x[xx] * C + c - xbyte0g);
         }
     }
 
@@ -329,7 +332,7 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
     const uint8_t *vcol = &sm.ring[0][VB * lane];
     const int t0_first = (rs - A - G::S0) / D;                 // exact division (also for negative values)
     int ybase = N * t0_first;                                  // output row of bit 0 of `fixrows` for the current chunk
-    uint8_t *ocol = out_frame + obyte0 + VB * lane + (long long)(ybase - p.out_row0) * opitch;
+    uint8_t *ocol = out_frame + (obyte0 - p.out_byte0) + VB * lane + (long long)(ybase - p.out_row0) * opitch;
 
     auto v_pass = [&](int chunk) {
         const int bslot = (chunk % G::REGIONS) * RB;
@@ -433,12 +436,13 @@ lanczos_dyn_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
 template <int C, int A, int N, int D, int MODE>
 int launch_dyn_one(const KParams &k, const FastHostTables &t, LaunchShape *shape, cudaStream_t s) {
     using G = GeoD<C, A, N, D>;
-    const int row_bytes = k.out_w * C;
-    const int strips = (row_bytes + G::SWB - 1) / G::SWB;
-    // every strip's input must fit the staged row: check with the host copy of the tap table
+    const int byte0 = k.out_col0 * C, row_end = byte0 + k.out_cols * C, in_byte0 = k.in_col0 * C;
+    const int strips = (k.out_cols * C + G::SWB - 1) / G::SWB;
+    // every strip's input must fit the staged row: check with the host copy of the tap table (global byte columns;
+    // the box starts on a 16-byte boundary of the rect)
     for (int sI = 0; sI < strips; sI++) {
-        const int ob0 = sI * G::SWB, ob1 = std::min(row_bytes, ob0 + G::SWB) - 1;
-        const int xb0 = ((t.i0x_host[ob0 / C] * C) >> 4) << 4;
+        const int ob0 = byte0 + sI * G::SWB, ob1 = std::min(row_end, ob0 + G::SWB) - 1;
+        const int xb0 = (((t.i0x_host[ob0 / C] * C - in_byte0) >> 4) << 4) + in_byte0;
         const int last = (t.i0x_host[ob1 / C] + 2 * A) * C;      // one past the last byte read
         if (last - xb0 > G::BOX_B) return -1;
     }

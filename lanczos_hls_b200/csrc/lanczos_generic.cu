@@ -38,10 +38,10 @@ __global__ void __launch_bounds__(GT_THREADS) lanczos_generic_kernel(const KPara
 
     const int tid = threadIdx.x;
     const int taps = p.taps;
-    const int x0 = blockIdx.x * GT_W;                 // first output pixel of the tile
+    const int x0 = p.out_col0 + blockIdx.x * GT_W;    // first output pixel of the tile (global index)
     const int y0 = p.out_row0 + blockIdx.y * GT_H;    // first output row (global index)
     const int frame = blockIdx.z;
-    const int tw = min(GT_W, p.out_w - x0);
+    const int tw = min(GT_W, p.out_col0 + p.out_cols - x0);
     const int th = min(GT_H, p.out_row0 + p.out_rows - y0);
     const uint8_t *in = p.in + (long long)frame * p.in_frame_stride;
     uint8_t *out = p.out + (long long)frame * p.out_frame_stride;
@@ -62,7 +62,8 @@ __global__ void __launch_bounds__(GT_THREADS) lanczos_generic_kernel(const KPara
     const int ry0 = s_i0y[0];
     const int nrows = s_i0y[th - 1] + taps - ry0;    // input rows spanned (<= GT_IN_ROWS)
 
-    // stage the input tile + halo; everything outside the image is 0 (full_TB.h:59,72 drop those taps)
+    // stage the input tile + halo; everything outside the image is 0 (full_TB.h:59,72 drop those taps).  Inside the
+    // image every staged byte is a tap of a window pixel, so it lies in the supplied input rect.
     const int row_bytes = ncols * C;
     for (int idx = tid; idx < nrows * row_bytes; idx += GT_THREADS) {
         const int r = idx / row_bytes, b = idx - r * row_bytes;
@@ -70,7 +71,7 @@ __global__ void __launch_bounds__(GT_THREADS) lanczos_generic_kernel(const KPara
         const int gb = cx0 * C + b;
         uint8_t v = 0;
         if (gy >= 0 && gy < p.in_h && gb >= 0 && gb < p.in_w * C)
-            v = in[(long long)(gy - p.in_row0) * p.in_pitch + gb];
+            v = in[(long long)(gy - p.in_row0) * p.in_pitch + gb - p.in_col0 * C];
         s_in[r][b] = v;
     }
     __syncthreads();
@@ -106,7 +107,7 @@ __global__ void __launch_bounds__(GT_THREADS) lanczos_generic_kernel(const KPara
             q = strict_sample(w, taps, [&](int k) { return s_mid[rb + k][j]; });
             if (p.strict_counter) atomicAdd(p.strict_counter, 1ULL);
         }
-        out[(long long)(y0 + ly - p.out_row0) * p.out_pitch + (long long)x0 * C + j] = q;
+        out[(long long)(y0 + ly - p.out_row0) * p.out_pitch + (long long)(x0 - p.out_col0) * C + j] = q;
     }
 }
 
@@ -114,16 +115,17 @@ __global__ void __launch_bounds__(GT_THREADS) lanczos_generic_kernel(const KPara
 // The reference's column pass works in place from the bottom row up (full_TB.h:67-77).  Row xx
 // reads rows first..last of the same plane; every row i > xx in that window has already been
 // overwritten with its FINAL value, rows i <= xx still hold the horizontal result.  That only
-// happens for the first `alias_rows` rows.  One thread per output byte column walks rows
+// happens for the first `alias_rows` rows.  One thread per output byte column of the window walks rows
 // alias_top_row..0 with the reference's exact double arithmetic and writes rows < alias_rows.
 __global__ void __launch_bounds__(128) lanczos_alias_rows_kernel(const KParams p) {
     const int C = p.channels, taps = p.taps;
-    const long long col = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // output byte column
-    if (col >= (long long)p.out_w * C) return;
+    const long long col = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // output byte column of the window
+    if (col >= (long long)p.out_cols * C) return;
     const int frame = blockIdx.y;
     const uint8_t *in = p.in + (long long)frame * p.in_frame_stride;
     uint8_t *out = p.out + (long long)frame * p.out_frame_stride;
-    const int xx = (int)(col / C), c = (int)(col - (long long)xx * C);
+    const long long gcol = (long long)p.out_col0 * C + col;                  // ... and of the image
+    const int xx = (int)(gcol / C), c = (int)(gcol - (long long)xx * C);
     const int i0x = p.i0x[xx];
     double wx[8];
     for (int k = 0; k < taps; k++) wx[k] = p.wdx[(long long)xx * taps + k];
@@ -133,7 +135,7 @@ __global__ void __launch_bounds__(128) lanczos_alias_rows_kernel(const KParams p
         const uint8_t *row = in + (long long)(i - p.in_row0) * p.in_pitch;
         return strict_sample(wx, taps, [&](int k) -> uint8_t {
             const int px = i0x + k;
-            return (px >= 0 && px < p.in_w) ? row[(long long)px * C + c] : (uint8_t)0;
+            return (px >= 0 && px < p.in_w) ? row[(long long)(px - p.in_col0) * C + c] : (uint8_t)0;
         });
     };
 
@@ -182,7 +184,7 @@ __global__ void rgb_to_words_kernel(const uint8_t *rgb, uint32_t *words, long lo
 }  // namespace
 
 int launch_generic(const KParams &p, LaunchShape *shape, cudaStream_t s) {
-    dim3 grid((p.out_w + GT_W - 1) / GT_W, (p.out_rows + GT_H - 1) / GT_H, p.n_frames);
+    dim3 grid((p.out_cols + GT_W - 1) / GT_W, (p.out_rows + GT_H - 1) / GT_H, p.n_frames);
     *shape = LaunchShape{(int)grid.x, (int)grid.y, (int)grid.z};
     dim3 block(GT_THREADS);
     switch (p.channels) {
@@ -195,7 +197,7 @@ int launch_generic(const KParams &p, LaunchShape *shape, cudaStream_t s) {
 }
 
 int launch_alias_rows(const KParams &p, cudaStream_t s) {
-    const long long cols = (long long)p.out_w * p.channels;
+    const long long cols = (long long)p.out_cols * p.channels;
     dim3 grid((unsigned)((cols + 127) / 128), p.n_frames);
     lanczos_alias_rows_kernel<<<grid, 128, 0, s>>>(p);
     return (int)cudaGetLastError();

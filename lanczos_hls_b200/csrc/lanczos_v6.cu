@@ -62,6 +62,7 @@ struct V6Params : StripParams {
     float p0c[5];
     float wtab[32 * 8];       // polyphase table [N][8] (padded to 8 taps), N <= 32, times 2^24
     double wdtab[8 * 8];      // double polyphase table [N][8] for N <= 8 (valid when uniform_*)
+    int out_byte0, in_byte0;  // window columns of StripParams (last: see there)
 };
 
 __host__ __device__ constexpr int cmax6(int a, int b) { return a > b ? a : b; }
@@ -476,19 +477,25 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
     // (both are no-ops for a launch without the attribute)
     asm volatile("griddepcontrol.launch_dependents;");
     if (!p.independent) asm volatile("griddepcontrol.wait;" ::: "memory");
-    if (strip * G::SWV >= p.out_w * C) return;
+    if (strip * G::SWV >= p.out_bytes) return;
     uint8_t *out_frame = p.out + (long long)frame * p.out_frame_stride;
 
-    // horizontal extent
-    const int vbyte0 = strip * G::SWV;                        // first output byte column of the strip (V pass, stores)
-    const int row_bytes = p.out_w * C;
-    const int valid_bytes = min(G::SWV, row_bytes - vbyte0);  // > 0 by construction of the grid
-    const int obyte0 = (vbyte0 / G::OUT_B) * G::OUT_B;        // first output byte column of the H items that cover it
-    const int voff = vbyte0 - obyte0;                         // 0, 16 or 32 for 48-byte items
+    // horizontal extent: the strip is window bytes [vbyte0, vbyte0 + SWV), global bytes from p.out_byte0 + vbyte0.
+    // H items stay aligned to OUT_B in global bytes, so the phase pattern is the static one of the full image.
+    const int vbyte0 = strip * G::SWV;                        // first window byte column of the strip (V pass, stores)
+    const int valid_bytes = min(G::SWV, p.out_bytes - vbyte0);   // > 0 by construction of the grid
+    const int gbyte0 = p.out_byte0 + vbyte0;                  // ... as a global byte column
+    const int obyte0 = (gbyte0 / G::OUT_B) * G::OUT_B;        // first global output byte column of the H items that cover it
+    const int voff = gbyte0 - obyte0;                         // 0, 16 or 32 for 48-byte items (<= VOFF_MAX: launch_v6_one)
     const int groups = min(G::MAX_GROUPS, (voff + valid_bytes + G::OUT_B - 1) / G::OUT_B);
-    const int hvalid = min(groups * G::OUT_B, row_bytes - obyte0);   // bytes of the H items inside the image
-    const int ibyte0 = (obyte0 / (N * C)) * (D * C);          // first input byte column of the H items
-    const int xshift = (ibyte0 - G::PAD_L) & 15;              // 0 or 8: the TMA box starts that many bytes early
+    const int hvalid = min(groups * G::OUT_B, p.out_byte0 + p.out_bytes - obyte0);   // bytes of the H items inside the window
+    const int ibyte0 = (obyte0 / (N * C)) * (D * C);          // first global input byte column of the H items
+    const int rbyte0 = ibyte0 - p.in_byte0;                   // ... in the input rect
+    const int xshift = (rbyte0 - G::PAD_L) & 15;              // 0 or 8: the TMA box starts that many bytes early
+    // what the out-of-line h_fix needs, held in registers: recomputed from the window inside the H loop, it took the
+    // headline kernel's H loop from 478 to 485 instructions (480 with this)
+    int hvalid_r = hvalid, obyte0_r = obyte0, ibyte0_r = ibyte0;
+    asm volatile("" : "+r"(hvalid_r), "+r"(obyte0_r), "+r"(ibyte0_r));
     SegRows sr;
     if (!segment_rows<A, N, D, G::RB>(p, seg, sr)) return;
     const int ys = sr.ys, ye = sr.ye, rs = sr.rs, nchunks = sr.nchunks;
@@ -506,7 +513,7 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
     auto issue = [&](int chunk) {
         const uint32_t bar = full0 + 8 * (chunk % G::STAGES);
         mbar_expect_tx(bar, kStageBytes);
-        tma_load_3d(smem_u32(&sm.in[chunk % G::STAGES][0]), &in_map, (ibyte0 - G::PAD_L - xshift) / 4, rs + chunk * G::RB - p.in_row0, frame, bar);
+        tma_load_3d(smem_u32(&sm.in[chunk % G::STAGES][0]), &in_map, (rbyte0 - G::PAD_L - xshift) / 4, rs + chunk * G::RB - p.in_row0, frame, bar);
     };
     if (tid == 0) {
         for (int i = 0; i < G::STAGES && i < nchunks; i++) issue(i);
@@ -688,7 +695,7 @@ lanczos_v6_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_const
                 HFixArgs a;
                 const int lr = item / groups, g = item - lr * groups;
                 a.in_row = &sm.in[st][lr * G::BOX_B + xshift]; a.ring_row = drow; a.gbyte0 = g * G::OUT_B;
-                a.obyte0 = obyte0; a.ibyte0 = ibyte0; a.valid_bytes = hvalid;
+                a.obyte0 = obyte0_r; a.ibyte0 = ibyte0_r; a.valid_bytes = hvalid_r;
                 a.fix_g = fix_g; a.guard = guard_h;
                 n_strict += h_fix<G, C, A, N, D, PH>(p, a);
             }
@@ -941,13 +948,18 @@ SegPlan plan_v6_segments(int vperiods, int D, int A, int RB, long long cols, lon
 template <int C, int A, int N, int D, int PH, int KM, int MODE, bool ST64>
 int launch_v6_one(const KParams &k, const FastHostTables &t, int *alias_in_kernel, LaunchShape *shape, cudaStream_t s) {
     using G = Geo6<C, A, N, D, PH, MODE>;
+    // A window keeps the static phase pattern when its strips start at most VOFF_MAX bytes into their first H item
+    // (H items are aligned to OUT_B in global bytes), and the TMA box keeps its start when the input rect begins on the
+    // 16-byte grid of the image (or on its 8-byte grid where the box has XSHIFT_MAX = 8 spare bytes).
+    if ((k.out_col0 * C) % gcd6(G::SWV, G::OUT_B) != 0) return -1;
+    if ((k.in_col0 * C) % (G::XSHIFT_MAX == 8 ? 8 : 16) != 0) return -1;
     CUtensorMap map;
     if (!encode_input_map(&map, k, G::BOX_B, G::RB)) return -1;
     auto kern = lanczos_v6_kernel<C, A, N, D, PH, KM, MODE, ST64>;
     static std::atomic<int> ctas_per_sm[64] = {};
     const Residency res = resident_ctas(ctas_per_sm, kern, strip_smem_bytes<G>());
     if (res.ctas == 0) return -1;
-    const int strips = (k.out_w * C + G::SWV - 1) / G::SWV;   // one strip of SWV = 256 output bytes per warp
+    const int strips = (k.out_cols * C + G::SWV - 1) / G::SWV;   // one strip of SWV = 256 window bytes per warp
     const long long cols = (long long)strips * k.n_frames;
     const int vperiod0 = k.out_row0 / N;
     const int vperiods = (k.out_row0 + k.out_rows + N - 1) / N - vperiod0;
@@ -983,7 +995,7 @@ int launch_v6(const KParams &k, const FastHostTables &t, int *kernel_id, int *al
               cudaStream_t s) {
     if (!strip_layout_ok(k)) return -1;
     // 64-bit stores of the V pass
-    const bool st64 = (k.out_w * k.channels) % 8 == 0 && k.out_pitch % 8 == 0 && (reinterpret_cast<uintptr_t>(k.out) & 7) == 0 &&
+    const bool st64 = (k.out_cols * k.channels) % 8 == 0 && k.out_pitch % 8 == 0 && (reinterpret_cast<uintptr_t>(k.out) & 7) == 0 &&
                       (k.n_frames <= 1 || k.out_frame_stride % 8 == 0);
     if (!t.exact_x || !t.exact_y) return -1;     // phase-0 coordinates not exactly integral in double: other kernels
     const int mode = (k.flags & LANCZOS_FLAG_TOLERANCE_1LSB) ? 1 : 0;

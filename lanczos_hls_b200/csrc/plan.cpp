@@ -287,4 +287,12 @@ void band_rows(const Plan &p, int out_row0, int out_rows, int *in_row0, int *in_
     *in_rows = hi - lo + 1;
 }
 
+void band_cols(const Plan &p, int out_col0, int out_cols, int *in_col0, int *in_cols) {
+    const int lo = std::min(p.d.in_w - 1, std::max(0, p.x.i0[out_col0]));
+    int hi = std::min(p.d.in_w - 1, p.x.i0[out_col0 + out_cols - 1] + p.taps - 1);
+    if (hi < lo) hi = lo;
+    *in_col0 = lo;
+    *in_cols = hi - lo + 1;
+}
+
 }  // namespace lzb

@@ -69,5 +69,7 @@ bool float_floor_exact(int from, int to, int n, int d);
 
 // Input row range needed for a band of output rows (global indices).
 void band_rows(const Plan &p, int out_row0, int out_rows, int *in_row0, int *in_rows);
+// Its column twin: input column range needed for a range of output columns (global indices).
+void band_cols(const Plan &p, int out_col0, int out_cols, int *in_col0, int *in_cols);
 
 }  // namespace lzb
