@@ -8,19 +8,17 @@ chain (tests/golden/near_ties_any_ratio.npz), on flat and dark patches, at ratio
 at output sizes unrelated to the ratio and on buffer layouts the specialised kernels decline.  The oracle stays the
 truth: every byte must equal it.
 """
-import ctypes as C
 import math
 import os
 
 import numpy as np
 import pytest
 
-import test_near_ties as NTT
-from util import dark_hwc, noise_hwc
+from harness import canary_call, device_upscale, torch_cuda  # noqa: F401
+from util import (KERNEL_OF, NEAR, NT, WRONG, config_rows, dark_hwc, h_image, noise_hwc, planar, strict_floor, tap0,
+                  up_len, v_image)
 
-NT = NTT.NT
 HERE = os.path.dirname(os.path.abspath(__file__))
-TIE, WRONG, NEAR = NT.TIE, NT.WRONG, NT.NEAR
 
 
 def any_windows():
@@ -29,7 +27,6 @@ def any_windows():
 
 
 ANY = any_windows()
-INSTANCE_OF = {v: k for k, v in NTT.INSTANCES.items()}          # (C, a, N, D) -> kernel id
 
 
 def reduced_ratios(limit):
@@ -147,13 +144,6 @@ def test_alias_rows_and_band_rows_at_every_ratio(lz):
 
 # ---- GPU tests ---------------------------------------------------------------------------------------------
 
-@pytest.fixture(scope="module")
-def torch_cuda():
-    import torch
-    assert torch.cuda.is_available(), "GPU tests need a CUDA device"
-    return torch
-
-
 def patch_image(oracle, h, w, c, seed):
     """Top half dark noise (0..15), bottom half flat 8x8 blocks of extreme and middle values."""
     img = dark_hwc(oracle, h, w, c, seed=seed)
@@ -181,35 +171,23 @@ def sweep_cases():
 SWEEP = sweep_cases()
 
 
-def run_device(torch, lz, img, ow, oh, a, n, d, flags, stats):
-    d_in = torch.from_numpy(img).cuda()
-    d_out = torch.empty((oh, ow, img.shape[2]), dtype=torch.uint8, device="cuda")
-    lz.enable_stats(stats)
-    try:
-        lz.upscale_device(d_in, d_out, a=a, scale_n=n, scale_d=d, flags=flags)
-        torch.cuda.synchronize()
-        st = lz.stats()
-    finally:
-        lz.enable_stats(False)
-    return d_out.cpu().numpy(), st
-
-
 def check_all_paths(torch, lz, oracle, img, planted, a, n, d, what):
     """Default dispatch and FLAG_GENERIC_KERNEL, each with the in-place top rows and with FLAG_NO_ALIAS: bit for bit,
     the expected kernel, and on the generic kernel every planted near and wrong-side window re-evaluated."""
     h, w, c = img.shape
     ow, oh = w * n // d, h * n // d
-    kid = INSTANCE_OF.get((c, a, n, d), 0)                   # every image here has a layout the instances take
+    kid = KERNEL_OF.get((c, a, n, d), 0)                   # every image here has a layout the instances take
     for variant, alias_flag in ((oracle.VERBATIM, 0), (oracle.CLEAN, lz.FLAG_NO_ALIAS)):
         want = oracle.upscale(img, ow, oh, a, n, d, variant=variant)
         for generic in (False, True):
-            got, st = run_device(torch, lz, img, ow, oh, a, n, d, alias_flag | (lz.FLAG_GENERIC_KERNEL if generic else 0),
+            got = device_upscale(torch, lz, img, ow, oh, a, n, d, alias_flag | (lz.FLAG_GENERIC_KERNEL if generic else 0),
                                  stats=True)
+            st = lz.stats()
             assert st["kernel_id"] == (0 if generic else kid), (what, generic, st)
             bad = np.argwhere(got != want)
             assert len(bad) == 0, (what, "generic" if generic else "default", variant, len(bad), bad[:8].tolist())
             if st["kernel_id"] == 0:
-                assert st["strict_samples"] >= NTT.strict_floor(planted, ANY), (what, st, NTT.strict_floor(planted, ANY))
+                assert st["strict_samples"] >= strict_floor(planted, ANY), (what, st, strict_floor(planted, ANY))
 
 
 @pytest.mark.gpu
@@ -218,12 +196,12 @@ def test_every_ratio_bit_exact(torch_cuda, lz, oracle, case):
     n, d, a, c, size = case
     seed = 97 * n + 13 * d + a
     if size is None:
-        img, hp = NTT.h_image(oracle, n, d, a, c, seed=seed, win=ANY)
+        img, hp = h_image(oracle, n, d, a, c, seed=seed, win=ANY)
         check_all_paths(torch_cuda, lz, oracle, img, hp, a, n, d, "H windows")
-        in_h = max([NTT.tap0(int(x), n, d, a) + 2 * a for x in ANY["coord"][NTT.config_rows(n, d, a, ANY)]] + [64]) + 4
-        ow = NTT.up_len(16 * d, n, d)
-        top = lz.alias_rows(lz.make_desc(16 * d, in_h, ow, NTT.up_len(in_h, n, d), c, a, n, d))
-        img, vp = NTT.v_image(oracle, n, d, a, c, seed=seed, nblk=8, win=ANY,
+        in_h = max([tap0(int(x), n, d, a) + 2 * a for x in ANY["coord"][config_rows(n, d, a, ANY)]] + [64]) + 4
+        ow = up_len(16 * d, n, d)
+        top = lz.alias_rows(lz.make_desc(16 * d, in_h, ow, up_len(in_h, n, d), c, a, n, d))
+        img, vp = v_image(oracle, n, d, a, c, seed=seed, nblk=8, win=ANY,
                               place=lambda i: int(ANY["coord"][i]) if ANY["coord"][i] >= max(top, 1) else None)
         check_all_paths(torch_cuda, lz, oracle, img, vp, a, n, d, "V windows")
         iw, ih = 16 * d * max(1, -(-256 * d // n) // (16 * d)), max(2 * a, 256 * d // n)
@@ -261,47 +239,7 @@ def test_bands_through_the_alias_rows(torch_cuda, lz, oracle, case):
         assert len(bad) == 0, (cuts, len(bad), bad[:8].tolist())
 
 
-# ---- raw launches with canaries ----------------------------------------------------------------------------
-
-CANARY = 0x5C
-
-
-def launch_raw(torch, lz, frames, ow, oh, a, n, d, in_off=0, in_pad=0, in_gap=0, out_off=0, out_pad=0, flags=0):
-    """One call on device buffers laid out as asked: the input base `in_off` bytes past a 256-byte boundary, rows
-    padded by `in_pad` bytes, frames `in_gap` bytes apart; the output likewise, surrounded by canary bytes.  Returns
-    (outputs, kernel id) after checking every canary."""
-    nf = len(frames)
-    ih, iw, c = frames[0].shape
-    in_pitch, out_pitch = iw * c + in_pad, ow * c + out_pad
-    in_fs = in_pitch * ih + in_gap
-    src = np.zeros(in_off + in_fs * nf + 64, np.uint8)
-    for f, img in enumerate(frames):
-        v = np.lib.stride_tricks.as_strided(src[in_off + f * in_fs:], shape=(ih, iw * c), strides=(in_pitch, 1))
-        v[...] = img.reshape(ih, iw * c)
-    out_fs = out_pitch * oh + 4
-    lead = 64 + out_off
-    total = lead + out_fs * nf + 2 * out_pitch + 64
-    d_in = torch.from_numpy(src).cuda()
-    buf = torch.full((total,), CANARY, dtype=torch.uint8, device="cuda")
-    assert d_in.data_ptr() % 256 == 0 and buf.data_ptr() % 256 == 0
-    desc = lz.make_desc(iw, ih, ow, oh, c, a, n, d, in_pitch, out_pitch, flags)
-    stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-    L = lz.lib()
-    rc = L.lanczos_b200_upscale_batch(C.byref(desc), C.c_void_p(d_in.data_ptr() + in_off),
-                                      C.c_void_p(buf.data_ptr() + lead), nf, in_fs, out_fs, 0, stream)
-    torch.cuda.synchronize()
-    assert rc == 0, (rc, L.lanczos_b200_strerror(rc))
-    kid = lz.stats()["kernel_id"]
-    host = buf.cpu().numpy()
-    rb = ow * c
-    view = np.lib.stride_tricks.as_strided(host[lead:], shape=(nf, oh, rb), strides=(out_fs, out_pitch, 1))
-    outs = [np.array(view[f]).reshape(oh, ow, c) for f in range(nf)]
-    canary = np.ones(total, bool)
-    np.lib.stride_tricks.as_strided(canary[lead:], shape=(nf, oh, rb), strides=(out_fs, out_pitch, 1))[...] = False
-    hit = np.nonzero(canary & (host != CANARY))[0]
-    assert len(hit) == 0, ("canary bytes overwritten", len(hit), [int(i) - lead for i in hit[:8]])
-    return outs, kid
-
+# ---- raw lanczos_b200_upscale_batch calls with canaries, output frames 4 bytes apart ----------------------
 
 # (channels, a, N, D, input width, input height) of the generic kernel, one v6 and one dyn instance
 FAMILIES = {"generic": (3, 3, 5, 4, 64, 40), "v6": (3, 3, 2, 1, 64, 40), "dyn": (3, 2, 3, 1, 48, 36)}
@@ -313,13 +251,14 @@ def test_output_size_independent_of_ratio_any_kernel(torch_cuda, lz, oracle, fam
     """Output widths below and far above in_w*N/D (columns with no tap inside the image), narrower than the input,
     and heights past in_h*N/D with a band entirely below the input: every kernel takes the sizes as loop bounds."""
     c, a, n, d, iw, ih = FAMILIES[family]
-    kid = INSTANCE_OF.get((c, a, n, d), 0)
+    kid = KERNEL_OF.get((c, a, n, d), 0)
     img = noise_hwc(oracle, ih, iw, c, seed=5)
     full_w, full_h = iw * n // d, ih * n // d
     empty_w = (iw + a + 2) * n // d + 8                           # past this column no tap lies inside the image
     for (ow, oh) in [(full_w - 12, full_h), (empty_w // 4 * 4 + 16, full_h), (iw - 8, ih + 4), (full_w, full_h + 24 * n)]:
-        outs, got_kid = launch_raw(torch_cuda, lz, [img], ow, oh, a, n, d)
-        assert got_kid == kid, (family, ow, oh, got_kid)
+        desc = lz.make_desc(iw, ih, ow, oh, c, a, n, d)
+        outs, st, _ = canary_call(torch_cuda, lz, desc, [img], "upscale_batch", out_gap=4)
+        assert st["kernel_id"] == kid, (family, ow, oh, st)
         want = oracle.upscale(img, ow, oh, a, n, d)
         assert np.array_equal(outs[0], want), (family, ow, oh)
     # a band that lies entirely below the last input row
@@ -349,7 +288,7 @@ BROKEN = {
 @pytest.mark.parametrize("layout", sorted(BROKEN))
 def test_layouts_the_instances_decline_fall_back(torch_cuda, lz, oracle, family, layout):
     c, a, n, d, iw, ih = FAMILIES[family]
-    kid = INSTANCE_OF[(c, a, n, d)]
+    kid = KERNEL_OF[(c, a, n, d)]
     kw = dict(BROKEN[layout])
     nf = kw.pop("frames", 1)
     frames = [noise_hwc(oracle, ih, iw, c, seed=f + 1) for f in range(nf)]
@@ -357,9 +296,10 @@ def test_layouts_the_instances_decline_fall_back(torch_cuda, lz, oracle, family,
     ow, oh = iw * n // d, ih * n // d
     for flags, variant in ((0, oracle.VERBATIM), (lz.FLAG_NO_ALIAS, oracle.CLEAN)):
         twin = {k: 16 for k in kw}                                          # the same offsets, aligned
+        desc = lz.make_desc(iw, ih, ow, oh, c, a, n, d, flags=flags)
         for args, want_kid in ((kw, 0), (twin, kid)):
-            outs, got_kid = launch_raw(torch_cuda, lz, frames, ow, oh, a, n, d, flags=flags, **args)
-            assert got_kid == want_kid, (family, layout, args, got_kid)
+            outs, st, _ = canary_call(torch_cuda, lz, desc, frames, "upscale_batch", out_gap=4, **args)
+            assert st["kernel_id"] == want_kid, (family, layout, args, st)
             for f, img in enumerate(frames):
                 assert np.array_equal(outs[f], oracle.upscale(img, ow, oh, a, n, d, variant=variant)), (layout, args, f)
 
@@ -377,9 +317,9 @@ def test_host_entry_points_accept_what_the_device_accepts(torch_cuda, lz, oracle
     img = noise_hwc(oracle, ih, iw, c, seed=iw)
     img[: ih // 2, : iw // 2] = dark_hwc(oracle, ih // 2, iw // 2, c, seed=3)
     want = oracle.upscale(img, ow, oh, a, n, d)
-    dev, _ = run_device(torch_cuda, lz, img, ow, oh, a, n, d, 0, stats=False)
+    dev = device_upscale(torch_cuda, lz, img, ow, oh, a, n, d)
     assert np.array_equal(dev, want)
     assert np.array_equal(lz.upscale(img, ow, oh, a=a, scale_n=n, scale_d=d), want), "upscale"
     assert np.array_equal(lz.upscale_bands_multi_gpu(img, ow, oh, [0, 0], a=a, scale_n=n, scale_d=d), want), "bands"
-    got = lz.lanczos_expected(NTT.to_planar(img), ow, oh, a=a, scale_n=n, scale_d=d)
-    assert np.array_equal(got, oracle.expected_planar(NTT.to_planar(img), ow, oh, a, n, d)), "lanczos_expected"
+    got = lz.lanczos_expected(planar(img), ow, oh, a=a, scale_n=n, scale_d=d)
+    assert np.array_equal(got, oracle.expected_planar(planar(img), ow, oh, a, n, d)), "lanczos_expected"

@@ -13,11 +13,9 @@ import concurrent.futures
 import numpy as np
 import pytest
 
-import test_near_ties as TN
-from util import noise_hwc, smooth_hwc
+from harness import torch_cuda  # noqa: F401
+from util import NEAR, NT, V_TOP, WIN, WRONG, config_rows, noise_hwc, planted_counts, smooth_hwc, strict_floor, v_image
 
-NT = TN.NT
-WIN = TN.WIN
 CANARY = 0xA5
 TAIL = 1 << 16          # canary bytes after the last output frame
 EDGE_ROWS = 16          # top and bottom output rows checked in every frame
@@ -57,13 +55,13 @@ def near_tie_rows(n, d, a, oh, boundary):
     groups = [list(range(boundary, boundary + span)), list(range(boundary - span, boundary)),
               list(range(oh - span, oh - a * n // d))]
     mid, last = {}, {}
-    for j, i in enumerate(TN.config_rows(n, d, a)):
+    for j, i in enumerate(config_rows(n, d, a)):
         g = j % 3
         yy = relocate(i, groups[g], n, d, a)
         if yy is None:
             yy = int(WIN["coord"][i])
             g = 0
-            if not TN.V_TOP <= yy < oh - 2 * a * n // d:
+            if not V_TOP <= yy < oh - 2 * a * n // d:
                 continue
         (last if g == 2 else mid)[int(i)] = yy
     return mid, last
@@ -105,13 +103,6 @@ def test_oracle_bands_equal_the_whole_frame(oracle):
 
 
 # ---- GPU helpers ------------------------------------------------------------------------------------
-
-@pytest.fixture(scope="module")
-def torch_cuda():
-    import torch
-    assert torch.cuda.is_available(), "GPU tests need a CUDA device"
-    return torch
-
 
 def need_memory(torch, nbytes):
     free, _ = torch.cuda.mem_get_info()
@@ -227,7 +218,7 @@ def batch_case(torch, lz, oracle, shape, seed, flags_list=(0,), min_chunks=0, pl
                     torch.cuda.synchronize()
                 finally:
                     lz.enable_stats(False)
-                assert st["strict_samples"] >= TN.strict_floor(planted), (st, TN.strict_floor(planted))
+                assert st["strict_samples"] >= strict_floor(planted), (st, strict_floor(planted))
             variant = oracle.CLEAN if flags & lz.FLAG_NO_ALIAS else oracle.VERBATIM
             compare_batch(torch, oracle, d_in, d_out, shape, launch, whole_frames(F), variant)
             assert_tail(torch, buf, n_out)
@@ -245,13 +236,13 @@ def plant_near_ties(torch, oracle, d_in, shape, launch):
     f_mid = 2 * (F // 4) + 1
     planted = []
     for f, rows in ((f_mid, mid), (F - 1, last)):
-        img, p = TN.v_image(oracle, n, d, a, c, base=d_in[f].cpu().numpy(), place=rows.get)
+        img, p = v_image(oracle, n, d, a, c, base=d_in[f].cpu().numpy(), place=rows.get)
         for (_, _, _, i) in p:
             assert NT.classify(WIN["win"][i], rows[i], n, d, a)[0] == WIN["cls"][i]
         d_in[f].copy_(torch.from_numpy(img))
         planted += p
-    counts = TN.planted_counts(planted)
-    assert counts[TN.NEAR] + counts[TN.WRONG] > 0, counts
+    counts = planted_counts(planted)
+    assert counts[NEAR] + counts[WRONG] > 0, counts
     return planted
 
 

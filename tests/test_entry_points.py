@@ -9,24 +9,13 @@ on their own scratch buffers.  The GPU tests pin what their counters report agai
 same work.
 """
 import ctypes as C
-import threading
 
 import numpy as np
 import pytest
 
+from harness import (ERR_ALIGN, ERR_CUDA, ERR_DIMS, ERR_NULL, ERR_TAPS, NO_DEVICE, device_upscale, in_thread,  # noqa: F401
+                     torch_cuda)
 from util import noise_hwc, planar
-
-NO_DEVICE = 1 << 20
-ERR_NULL, ERR_DIMS, ERR_TAPS, ERR_CUDA, ERR_ALIGN = -1, -2, -4, -8, -10
-
-
-def in_thread(fn):
-    """fn() on a thread of its own: the failed cudaSetDevice stays in that thread's CUDA error state."""
-    out = []
-    t = threading.Thread(target=lambda: out.append(fn()))
-    t.start()
-    t.join()
-    return out[0]
 
 
 def entry_calls(lz, desc, null=False):
@@ -102,13 +91,6 @@ HOST_CASES = {
 }
 
 
-@pytest.fixture(scope="module")
-def torch_cuda():
-    import torch
-    assert torch.cuda.is_available(), "GPU tests need a CUDA device"
-    return torch
-
-
 def band_call(torch, lz, desc, img, r0, rows):
     """Output rows [r0, r0 + rows) of img through lanczos_b200_upscale_band: (rows, stats, launch)."""
     in0, inn = lz.band_input_rows(desc, r0, rows)
@@ -121,10 +103,7 @@ def band_call(torch, lz, desc, img, r0, rows):
 
 def frame_call(torch, lz, case, img):
     iw, ih, ow, oh, c, a, n, d, flags = case
-    d_out = torch.empty((oh, ow, c), dtype=torch.uint8, device="cuda")
-    lz.upscale_device(torch.from_numpy(img).cuda(), d_out, a, n, d, flags)
-    torch.cuda.synchronize()
-    return d_out.cpu().numpy(), lz.stats(), lz.launch()
+    return device_upscale(torch, lz, img, ow, oh, a, n, d, flags), lz.stats(), lz.launch()
 
 
 @pytest.mark.gpu

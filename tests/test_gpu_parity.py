@@ -8,24 +8,10 @@ import os
 import numpy as np
 import pytest
 
-from util import dark_hwc, diff_stats, golden_files, interleaved, noise_hwc, planar, smooth_hwc
+from harness import device_upscale, torch_cuda  # noqa: F401
+from util import dark_hwc, diff_stats, golden_files, interleaved, noise_hwc, patchwork_hwc, planar, smooth_hwc
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module")
-def torch_cuda():
-    import torch
-    assert torch.cuda.is_available(), "GPU tests need a CUDA device"
-    return torch
-
-
-def gpu_upscale(torch, lz, img, ow, oh, a, n, d, flags=0):
-    d_in = torch.from_numpy(img).cuda()
-    d_out = torch.empty((oh, ow, img.shape[2]), dtype=torch.uint8, device="cuda")
-    lz.upscale_device(d_in, d_out, a=a, scale_n=n, scale_d=d, flags=flags)
-    torch.cuda.synchronize()
-    return d_out.cpu().numpy()
 
 
 SMALL = [  # in_w, in_h, n, d, a, c
@@ -43,11 +29,11 @@ def test_small_images_bit_exact(torch_cuda, lz, oracle, cfg, kind):
     ow, oh = oracle.out_dims(iw, ih, n, d)
     img = {"noise": noise_hwc, "smooth": smooth_hwc, "dark": dark_hwc}[kind](oracle, ih, iw, c, seed=iw)
     want = oracle.upscale(img, ow, oh, a, n, d, variant=oracle.VERBATIM)
-    got = gpu_upscale(torch_cuda, lz, img, ow, oh, a, n, d)
+    got = device_upscale(torch_cuda, lz, img, ow, oh, a, n, d)
     st = diff_stats(got, want)
     assert st["n_diff"] == 0, st
     want_clean = oracle.upscale(img, ow, oh, a, n, d, variant=oracle.CLEAN)
-    got_clean = gpu_upscale(torch_cuda, lz, img, ow, oh, a, n, d, flags=lz.FLAG_NO_ALIAS)
+    got_clean = device_upscale(torch_cuda, lz, img, ow, oh, a, n, d, flags=lz.FLAG_NO_ALIAS)
     assert np.array_equal(got_clean, want_clean)
 
 
@@ -78,9 +64,9 @@ def test_structured_known_answers(torch_cuda, lz, oracle):
         for (n, d) in [(2, 1), (3, 2), (17, 10)]:
             ow, oh = oracle.out_dims(w, h, n, d)
             want = oracle.upscale(img, ow, oh, 3, n, d)
-            got = gpu_upscale(torch_cuda, lz, img, ow, oh, 3, n, d)
+            got = device_upscale(torch_cuda, lz, img, ow, oh, 3, n, d)
             assert np.array_equal(got, want), (name, n, d)
-    assert not gpu_upscale(torch_cuda, lz, imgs["zero"], 128, 96, 3, 2, 1).any()
+    assert not device_upscale(torch_cuda, lz, imgs["zero"], 128, 96, 3, 2, 1).any()
 
 
 def test_batch_equals_single_frames(torch_cuda, lz, oracle):
@@ -201,7 +187,7 @@ def test_stream_shim_after_a_pitched_call_on_the_same_geometry(torch_cuda, lz, o
     got = np.stack([(out >> (8 * i)) & 0xFF for i in range(3)], axis=-1).astype(np.uint8)
     assert np.array_equal(got, want)
     # and the dense device entry point after the padded one
-    assert np.array_equal(gpu_upscale(torch, lz, img, ow, oh, 3, 2, 1), want)
+    assert np.array_equal(device_upscale(torch, lz, img, ow, oh, 3, 2, 1), want)
 
 
 @pytest.mark.parametrize("cfg", [(50, 33, 2, 1, 3), (64, 40, 2, 1, 3), (44, 30, 3, 2, 4)])
@@ -324,7 +310,7 @@ def test_headline_config_full_size(torch_cuda, lz, oracle):
     """BASELINE config 2: 1920x1080 -> 3840x2160 RGB8, 2x, Lanczos-3, uniform noise, full frame."""
     img = noise_hwc(oracle, 1080, 1920, 3, seed=0)
     want = oracle.upscale(img, 3840, 2160, 3, 2, 1)
-    got = gpu_upscale(torch_cuda, lz, img, 3840, 2160, 3, 2, 1)
+    got = device_upscale(torch_cuda, lz, img, 3840, 2160, 3, 2, 1)
     st = diff_stats(got, want)
     assert st["n_diff"] == 0, st
 
@@ -333,7 +319,7 @@ def test_config3_rgba_three_halves_full_size(torch_cuda, lz, oracle):
     """BASELINE config 3 (one frame of the batch): 2560x1440 -> 3840x2160 RGBA8, 3/2 via gcd."""
     img = smooth_hwc(oracle, 1440, 2560, 4, seed=1)
     want = oracle.upscale(img, 3840, 2160, 3, 3, 2)
-    got = gpu_upscale(torch_cuda, lz, img, 3840, 2160, 3, 0, 0)
+    got = device_upscale(torch_cuda, lz, img, 3840, 2160, 3, 0, 0)
     assert np.array_equal(got, want)
 
 
@@ -346,10 +332,10 @@ def test_config5_shape_reduced_and_properties(torch_cuda, lz, oracle):
     ow = oh = 2048 * 17 // 10
     assert (ow * 3) % 16 != 0
     want = oracle.upscale(img, ow, oh, 3, 17, 10)
-    assert np.array_equal(gpu_upscale(torch, lz, img, ow, oh, 3, 17, 10), want)
+    assert np.array_equal(device_upscale(torch, lz, img, ow, oh, 3, 17, 10), want)
     big = np.tile(img, (2, 2, 1))
     bw = bh = 4096 * 17 // 10
-    full = gpu_upscale(torch, lz, big, bw, bh, 3, 17, 10)
+    full = device_upscale(torch, lz, big, bw, bh, 3, 17, 10)
     desc = lz.make_desc(4096, 4096, bw, bh, 3, 3, 17, 10)
     for rank in range(8):
         r0, r1 = band_range(bh, rank, 8)
@@ -400,13 +386,9 @@ def test_config5_full_size_hash(torch_cuda, lz, oracle, cfg):
 
 def test_determinism_and_strict_counter(torch_cuda, lz, oracle):
     img = noise_hwc(oracle, 270, 480, 3, seed=6)
-    a = gpu_upscale(torch_cuda, lz, img, 960, 540, 3, 2, 1)
-    lz.enable_stats(True)
-    try:
-        b = gpu_upscale(torch_cuda, lz, img, 960, 540, 3, 2, 1)
-        st = lz.stats()
-    finally:
-        lz.enable_stats(False)
+    a = device_upscale(torch_cuda, lz, img, 960, 540, 3, 2, 1)
+    b = device_upscale(torch_cuda, lz, img, 960, 540, 3, 2, 1, stats=True)
+    st = lz.stats()
     assert np.array_equal(a, b)
     assert st["kernel_launches"] >= 1 and st["alias_rows"] == 5
     assert st["strict_samples"] > 0      # noise always has sums near an integer
@@ -418,7 +400,7 @@ def test_fast_aligned_flag_is_within_one_lsb(torch_cuda, lz, oracle):
     for maker, seed in ((dark_hwc, 3), (noise_hwc, 4)):
         img = maker(oracle, 270, 480, 3, seed=seed)
         want = oracle.upscale(img, 960, 540, 3, 2, 1)
-        got = gpu_upscale(torch_cuda, lz, img, 960, 540, 3, 2, 1, flags=lz.FLAG_FAST_ALIGNED)
+        got = device_upscale(torch_cuda, lz, img, 960, 540, 3, 2, 1, flags=lz.FLAG_FAST_ALIGNED)
         d = got.astype(np.int16) - want.astype(np.int16)
         assert np.abs(d).max() <= 1
         ys = np.nonzero(d)[0]
@@ -450,21 +432,10 @@ def test_specialised_kernels_bit_exact(torch_cuda, lz, oracle, cfg, kind):
     ow, oh = oracle.out_dims(iw, ih, n, d)
     img = {"noise": noise_hwc, "smooth": smooth_hwc, "dark": dark_hwc}[kind](oracle, ih, iw, c, seed=iw + ih)
     want = oracle.upscale(img, ow, oh, a, n, d, variant=oracle.VERBATIM)
-    got = gpu_upscale(torch_cuda, lz, img, ow, oh, a, n, d)
+    got = device_upscale(torch_cuda, lz, img, ow, oh, a, n, d)
     assert lz.stats()["kernel_id"] == kid
     st = diff_stats(got, want)
     assert st["n_diff"] == 0, st
-
-
-def patchwork_hwc(oracle, h, w, c, seed, band, col):
-    """Image-like, uniform-noise and dark-noise patches side by side: `band` rows x `col` pixels each, in turn."""
-    kinds = [smooth_hwc(oracle, h, w, c, seed), noise_hwc(oracle, h, w, c, seed + 1), dark_hwc(oracle, h, w, c, seed + 2)]
-    yy, xx = np.mgrid[0:h, 0:w]
-    sel = ((yy // band) + (xx // col)) % 3
-    img = np.zeros((h, w, c), dtype=np.uint8)
-    for k in range(3):
-        img[sel == k] = kinds[k][sel == k]
-    return img
 
 
 @pytest.mark.parametrize("cfg", [  # in_w, in_h, n, d, a, c, kernel id, patch rows, patch pixels
@@ -481,7 +452,7 @@ def test_patchwork_content_switches_phase0_modes(torch_cuda, lz, oracle, cfg):
     ow, oh = oracle.out_dims(iw, ih, n, d)
     img = patchwork_hwc(oracle, ih, iw, c, seed=iw + band, band=band, col=col)
     want = oracle.upscale(img, ow, oh, a, n, d, variant=oracle.VERBATIM)
-    got = gpu_upscale(torch_cuda, lz, img, ow, oh, a, n, d)
+    got = device_upscale(torch_cuda, lz, img, ow, oh, a, n, d)
     assert lz.stats()["kernel_id"] == kid
     st = diff_stats(got, want)
     assert st["n_diff"] == 0, st
@@ -510,7 +481,7 @@ def test_tolerance_mode_is_within_one_lsb(torch_cuda, lz, oracle, cfg):
     for maker, floor in ((smooth_hwc, 0.9999), (noise_hwc, 0.98), (dark_hwc, 0.98)):
         img = maker(oracle, ih, iw, c, seed=5)
         want = oracle.upscale(img, ow, oh, a, n, d, variant=oracle.CLEAN)
-        got = gpu_upscale(torch_cuda, lz, img, ow, oh, a, n, d, flags=lz.FLAG_TOLERANCE_1LSB | lz.FLAG_NO_ALIAS)
+        got = device_upscale(torch_cuda, lz, img, ow, oh, a, n, d, flags=lz.FLAG_TOLERANCE_1LSB | lz.FLAG_NO_ALIAS)
         dlt = np.abs(got.astype(np.int16) - want.astype(np.int16))
         assert dlt.max() <= 1                                  # the tolerance: 1 LSB
         exact = float((dlt == 0).mean())
@@ -518,7 +489,7 @@ def test_tolerance_mode_is_within_one_lsb(torch_cuda, lz, oracle, cfg):
     # with the in-place top rows (default flags) the top rows are still produced exactly by the alias kernel
     img = smooth_hwc(oracle, ih, iw, c, seed=6)
     want = oracle.upscale(img, ow, oh, a, n, d, variant=oracle.VERBATIM)
-    got = gpu_upscale(torch_cuda, lz, img, ow, oh, a, n, d, flags=lz.FLAG_TOLERANCE_1LSB)
+    got = device_upscale(torch_cuda, lz, img, ow, oh, a, n, d, flags=lz.FLAG_TOLERANCE_1LSB)
     assert np.abs(got.astype(np.int16) - want.astype(np.int16)).max() <= 1
 
 
@@ -526,9 +497,9 @@ def test_generic_and_specialised_kernels_agree(torch_cuda, lz, oracle):
     """Both code paths must give the reference's bits (kernel_id tells which one ran)."""
     img = noise_hwc(oracle, 200, 320, 3, seed=12)
     want = oracle.upscale(img, 640, 400, 3, 2, 1)
-    a = gpu_upscale(torch_cuda, lz, img, 640, 400, 3, 2, 1)
+    a = device_upscale(torch_cuda, lz, img, 640, 400, 3, 2, 1)
     ka = lz.stats()["kernel_id"]
-    b = gpu_upscale(torch_cuda, lz, img, 640, 400, 3, 2, 1, flags=lz.FLAG_GENERIC_KERNEL)
+    b = device_upscale(torch_cuda, lz, img, 640, 400, 3, 2, 1, flags=lz.FLAG_GENERIC_KERNEL)
     kb = lz.stats()["kernel_id"]
     assert ka == 1 and kb == 0
     assert np.array_equal(a, want) and np.array_equal(b, want)
@@ -539,7 +510,7 @@ def test_config4_shape_4k_to_8k_one_frame(torch_cuda, lz, oracle):
     img = smooth_hwc(oracle, 2160, 3840, 3, seed=5)
     img[:300, :400] = noise_hwc(oracle, 300, 400, 3, seed=6)      # a noisy corner keeps the exact path busy
     want = oracle.upscale(img, 7680, 4320, 3, 2, 1)
-    got = gpu_upscale(torch_cuda, lz, img, 7680, 4320, 3, 2, 1)
+    got = device_upscale(torch_cuda, lz, img, 7680, 4320, 3, 2, 1)
     assert np.array_equal(got, want)
 
 
@@ -554,7 +525,7 @@ def test_output_size_independent_of_ratio(torch_cuda, lz, oracle, cfg, kind):
     iw, ih, ow, oh, n, d, a, c = cfg
     img = {"noise": noise_hwc, "smooth": smooth_hwc}[kind](oracle, ih, iw, c, seed=iw + oh)
     want = oracle.upscale(img, ow, oh, a, n, d)
-    got = gpu_upscale(torch_cuda, lz, img, ow, oh, a, n, d)
+    got = device_upscale(torch_cuda, lz, img, ow, oh, a, n, d)
     st = diff_stats(got, want)
     assert st["max"] == 0, st
 

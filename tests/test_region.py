@@ -17,19 +17,17 @@ import math
 import numpy as np
 import pytest
 
-import test_every_instance as TEI
-import test_near_ties as NTT
-from test_entry_points import NO_DEVICE, ERR_NULL, ERR_DIMS, ERR_TAPS, ERR_CUDA, in_thread
-
-ERR_BAND = -7
+from harness import (ERR_BAND, ERR_CUDA, ERR_DIMS, ERR_NULL, ERR_TAPS, NO_DEVICE, canary_call, in_thread,  # noqa: F401
+                     torch_cuda)
+from util import EMPTY, INSTANCES, h_image, patchwork, patchwork_hwc, tap0, v_image
 
 
 # ---- the rect a window reads ----------------------------------------------------------------------------------
 
 def needed_cols(iw, n, d, a, x0, w):
     """First and last input column that the output columns [x0, x0 + w) read, clipped to the image."""
-    lo = max(0, NTT.tap0(x0, n, d, a))
-    hi = min(iw - 1, NTT.tap0(x0 + w - 1, n, d, a) + 2 * a - 1)
+    lo = max(0, tap0(x0, n, d, a))
+    hi = min(iw - 1, tap0(x0 + w - 1, n, d, a) + 2 * a - 1)
     return lo, hi
 
 
@@ -60,7 +58,7 @@ def test_region_input_rect(lz, n, d):
                 assert (iy, ihr) == lz.band_input_rows(desc, y0, h)
                 assert 0 <= ix and ix + iwr <= iw and (ix * c) % 16 == 0
                 xx = np.arange(x0, x0 + w)
-                taps = NTT.tap0(xx, n, d, a)[:, None] + np.arange(2 * a)[None, :]
+                taps = tap0(xx, n, d, a)[:, None] + np.arange(2 * a)[None, :]
                 inside = (taps >= 0) & (taps < iw)
                 assert np.all(~inside | ((taps >= ix) & (taps < ix + iwr))), (n, d, a, c, x0, w)
                 lo, hi = needed_cols(iw, n, d, a, x0, w)
@@ -106,17 +104,6 @@ def test_error_order_of_region_entry_points(lz):
 
 # ---- GPU --------------------------------------------------------------------------------------------------------
 
-@pytest.fixture(scope="module")
-def torch_cuda():
-    import torch
-    assert torch.cuda.is_available(), "GPU tests need a CUDA device"
-    return torch
-
-
-CANARY = 0xA7
-LEAD = 64
-
-
 def word_rect(rect, iw, c):
     """The rect widened to the right, inside the image, until its rows are whole 32-bit words (the fast kernels
     read the rect through a map of words)."""
@@ -126,59 +113,20 @@ def word_rect(rect, iw, c):
     return ix, iy, w, h
 
 
-def run_region(torch, lz, desc, frames, win, rect=None, flags=None, stats=False, in_fstride_pad=0, out_fstride_pad=0,
-               whole=False):
+def run_region(torch, lz, desc, frames, win, rect=None, flags=None, stats=False, in_gap=0, out_gap=0, whole=False):
     """Window win = (x0, y0, w, h) of `frames` (list of [H][W][C] host images) through lanczos_b200_upscale_region
-    (whole: the whole image through lanczos_b200_upscale, same buffers).  The rect (default: region_input_rect widened
-    to whole words) is copied into a buffer of random bytes with padded rows; the window lands in a buffer of canaries.
-    Returns (windows, stats, launch) and checks every canary."""
-    x0, y0, w, h = win
+    (whole: the whole image through lanczos_b200_upscale, same buffers) with canary_call.  The rect (default:
+    region_input_rect widened to whole words) has rows padded past the next 16 bytes; the window's rows are padded past
+    the next 8.  `flags` replaces desc.flags.  Returns (windows, stats, launch)."""
+    x0, y0, w, _ = win
     ih, iw, c = frames[0].shape
     rect = rect or word_rect(lz.region_input_rect(desc, *win), iw, c)
-    ix, iy, riw, rih = rect
-    nf = len(frames)
-    rng = np.random.default_rng(x0 * 7919 + y0 * 31 + w + nf)
-    in_pitch = -(-riw * c // 16) * 16 + 16
-    in_fs = in_pitch * rih + in_fstride_pad
-    src = rng.integers(0, 256, 256 + in_fs * nf + 256, dtype=np.uint8)
-    for f, img in enumerate(frames):
-        view = np.lib.stride_tricks.as_strided(src[256 + f * in_fs:], shape=(rih, riw * c), strides=(in_pitch, 1))
-        view[...] = img[iy:iy + rih, ix:ix + riw].reshape(rih, riw * c)
-    rb = w * c
-    out_pitch = -(-rb // 8) * 8 + 8
-    out_fs = out_pitch * h + out_fstride_pad
-    total = LEAD + out_fs * (nf - 1) + out_pitch * h + 2 * out_pitch + 64
-    d_in = torch.from_numpy(src).cuda()
-    buf = torch.full((total,), CANARY, dtype=torch.uint8, device="cuda")
-    d = lz.Desc.from_buffer_copy(desc)
-    d.in_pitch, d.out_pitch = in_pitch, out_pitch
     if flags is not None:
-        d.flags = flags
-    L = lz.lib()
-    lz.enable_stats(stats)
-    try:
-        stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-        if whole:
-            rc = L.lanczos_b200_upscale(C.byref(d), C.c_void_p(d_in.data_ptr() + 256), C.c_void_p(buf.data_ptr() + LEAD),
-                                        0, stream)
-        else:
-            rc = L.lanczos_b200_upscale_region(C.byref(d), C.c_void_p(d_in.data_ptr() + 256),
-                                               C.c_void_p(buf.data_ptr() + LEAD), x0, y0, w, h, ix, iy, riw, rih, nf,
-                                               in_fs if nf > 1 else 0, out_fs if nf > 1 else 0, 0, stream)
-        torch.cuda.synchronize()
-        st, ln = lz.stats(), lz.launch()
-    finally:
-        lz.enable_stats(False)
-    assert rc == 0, (rc, L.lanczos_b200_strerror(rc), win, rect)
-    host = buf.cpu().numpy()
-    outs = [np.array(np.lib.stride_tricks.as_strided(host[LEAD + f * out_fs:], shape=(h, rb), strides=(out_pitch, 1)))
-            .reshape(h, w, c) for f in range(nf)]
-    canary = np.ones(total, bool)
-    for f in range(nf):
-        np.lib.stride_tricks.as_strided(canary[LEAD + f * out_fs:], shape=(h, rb), strides=(out_pitch, 1))[...] = False
-    hit = np.nonzero(canary & (host != CANARY))[0]
-    assert len(hit) == 0, ("canary bytes overwritten", win, len(hit), [int(i) - LEAD for i in hit[:8]])
-    return outs, st, ln
+        desc = lz.Desc.from_buffer_copy(desc)
+        desc.flags = flags
+    return canary_call(torch, lz, desc, frames, "upscale" if whole else "upscale_region", win=win, rect=rect, in_off=256,
+                       in_pad=(-rect[2] * c) % 16 + 16, in_gap=in_gap, out_pad=(-w * c) % 8 + 8, out_gap=out_gap,
+                       seed=x0 * 7919 + y0 * 31 + w + len(frames), stats=stats)
 
 
 def full_frame(torch, lz, desc, img, flags):
@@ -196,9 +144,10 @@ def crop(ref, win):
 GENERIC = 1 << 2   # LANCZOS_FLAG_GENERIC_KERNEL
 
 # (name, channels, a, N, D, flags, kernel id of aligned windows, kernel id of unaligned windows)
-DYN_IDS = {(c, a, n, d): kid for (kid, c, a, n, d) in TEI.DYN}
-FAMILIES = ([("v6_%d" % kid, c, a, n, d, 0, kid, DYN_IDS.get((c, a, n, d), 0)) for (kid, c, a, n, d, ph, km) in TEI.V6]
-            + [("dyn_%d" % kid, c, a, n, d, 0, kid, kid) for (kid, c, a, n, d) in TEI.DYN]
+DYN_IDS = {(i.c, i.a, i.n, i.d): i.kid for i in INSTANCES if i.family == "dyn"}
+FAMILIES = ([("v6_%d" % i.kid, i.c, i.a, i.n, i.d, 0, i.kid, DYN_IDS.get((i.c, i.a, i.n, i.d), 0))
+             for i in INSTANCES if i.family == "v6"]
+            + [("dyn_%d" % i.kid, i.c, i.a, i.n, i.d, 0, i.kid, i.kid) for i in INSTANCES if i.family == "dyn"]
             + [("generic_c%d" % c, c, a, n, d, GENERIC, 0, 0) for (c, a, n, d) in [(1, 3, 4, 1), (2, 3, 5, 3), (3, 2, 17, 10),
                                                                                  (4, 3, 7, 4)]]
             + [("alias_rows", 3, 3, 3, 2, 0, 6, 6)])
@@ -231,7 +180,7 @@ def family_windows(ow, oh, c, n, d, alias):
 def test_windows_of_every_family(torch_cuda, lz, oracle, name):
     torch = torch_cuda
     c, a, n, d, flags, kid_aligned, kid_unaligned = FAMILY[name]
-    img = TEI.patchwork(oracle, c, n, d, seed=400 + c * 7 + n)
+    img = patchwork(oracle, c, n, d, seed=400 + c * 7 + n)
     ih, iw, _ = img.shape
     ow, oh = oracle.out_dims(iw, ih, n, d)
     desc = lz.make_desc(iw, ih, ow, oh, c, a, n, d, flags=flags)
@@ -258,12 +207,12 @@ def test_windows_of_every_family(torch_cuda, lz, oracle, name):
 @pytest.mark.gpu
 @pytest.mark.parametrize("kid", [f[6] for f in FAMILIES if f[0].startswith(("v6", "dyn"))])
 def test_strict_paths_at_column_offsets(torch_cuda, lz, oracle, kid):
-    """The near-tie images of test_near_ties.py: the exact re-evaluation runs at a column offset, and is right."""
+    """The near-tie images of tests/util.py: the exact re-evaluation runs at a column offset, and is right."""
     torch = torch_cuda
     name = [f[0] for f in FAMILIES if f[6] == kid and f[0].startswith(("v6", "dyn"))][0]
     c, a, n, d, flags, _, _ = FAMILY[name]
     step = 16 // math.gcd(16, c)
-    for img, _ in (NTT.h_image(oracle, n, d, a, c, seed=500 + kid), NTT.v_image(oracle, n, d, a, c, seed=500 + kid)):
+    for img, _ in (h_image(oracle, n, d, a, c, seed=500 + kid), v_image(oracle, n, d, a, c, seed=500 + kid)):
         ih, iw, _ = img.shape
         ow, oh = oracle.out_dims(iw, ih, n, d)
         desc = lz.make_desc(iw, ih, ow, oh, c, a, n, d)
@@ -275,7 +224,7 @@ def test_strict_paths_at_column_offsets(torch_cuda, lz, oracle, kid):
         bad = np.argwhere(got != crop(ref, win))
         assert len(bad) == 0, (name, win, len(bad), bad[:8].tolist())
         assert st["kernel_id"] == kid, (name, st)
-        assert st["strict_samples"] > 0 or (n, d, a) in NTT.EMPTY, (name, st)   # EMPTY: the ratio has no near ties
+        assert st["strict_samples"] > 0 or (n, d, a) in EMPTY, (name, st)   # EMPTY: the ratio has no near ties
 
 
 # 2/1 RGB (v6 id 1), 3/2 RGBA (v6 id 3), 17/10 RGB (dyn id 5) and 17/10 RGB with a = 2 (generic only)
@@ -286,7 +235,7 @@ TILE_CASES = [(3, 3, 2, 1, 1), (4, 3, 3, 2, 3), (3, 3, 17, 10, 5), (3, 2, 17, 10
 @pytest.mark.parametrize("c,a,n,d,kid", TILE_CASES)
 def test_tiles_assemble_to_the_whole_image(torch_cuda, lz, oracle, c, a, n, d, kid):
     torch = torch_cuda
-    img = TEI.patchwork(oracle, c, n, d, seed=600 + n)
+    img = patchwork(oracle, c, n, d, seed=600 + n)
     ih, iw, _ = img.shape
     ow, oh = oracle.out_dims(iw, ih, n, d)
     desc = lz.make_desc(iw, ih, ow, oh, c, a, n, d)
@@ -317,15 +266,15 @@ def test_tiles_assemble_to_the_whole_image(torch_cuda, lz, oracle, c, a, n, d, k
 def test_batch_window_with_frame_strides(torch_cuda, lz, oracle, name):
     torch = torch_cuda
     c, a, n, d, flags, _, _ = FAMILY[name]
-    frames = [TEI.patchwork(oracle, c, n, d, seed=700 + f) for f in range(3)]
+    frames = [patchwork(oracle, c, n, d, seed=700 + f) for f in range(3)]
     ih, iw, _ = frames[0].shape
     ow, oh = oracle.out_dims(iw, ih, n, d)
     desc = lz.make_desc(iw, ih, ow, oh, c, a, n, d, flags=flags)
+    refs = [oracle.upscale(img, ow, oh, a, n, d, variant=oracle.VERBATIM) for img in frames]
     for win in [(16, 5, 160, 40), (33, 0, 100, 30)]:
-        got, st, ln = run_region(torch, lz, desc, frames, win, in_fstride_pad=48, out_fstride_pad=12)
+        got, st, ln = run_region(torch, lz, desc, frames, win, in_gap=48, out_gap=12)
         assert ln["grid_z"] == 3, ln
-        for f, img in enumerate(frames):
-            ref = TEI.oracle_ref(oracle, img, a, n, d, oracle.VERBATIM)
+        for f, ref in enumerate(refs):
             assert np.array_equal(got[f], crop(ref, win)), (name, win, f)
 
 
@@ -335,7 +284,7 @@ def test_tolerance_mode_window(torch_cuda, lz, oracle, name):
     """A window of the tolerance-mode result equals the same pixels of the whole image in that mode."""
     torch = torch_cuda
     c, a, n, d, _, kid, _ = FAMILY[name]
-    img = TEI.patchwork(oracle, c, n, d, seed=800)
+    img = patchwork(oracle, c, n, d, seed=800)
     ih, iw, _ = img.shape
     ow, oh = oracle.out_dims(iw, ih, n, d)
     desc = lz.make_desc(iw, ih, ow, oh, c, a, n, d)
@@ -353,7 +302,7 @@ def test_tolerance_mode_window(torch_cuda, lz, oracle, name):
 def test_independent_flag_on_consecutive_windows(torch_cuda, lz, oracle):
     torch = torch_cuda
     c, a, n, d = 3, 3, 2, 1
-    img = TEI.patchwork(oracle, c, n, d, seed=900)
+    img = patchwork(oracle, c, n, d, seed=900)
     ih, iw, _ = img.shape
     ow, oh = oracle.out_dims(iw, ih, n, d)
     full = torch.from_numpy(np.ascontiguousarray(np.pad(img, ((0, 0), (0, (-iw) % 16), (0, 0))))).cuda()[:, :iw]
@@ -378,7 +327,7 @@ def test_independent_flag_on_consecutive_windows(torch_cuda, lz, oracle):
 @pytest.mark.parametrize("c,n,d", [(3, 2, 1), (3, 17, 10), (4, 3, 2)])
 def test_torch_view_equals_tight_copy(torch_cuda, lz, oracle, c, n, d):
     torch = torch_cuda
-    img = TEI.patchwork(oracle, c, n, d, seed=1000)
+    img = patchwork(oracle, c, n, d, seed=1000)
     ih, iw, _ = img.shape
     ow, oh = oracle.out_dims(iw, ih, n, d)
     desc = lz.make_desc(iw, ih, ow, oh, c, 3, n, d)
@@ -398,7 +347,7 @@ def test_torch_view_equals_tight_copy(torch_cuda, lz, oracle, c, n, d):
 @pytest.mark.gpu
 @pytest.mark.parametrize("iw,ih,c,n,d", [(61, 37, 3, 2, 1), (64, 40, 4, 3, 2), (57, 30, 1, 3, 1), (45, 25, 2, 2, 1)])
 def test_host_region(lz, oracle, iw, ih, c, n, d):
-    img = TEI.patchwork_hwc(oracle, ih, iw, c, seed=c, band=7, col=11)
+    img = patchwork_hwc(oracle, ih, iw, c, seed=c, band=7, col=11)
     ow, oh = oracle.out_dims(iw, ih, n, d)
     ref = oracle.upscale(img, ow, oh, 3, n, d)
     for win in [(0, 0, ow, oh), (3, 1, 11, 7), (ow - 9, oh - 5, 9, 5), (ow // 2, 0, 1, oh)]:
