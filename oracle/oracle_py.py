@@ -155,12 +155,15 @@ def hls_lut(a, n, bp=8):
     return np.array(buf[:], dtype=np.int32)
 
 
-def hls_upscale(img, n, a=3, bp=8):
-    """Fixed-point HLS path on an interleaved [H][W][C] image, integer scale n."""
+def hls_upscale(img, n, a=3, bp=8, out_w=None, out_h=None):
+    """Fixed-point HLS path on an interleaved [H][W][C] image, integer scale n; the output is
+    out_w x out_h (default w*n x h*n), also when that is not the input's size times n."""
     img = np.ascontiguousarray(img, dtype=np.uint8)
     h, w, c = img.shape
-    out = np.empty((h * n, w * n, c), dtype=np.uint8)
-    if lib().oracle_hls_upscale(_p(img), _p(out), c, w, h, w * n, h * n, a, n, bp) != 0:
+    out_w = w * n if out_w is None else out_w
+    out_h = h * n if out_h is None else out_h
+    out = np.empty((out_h, out_w, c), dtype=np.uint8)
+    if lib().oracle_hls_upscale(_p(img), _p(out), c, w, h, out_w, out_h, a, n, bp) != 0:
         raise ValueError("oracle rejected the HLS arguments")
     return out
 

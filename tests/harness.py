@@ -64,9 +64,10 @@ def overwritten(host, base, frames, rows, row_bytes, pitch, fstride):
 
 
 def canary_call(torch, lz, desc, frames, entry, win=None, rect=None, in_off=0, in_pad=0, in_gap=0, out_off=0,
-                out_pad=0, out_gap=0, seed=0, stats=False):
-    """One call of lanczos_b200_<entry> (upscale, upscale_batch or upscale_region) on `frames` (list of [H][W][C] host
-    images) with `desc` (its pitches are replaced), on device buffers laid out as asked.
+                out_pad=0, out_gap=0, seed=0, stats=False, bit_precision=8):
+    """One call of lanczos_b200_<entry> (upscale, upscale_batch, upscale_region or upscale_hls, the last with
+    `bit_precision`) on `frames` (list of [H][W][C] host images) with `desc` (its pitches are replaced), on device
+    buffers laid out as asked.
 
     Input: the rect (ix, iy, w, h) of every frame (default the whole frame) at `in_off` bytes past a 256-byte
     boundary, rows padded by `in_pad` bytes, frames `in_gap` bytes apart; every other byte of the buffer is random
@@ -100,6 +101,8 @@ def canary_call(torch, lz, desc, frames, entry, win=None, rect=None, in_off=0, i
             rc = L.lanczos_b200_upscale(C.byref(d), p_in, p_out, 0, stream)
         elif entry == "upscale_batch":
             rc = L.lanczos_b200_upscale_batch(C.byref(d), p_in, p_out, nf, in_fs, out_fs, 0, stream)
+        elif entry == "upscale_hls":
+            rc = L.lanczos_b200_upscale_hls(C.byref(d), p_in, p_out, bit_precision, nf, in_fs, out_fs, 0, stream)
         else:
             assert entry == "upscale_region", entry
             rc = L.lanczos_b200_upscale_region(C.byref(d), p_in, p_out, x0, y0, w, h, ix, iy, riw, rih, nf, in_fs,

@@ -4,6 +4,7 @@ Xilinx hls::sinpi, absent here); the CUDA path is checked bit for bit against or
 import numpy as np
 import pytest
 
+from harness import CANARY
 from util import noise_hwc, smooth_hwc
 
 
@@ -49,7 +50,7 @@ def test_gpu_matches_integer_restatement(lz, oracle, cfg):
         img = maker(oracle, h, w, c, seed=w)
         want = oracle.hls_upscale(img, n, a, bp)
         d_in = torch.from_numpy(img).cuda()
-        d_out = torch.zeros((h * n, w * n, c), dtype=torch.uint8, device="cuda")
+        d_out = torch.full((h * n, w * n, c), CANARY, dtype=torch.uint8, device="cuda")
         lz.upscale_hls_device(d_in, d_out, a=a, bit_precision=bp)
         torch.cuda.synchronize()
         assert np.array_equal(d_out.cpu().numpy(), want)
@@ -62,7 +63,7 @@ def test_gpu_hls_batch_and_errors(lz, oracle):
     import torch
     frames = np.stack([noise_hwc(oracle, 20, 28, 3, seed=s) for s in range(3)])
     d_in = torch.from_numpy(frames).cuda()
-    d_out = torch.zeros((3, 40, 56, 3), dtype=torch.uint8, device="cuda")
+    d_out = torch.full((3, 40, 56, 3), CANARY, dtype=torch.uint8, device="cuda")
     lz.upscale_hls_device(d_in, d_out)
     torch.cuda.synchronize()
     for i in range(3):
